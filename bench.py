@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- fold-stage throughput on B200 (BASELINE.json metric: folded nt/sec, RNALfold -L 300, at 1/2/4/8 B200).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (encode -> c/fML band fill -> f3 -> plan/traceback/emission) over the whole
@@ -14,6 +14,9 @@ ranks only take part in the barriers (loci are independent: there is no data-pat
 the library's streams, max over devices); `e2e` = the same metric through the public host API mirfold_fold (host
 buffers in, hit records out, all copies inside the timed region).  `weak` keeps round 1's line: every rank folds its
 own parity-10k batch (BASELINE configs[1]) on its own GPU.
+
+--dump-outputs DIR writes the result of the last timed step as DIR/<name>.npy (see dump_outputs()), so that two builds
+run with the same arguments, hence on the same seeded inputs, can be compared output for output.
 """
 import argparse
 import hashlib
@@ -278,7 +281,7 @@ def weak_line(args, mp, torch, dist, rank, world, local_rank, barrier):
     buf, off = workload_packed(rank, 10000, "parity")
     nt = int(off[-1])
     mf = mp.MirFold(devices=[local_rank])
-    steps = max(2, min(args.steps, 3))
+    steps = args.steps
     with mf.upload(buf, off, SPAN) as batch:
         batch.fold().close()
         barrier()
@@ -351,6 +354,7 @@ def run_ours(args, rank, world, local_rank):
                 dev_ms.append(r.stats["ms_device"])     # CUDA events on the library's streams, max over devices
                 launches += r.stats["kernel_launches"]
                 n_chunks, tracebacks, cells = r.stats["n_chunks"], r.stats["tracebacks"], r.stats["cells"]
+                last_step = (r.nhits, r.ss_bytes)
         wall_resident = time.perf_counter() - t0
     barrier()
     if rank == 0:
@@ -444,6 +448,8 @@ def run_ours(args, rank, world, local_rank):
                 raise RuntimeError("parity broken: text sha256 %s != pinned %s" % (sha, pin["sha256"]))
         if world == 1 and not args.no_dropin:
             out["drop_in"] = drop_in_stages(mf, buf, off, lens)
+        if args.dump_outputs:
+            out["dump_outputs"] = dump_outputs(batch, last_step, lens, args.dump_outputs)
         batch.close()
         mf.close()
     barrier()
@@ -508,6 +514,55 @@ def drop_in_stages(mf, buf, off, lens):
     return out
 
 
+DUMP_SEED = 0
+DUMP_RECORDS = 1 << 20          # per-record arrays: every record up to this many, else a seeded sample of this size
+DUMP_HIT_NT = 300000            # per-hit arrays: the hits of a seeded sample of records with about this many input nt
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(batch, last_step, lens, outdir):
+    """Write the result of the timed path's last step under outdir as .npy files (float64; the dot-brackets float32).
+
+    The timed steps leave their results in HBM, so the same batch is folded once more outside the timed region with
+    the download on; the fold is deterministic, and its hit count and dot-bracket bytes must equal the last timed
+    step's.  Records are sampled by a seeded permutation, so the same arguments dump the same records:
+      records, total_mfe_dcal, hit_count         per record: its index, total MFE (dcal/mol), hairpin lines printed
+      hit_records                                the records whose hits follow (a prefix of the same permutation)
+      hit_start, hit_len, hit_mfe_dcal           their hits, record by record in RNALfold's print order
+      hit_ss                                     the hits' dot-brackets concatenated: '(' = 1, ')' = -1, '.' = 0
+    """
+    with batch.fold(download=True) as res:
+        if (res.nhits, res.ss_bytes) != last_step or res.nseq != len(lens):
+            raise RuntimeError("the downloaded fold (%d hits, %d B) differs from the last timed step (%d hits, %d B)"
+                               % ((res.nhits, res.ss_bytes) + tuple(last_step)))
+        perm = np.random.default_rng(DUMP_SEED).permutation(res.nseq)
+        rec = np.sort(perm[:DUMP_RECORDS])
+        arrays = {"records": rec.astype(np.float64), "total_mfe_dcal": res.total_mfe_dcal[rec].astype(np.float64),
+                  "hit_count": res.hit_count[rec].astype(np.float64)}
+        budget = DUMP_MAX_BYTES - sum(a.nbytes for a in arrays.values()) - 4096      # 4096: the .npy headers
+        k = max(1, int(np.searchsorted(np.cumsum(lens[perm]), DUMP_HIT_NT, side="right")))
+        while True:
+            hrec = np.sort(perm[:k])
+            hb, hc = res.hit_begin[hrec].astype(np.int64), res.hit_count[hrec].astype(np.int64)
+            rows = np.repeat(hb, hc) + (np.arange(int(hc.sum())) - np.repeat(np.cumsum(hc) - hc, hc))
+            hits = res.hit_table[rows]
+            n = hits["len"].astype(np.int64)
+            if 8 * (len(hrec) + 3 * len(rows)) + 4 * int(n.sum()) <= budget or k == 1:
+                break
+            k //= 2
+        chars = np.repeat(hits["ss_off"].astype(np.int64), n) + (np.arange(int(n.sum())) - np.repeat(np.cumsum(n) - n, n))
+        code = np.zeros(256, np.float32)
+        code[ord("(")], code[ord(")")] = 1, -1
+        arrays.update({"hit_records": hrec.astype(np.float64), "hit_start": hits["start"].astype(np.float64),
+                       "hit_len": n.astype(np.float64), "hit_mfe_dcal": hits["mfe_dcal"].astype(np.float64),
+                       "hit_ss": code[res.arena[chars]]})
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), a)
+    return {"dir": os.path.abspath(outdir), "files": sorted(arrays), "bytes": sum(a.nbytes for a in arrays.values()),
+            "records": len(rec), "hit_records": len(hrec), "hits": len(rows)}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -524,7 +579,12 @@ def main():
     ap.add_argument("--workload", default="arabidopsis", choices=sorted(WORKLOADS),
                     help="length law of SURVEY 8(d); the bench line of record is the default (arabidopsis-200k, BASELINE configs[2])")
     ap.add_argument("--span", type=int, default=300, help="RNALfold -L (default 300)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the result of --impl ours")
     global WORKLOAD, SPAN
     WORKLOAD, SPAN = args.workload, args.span
     if args.loci <= 0:

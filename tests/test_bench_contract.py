@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 from conftest import ROOT
 
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
@@ -64,3 +66,26 @@ def test_reference_arm_runs_here():
                           "--ref-loci-per-core", "1"], stdout=subprocess.PIPE, check=True, timeout=600).stdout.decode()
     d = json.loads(out.strip().splitlines()[-1])
     assert d["impl"] == "reference" and d["value"] > 0 and d["unit"] == "nt/s" and d["steps"] == 1
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_oracles_result(oracle, tmp_path):
+    """bench.py --dump-outputs on a small slice of the workload: the .npy files are the oracle's fold of the same loci."""
+    import numpy as np
+    from mir_prefer_b200.corpus import synth_loci
+    dump = tmp_path / "dump"
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--loci", "64", "--steps", "2", "--warmup", "1", "--no-cpu",
+                          "--no-sha", "--no-dropin", "--dump-outputs", str(dump)], stdout=subprocess.PIPE, check=True, timeout=600,
+                         env=dict(os.environ, MIRFOLD_CORPUS_DIR=str(tmp_path))).stdout.decode()
+    d = json.loads(out.strip().splitlines()[-1])
+    assert d["steps"] == 2 and d["dump_outputs"]["records"] == 64 and d["dump_outputs"]["bytes"] <= 64 << 20
+    a = {f.stem: np.load(f) for f in dump.glob("*.npy")}
+    assert len(a) == 8 and all(x.dtype in (np.float32, np.float64) for x in a.values())
+    want = [oracle.fold(s, 300) for s in synth_loci(1002, 64, "arabidopsis")]      # bench.WORKLOADS["arabidopsis"], rank 0
+    assert a["records"].tolist() == a["hit_records"].tolist() == list(range(64))
+    assert a["total_mfe_dcal"].tolist() == [o["total"] for o in want]
+    assert a["hit_count"].tolist() == [len(o["hits"]) for o in want]
+    hits = [h for o in want for h in o["hits"]]
+    assert a["hit_start"].tolist() == [h[2] for h in hits] and a["hit_mfe_dcal"].tolist() == [h[1] for h in hits]
+    assert a["hit_len"].tolist() == [len(h[0]) for h in hits]
+    assert "".join(".()"[int(v)] for v in a["hit_ss"]) == "".join(h[0] for h in hits)   # codes 0, 1, -1

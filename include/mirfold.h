@@ -161,6 +161,38 @@ int mirfold_batch_upload(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq
 int mirfold_batch_fold(mirfold_ctx *ctx, mirfold_batch *batch, uint32_t flags, int download, mirfold_result **out);
 void mirfold_batch_free(mirfold_batch *batch);
 
+/* Genome-resident input.  Replaces what dump_piece does per record before the fold (miR_PREFeR.py:1097-1108, :1131, :1177):
+ * ask `samtools faidx` for the bases of the extend region and reverse-complement minus-strand records.  The genome is
+ * uploaded once; records are then given as coordinates and cut, oriented and encoded on the device.
+ *   mirfold_genome_upload: contig c is seq[contig_off[c] .. contig_off[c+1]) (n_contigs+1 offsets, letters exactly as in
+ *     the FASTA); one copy is kept on every device of ctx, and its bytes are taken off the lanes' memory budget while it
+ *     lives (unless MIRFOLD_MEM_BUDGET_MB sets the budget).  mirfold_genome_free may be called before or after
+ *     mirfold_close (the context's host bookkeeping lives until its last result and genome are freed).
+ *   mirfold_genome_region: [start, end) is the extend region exactly as dump_piece prints it, strand '+' or '-', contig
+ *     an index into the upload (-1: a seqid that is not in the FASTA, an empty record).  The folded bases are samtools
+ *     0.1.18's `faidx seqid:start-(end-1)`: start clipped to >= 1, end-1 clipped to the contig length, empty if start >
+ *     end-1.  A minus-strand record is reversed and complemented with the reference's get_complement table
+ *     (miR_PREFeR.py:232-239): upper-case A T G C U only, so lower-case and IUPAC letters are reversed but not complemented.
+ * mirfold_fold_regions / _stream / mirfold_fold_candidates_regions return byte for byte what mirfold_fold /
+ * mirfold_fold_stream / mirfold_fold_candidates return on the host-extracted sequences; the duplex checks of the
+ * candidates see the unclipped (start, end).  Only descriptors are uploaded per call (stats.h2d_bytes).  Each returns
+ * MIRFOLD_ERR_ARG, and no result, for a contig index outside [-1, n_contigs), a strand other than '+' / '-', a genome of
+ * another context or a closed context. */
+typedef struct mirfold_genome mirfold_genome;
+typedef struct mirfold_genome_region {
+    int32_t contig;
+    int32_t start, end;   /* [start, end), 1-based genome coordinates */
+    int32_t strand;       /* '+' or '-' */
+} mirfold_genome_region;
+int mirfold_genome_upload(mirfold_ctx *ctx, const char *seq, const uint64_t *contig_off, uint32_t n_contigs,
+                          mirfold_genome **out);
+void mirfold_genome_free(mirfold_genome *genome);
+int mirfold_fold_regions(mirfold_ctx *ctx, const mirfold_genome *genome, const mirfold_genome_region *regions, uint32_t nseq,
+                         int span_L, uint32_t flags, mirfold_result **out);
+int mirfold_fold_regions_stream(mirfold_ctx *ctx, const mirfold_genome *genome, const mirfold_genome_region *regions,
+                                uint32_t nseq, int span_L, uint32_t flags, mirfold_chunk_fn fn, void *user,
+                                mirfold_stats *stats /* may be NULL */);
+
 /* Replaces: the split of the candidate FASTA into NUM_OF_CORE shards by locus count (miR_PREFeR.py:1329-1354)
  * that decides which RNALfold process folds which record (miR_PREFeR.py:3113-3118).  Here: greedy
  * longest-processing-time assignment by DP cells (SURVEY.md 8e), exactly the plan mirfold_fold() uses for a
@@ -312,6 +344,12 @@ int mirfold_fold_candidates(mirfold_ctx *ctx, const char *seqs, const uint64_t *
                             uint32_t flags, const mirfold_region *regions, const mirfold_mature *matures,
                             const uint64_t *mature_off, int minlen, int minloop, int min_mature_len, int max_mature_len,
                             mirfold_candidates **out);
+/* The same with the records given as regions of a resident genome (mirfold_genome_upload above); regions[r] also stands
+ * for the mirfold_region of record r, unclipped. */
+int mirfold_fold_candidates_regions(mirfold_ctx *ctx, const mirfold_genome *genome, const mirfold_genome_region *regions,
+                                    uint32_t nseq, int span_L, uint32_t flags, const mirfold_mature *matures,
+                                    const uint64_t *mature_off, int minlen, int minloop, int min_mature_len,
+                                    int max_mature_len, mirfold_candidates **out);
 void mirfold_free_candidates(mirfold_candidates *c);
 
 #ifdef __cplusplus

@@ -75,6 +75,10 @@ class Region(C.Structure):
     _fields_ = [("start", C.c_int32), ("end", C.c_int32)]
 
 
+class GenomeRegion(C.Structure):
+    _fields_ = [("contig", C.c_int32), ("start", C.c_int32), ("end", C.c_int32), ("strand", C.c_int32)]
+
+
 class Candidates(C.Structure):
     _fields_ = [("nseq", C.c_uint32), ("reserved", C.c_uint32), ("nstructs", C.c_uint64),
                 ("struct_begin", C.POINTER(C.c_uint64)), ("struct_count", C.POINTER(C.c_uint32)),
@@ -94,7 +98,9 @@ EXPORTS = ["mirfold_open", "mirfold_close", "mirfold_fold", "mirfold_fold_device
            "mirfold_free_result", "mirfold_strerror", "mirfold_last_error", "mirfold_version", "mirfold_duplex",
            "mirfold_duplex_fail_name", "mirfold_int_peak", "mirfold_format_records", "mirfold_free_text",
            "mirfold_classify", "mirfold_free_structures", "mirfold_fold_stream", "mirfold_batch_upload", "mirfold_batch_fold",
-           "mirfold_batch_free", "mirfold_plan_shards", "mirfold_int_peak2", "mirfold_fold_candidates", "mirfold_free_candidates", "mirfold_fold_text", "mirfold_plan_fill_units"]
+           "mirfold_batch_free", "mirfold_plan_shards", "mirfold_int_peak2", "mirfold_fold_candidates", "mirfold_free_candidates", "mirfold_fold_text", "mirfold_plan_fill_units",
+           "mirfold_genome_upload", "mirfold_genome_free", "mirfold_fold_regions", "mirfold_fold_regions_stream",
+           "mirfold_fold_candidates_regions"]
 
 _lib = None
 
@@ -173,5 +179,19 @@ def load():
     lib.mirfold_fold_candidates.restype = C.c_int
     lib.mirfold_free_candidates.argtypes = [C.POINTER(Candidates)]
     lib.mirfold_free_candidates.restype = None
+    if hasattr(lib, "mirfold_genome_upload") or not os.environ.get("MIRFOLD_LIB_PATH"):   # an A/B build may predate genomes
+        lib.mirfold_genome_upload.argtypes = [vp, C.c_void_p, C.POINTER(C.c_uint64), C.c_uint32, C.POINTER(vp)]
+        lib.mirfold_genome_upload.restype = C.c_int
+        lib.mirfold_genome_free.argtypes = [vp]
+        lib.mirfold_genome_free.restype = None
+        lib.mirfold_fold_regions.argtypes = [vp, vp, C.c_void_p, C.c_uint32, C.c_int, C.c_uint32, C.POINTER(C.POINTER(Result))]
+        lib.mirfold_fold_regions.restype = C.c_int
+        lib.mirfold_fold_regions_stream.argtypes = [vp, vp, C.c_void_p, C.c_uint32, C.c_int, C.c_uint32, CHUNK_FN, C.c_void_p,
+                                                    C.POINTER(Stats)]
+        lib.mirfold_fold_regions_stream.restype = C.c_int
+        lib.mirfold_fold_candidates_regions.argtypes = [vp, vp, C.c_void_p, C.c_uint32, C.c_int, C.c_uint32, C.c_void_p,
+                                                        C.POINTER(C.c_uint64), C.c_int, C.c_int, C.c_int, C.c_int,
+                                                        C.POINTER(C.POINTER(Candidates))]
+        lib.mirfold_fold_candidates_regions.restype = C.c_int
     _lib = lib
     return lib

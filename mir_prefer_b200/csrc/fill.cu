@@ -30,14 +30,21 @@ __global__ void k_prepare(const char *__restrict__ raw, const LocusDesc *__restr
                           unsigned char *__restrict__ codes, int *__restrict__ F)
 {
     // one CTA per locus; RNALfold main(): toupper, T->U; encode_char + alias (A.1)
+    // raw_off bit 63 (MF_RAW_REVERSE, uniform per CTA): a minus-strand genome region -- base k is raw[off + n - k]
+    // through the reference's get_complement table (upper-case A T G C U only; miR_PREFeR.py:232-239), then as above
     const LocusDesc L = loci[blockIdx.x];
-    const char *src = raw + L.raw_off;
+    const bool rev = (L.raw_off & MF_RAW_REVERSE) != 0;
+    const char *src = raw + (L.raw_off & ~MF_RAW_REVERSE);
     unsigned char *dst = codes + L.seq_off;
     int *f = F + L.seq_off;
     for (int k = threadIdx.x; k < L.n + 3; k += blockDim.x) {
         int s = 0;
         if (k >= 1 && k <= L.n) {
-            char ch = src[k - 1];
+            char ch;
+            if (rev) {
+                ch = src[L.n - k];
+                ch = ch == 'A' ? 'U' : ch == 'T' ? 'A' : ch == 'G' ? 'C' : ch == 'C' ? 'G' : ch == 'U' ? 'A' : ch;
+            } else ch = src[k - 1];
             if (ch >= 'a' && ch <= 'z') ch -= 32;
             switch (ch) {
             case 'A': s = 1; break;

@@ -168,7 +168,8 @@ struct mirfold_ctx {
     std::vector<HBuf> hits_pool;   // pinned hit tables returned by mirfold_free_result
     std::mutex pool_mu;
     int live_results = 0;          // results not yet freed (guarded by pool_mu)
-    bool closed = false;           // mirfold_close() was called; the last mirfold_free_result deletes the context
+    int live_genomes = 0;          // genomes not yet freed (guarded by pool_mu)
+    bool closed = false;           // mirfold_close() was called; the last mirfold_free_result / mirfold_genome_free deletes the context
     double arena_per_nt = 30.0;    // capacity estimates of the shared result buffers, raised when a call overflows them
     double hits_per_nt = 0.20;
 };
@@ -181,6 +182,18 @@ struct mirfold_batch {
     std::vector<std::vector<uint32_t>> shard;      // per device, descending DP cells
     std::vector<uint64_t> raw_off;                 // per record: offset inside its device's buffer
     std::vector<void *> d_raw;                     // per device
+};
+
+// A genome resident in HBM: one copy of the bases per distinct CUDA ordinal of the context.  The handle keeps its
+// context's host bookkeeping alive (live_genomes) and knows its own ordinals, so it may be freed before or after
+// mirfold_close().
+struct mirfold_genome {
+    mirfold_ctx *ctx = nullptr;
+    std::vector<uint64_t> contig_off;    // n_contigs + 1, from 0
+    std::vector<int> ordinal;            // distinct CUDA ordinals ...
+    std::vector<void *> replica;         // ... and the copy of the bases on each
+    std::vector<void *> d_raw;           // per device entry of the context (entries of one ordinal share its replica)
+    std::vector<size_t> budget_taken;    // per device entry: bytes taken off Device::mem_budget while the genome lives
 };
 
 namespace {
@@ -826,9 +839,14 @@ struct DevicePipeline {
         const uint64_t nhits = Ln.nhits;
         const CandArgs &ca = *J.cand;
         unsigned long long *hs = Ln.h_small.as<unsigned long long>();
-        k_gather_bounds<<<(nl + 1 + 255) / 256, 256, 0, hi>>>(tb.tb_base, Ln.hitidx.as<unsigned long long>(), tb.loci, tb.F,
-                                                              Ln.bounds.as<unsigned long long>(), Ln.totals.as<int>(), nl);
-        CK(cudaGetLastError());
+        if (tb.ntb) {
+            k_gather_bounds<<<(nl + 1 + 255) / 256, 256, 0, hi>>>(tb.tb_base, Ln.hitidx.as<unsigned long long>(), tb.loci, tb.F,
+                                                                  Ln.bounds.as<unsigned long long>(), Ln.totals.as<int>(), nl);
+            CK(cudaGetLastError());
+        } else {   // a hairpin-free chunk: hitidx was never scanned, every locus has no hits (as in back())
+            CK(cudaMemsetAsync(Ln.bounds.p, 0, (size_t)(nl + 1) * 8, hi));
+            CK(cudaMemsetAsync(Ln.totals.p, 0, (size_t)nl * 4, hi));
+        }
         CK(Ln.c_counts.ensure((nhits + 2) * 8)); CK(Ln.c_soff.ensure((nhits + 2) * 8));
         CK(Ln.c_lsb.ensure((size_t)(nl + 1) * 8));
         CandLaunch c{};
@@ -865,7 +883,7 @@ struct DevicePipeline {
         c.verdicts = Ln.c_verd.as<mirfold_duplex_verdict>(); c.verdict_mature = Ln.c_vmat.as<unsigned int>();
         c.out_arena = Ln.c_arena.as<char>(); c.out_base = 0; c.structs_out = Ln.c_sout.as<mirfold_structure>();
         CK(launch_cand_finish(c, P.max_Ls + 4, hi));
-        out.st.kernel_launches += 11;   // gather, 2 x classify, locus bounds, 3 x cub scan (2 kernels each), duplex, strings
+        out.st.kernel_launches += tb.ntb ? 11 : 10;   // gather (if any traceback), 2 x classify, locus bounds, 3 x cub scan (2 kernels each), duplex, strings
         CK(cudaEventRecord(Ln.ev[5], hi));
         if (last_chunk) CK(cudaEventRecord(D.ev_last, hi));
         CK(Ln.hc_structs.ensure(ns * sizeof(mirfold_structure) + 16)); CK(Ln.hc_arena.ensure(nb + 16));
@@ -1301,9 +1319,9 @@ void mirfold_close(mirfold_ctx *ctx)
         for (auto &b : ctx->arena_pool) b.release();
         for (auto &b : ctx->hits_pool) b.release();
         ctx->arena_pool.clear(); ctx->hits_pool.clear();
-        del = ctx->live_results == 0;
+        del = ctx->live_results == 0 && ctx->live_genomes == 0;
     }
-    if (del) delete ctx;   // otherwise the last mirfold_free_result() deletes it
+    if (del) delete ctx;   // otherwise the last mirfold_free_result() / mirfold_genome_free() deletes it
 }
 
 int mirfold_fold(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq_off, uint32_t nseq, int span_L, uint32_t flags,
@@ -1397,14 +1415,13 @@ struct CandOwner {
     mirfold_candidates pub;
     CandCollector c;
 };
-}  // namespace
 
-int mirfold_fold_candidates(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq_off, uint32_t nseq, int span_L, uint32_t flags,
-                            const mirfold_region *regions, const mirfold_mature *matures, const uint64_t *mature_off, int minlen,
-                            int minloop, int min_mature_len, int max_mature_len, mirfold_candidates **out)
+// mirfold_fold_candidates / mirfold_fold_candidates_regions: A carries the input (host text or genome regions)
+int fold_candidates_engine(mirfold_ctx *ctx, FoldArgs &A, const mirfold_region *regions, const mirfold_mature *matures,
+                           const uint64_t *mature_off, int minlen, int minloop, int min_mature_len, int max_mature_len,
+                           mirfold_candidates **out)
 {
-    if (!ctx || !out || !seq_off || (!regions && nseq) || !mature_off || (!matures && mature_off[nseq])) return MIRFOLD_ERR_ARG;
-    *out = nullptr;
+    const uint32_t nseq = A.nseq;
     for (uint32_t r = 0; r < nseq; r++) if (mature_off[r + 1] < mature_off[r]) { ctx->last_error = "mature_off is not non-decreasing"; return MIRFOLD_ERR_ARG; }
     std::unique_ptr<CandOwner> O(new CandOwner());
     O->c.struct_begin.assign((size_t)nseq + 1, 0);
@@ -1412,8 +1429,7 @@ int mirfold_fold_candidates(mirfold_ctx *ctx, const char *seqs, const uint64_t *
     CandArgs ca;
     ca.regions = regions; ca.matures = matures; ca.mature_off = mature_off; ca.nseq = nseq;
     ca.minlen = minlen; ca.minloop = minloop; ca.min_mature = min_mature_len; ca.max_mature = max_mature_len;
-    FoldArgs A;
-    A.seqs = seqs; A.seq_off = seq_off; A.nseq = nseq; A.span_L = span_L; A.flags = flags; A.sink = SINK_CAND;
+    A.sink = SINK_CAND;
     A.cand = &ca; A.collect = &O->c;
     uint64_t nhits = 0;
     A.nhits_out = &nhits;
@@ -1436,6 +1452,176 @@ int mirfold_fold_candidates(mirfold_ctx *ctx, const char *seqs, const uint64_t *
     p.stats = st;
     *out = &O.release()->pub;
     return MIRFOLD_OK;
+}
+
+// Genome regions -> the engine's inputs, in one pass: a synthetic seq_off from the clipped lengths (shard plan, chunking
+// and every per-record table work from it unchanged) and per record raw_off = contig start + start - 1 into the device
+// replica, | MF_RAW_REVERSE on the minus strand.  Clipping is samtools faidx's on "seqid:start-(end-1)" (FastaIndex.fetch).
+struct RegionInput {
+    std::vector<uint64_t> seq_off, raw_off;
+    std::vector<mirfold_region> cand;   // the unclipped (start, end): the region the duplex checks see
+};
+int region_input(mirfold_ctx *ctx, const mirfold_genome *g, const mirfold_genome_region *reg, uint32_t nseq, bool cand, RegionInput &I)
+{
+    if (!ctx || !g || (!reg && nseq) || ctx->closed) return MIRFOLD_ERR_ARG;
+    if (g->ctx != ctx) { ctx->last_error = "the genome belongs to another context"; return MIRFOLD_ERR_ARG; }
+    const int64_t nc = (int64_t)g->contig_off.size() - 1;
+    I.seq_off.resize((size_t)nseq + 1);
+    I.raw_off.resize((size_t)nseq + 1);
+    if (cand) I.cand.resize((size_t)nseq + 1);
+    I.seq_off[0] = 0;
+    uint64_t acc = 0;
+    char msg[128];
+    for (uint32_t r = 0; r < nseq; r++) {
+        const mirfold_genome_region &x = reg[r];
+        if (x.strand != '+' && x.strand != '-') {
+            snprintf(msg, sizeof msg, "region %u: strand %d is neither '+' nor '-'", r, x.strand);
+            ctx->last_error = msg;
+            return MIRFOLD_ERR_ARG;
+        }
+        if (x.contig < -1 || x.contig >= nc) {
+            snprintf(msg, sizeof msg, "region %u: contig %d out of range [-1, %lld)", r, x.contig, (long long)nc);
+            ctx->last_error = msg;
+            return MIRFOLD_ERR_ARG;
+        }
+        uint64_t len = 0, raw = 0;
+        if (x.contig >= 0) {
+            const uint64_t base = g->contig_off[x.contig], clen = g->contig_off[x.contig + 1] - base;
+            const int64_t s = std::max<int64_t>(x.start, 1), e = std::min<int64_t>((int64_t)x.end - 1, (int64_t)clen);
+            if (s <= e) { len = (uint64_t)(e - s + 1); raw = base + (uint64_t)(s - 1); }
+        }
+        I.raw_off[r] = raw | (x.strand == '-' ? MF_RAW_REVERSE : 0ULL);
+        acc += len;
+        I.seq_off[r + 1] = acc;
+        if (cand) I.cand[r] = mirfold_region{x.start, x.end};
+    }
+    return MIRFOLD_OK;
+}
+}  // namespace
+
+int mirfold_fold_candidates(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq_off, uint32_t nseq, int span_L, uint32_t flags,
+                            const mirfold_region *regions, const mirfold_mature *matures, const uint64_t *mature_off, int minlen,
+                            int minloop, int min_mature_len, int max_mature_len, mirfold_candidates **out)
+{
+    if (!ctx || !out || !seq_off || (!regions && nseq) || !mature_off || (!matures && mature_off[nseq])) return MIRFOLD_ERR_ARG;
+    *out = nullptr;
+    FoldArgs A;
+    A.seqs = seqs; A.seq_off = seq_off; A.nseq = nseq; A.span_L = span_L; A.flags = flags;
+    return fold_candidates_engine(ctx, A, regions, matures, mature_off, minlen, minloop, min_mature_len, max_mature_len, out);
+}
+
+int mirfold_genome_upload(mirfold_ctx *ctx, const char *seq, const uint64_t *contig_off, uint32_t n_contigs, mirfold_genome **out)
+{
+    if (!ctx || !out || !contig_off || ctx->closed) return MIRFOLD_ERR_ARG;
+    *out = nullptr;
+    for (uint32_t c = 0; c < n_contigs; c++)
+        if (contig_off[c + 1] < contig_off[c]) { ctx->last_error = "contig_off is not non-decreasing"; return MIRFOLD_ERR_ARG; }
+    const uint64_t bytes = contig_off[n_contigs] - contig_off[0];
+    if (!seq && bytes) return MIRFOLD_ERR_ARG;
+    std::unique_ptr<mirfold_genome> G(new mirfold_genome());
+    G->ctx = ctx;
+    G->contig_off.resize((size_t)n_contigs + 1);
+    for (uint32_t c = 0; c <= n_contigs; c++) G->contig_off[c] = contig_off[c] - contig_off[0];
+    const size_t nd = ctx->devs.size();
+    G->d_raw.assign(nd, nullptr);
+    G->budget_taken.assign(nd, 0);
+    cudaError_t e = cudaSuccess;
+    for (size_t k = 0; k < nd && e == cudaSuccess; k++) {
+        Device &D = ctx->devs[k];
+        const size_t j = std::find(G->ordinal.begin(), G->ordinal.end(), D.id) - G->ordinal.begin();
+        if (j == G->ordinal.size()) {
+            void *p = nullptr;
+            e = cudaSetDevice(D.id);
+            if (e == cudaSuccess) e = cudaMalloc(&p, (size_t)bytes + 16);
+            if (e != cudaSuccess) break;
+            G->ordinal.push_back(D.id);
+            G->replica.push_back(p);
+            if (bytes) e = cudaMemcpyAsync(p, seq + contig_off[0], (size_t)bytes, cudaMemcpyHostToDevice, D.lane[0].s_lo);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(D.lane[0].s_lo);
+        }
+        G->d_raw[k] = G->replica[j];
+    }
+    if (e != cudaSuccess) {
+        ctx->last_error = std::string("genome upload: ") + cudaGetErrorString(e);
+        cudaGetLastError();
+        for (size_t j = 0; j < G->ordinal.size(); j++) { cudaSetDevice(G->ordinal[j]); cudaFree(G->replica[j]); }
+        return e == cudaErrorMemoryAllocation ? MIRFOLD_ERR_NOMEM : MIRFOLD_ERR_CUDA;
+    }
+    // the lanes' budget was set from free HBM at mirfold_open; the replica now occupies part of it (split between the entries
+    // of one ordinal like the budget itself).  An explicit MIRFOLD_MEM_BUDGET_MB is taken as given.
+    std::lock_guard<std::mutex> lk(ctx->pool_mu);
+    if (!getenv("MIRFOLD_MEM_BUDGET_MB"))
+        for (size_t k = 0; k < nd; k++) {
+            Device &D = ctx->devs[k];
+            size_t share = 0;
+            for (const Device &o : ctx->devs) share += o.id == D.id;
+            const size_t keep = std::min(D.mem_budget, (size_t)256 << 20);
+            G->budget_taken[k] = std::min((size_t)bytes / share, D.mem_budget - keep);
+            D.mem_budget -= G->budget_taken[k];
+        }
+    ctx->live_genomes++;
+    *out = G.release();
+    return MIRFOLD_OK;
+}
+
+void mirfold_genome_free(mirfold_genome *g)
+{
+    if (!g) return;
+    for (size_t j = 0; j < g->ordinal.size(); j++) { cudaSetDevice(g->ordinal[j]); cudaFree(g->replica[j]); }
+    mirfold_ctx *ctx = g->ctx;
+    bool del;
+    {
+        std::lock_guard<std::mutex> lk(ctx->pool_mu);
+        if (!ctx->closed)
+            for (size_t k = 0; k < ctx->devs.size() && k < g->budget_taken.size(); k++) ctx->devs[k].mem_budget += g->budget_taken[k];
+        ctx->live_genomes--;
+        del = ctx->closed && ctx->live_results == 0 && ctx->live_genomes == 0;
+    }
+    delete g;
+    if (del) delete ctx;
+}
+
+int mirfold_fold_regions(mirfold_ctx *ctx, const mirfold_genome *genome, const mirfold_genome_region *regions, uint32_t nseq,
+                         int span_L, uint32_t flags, mirfold_result **out)
+{
+    if (!out) return MIRFOLD_ERR_ARG;
+    *out = nullptr;
+    RegionInput I;
+    const int rc = region_input(ctx, genome, regions, nseq, false, I);
+    if (rc != MIRFOLD_OK) return rc;
+    FoldArgs A;
+    A.seq_off = I.seq_off.data(); A.nseq = nseq; A.span_L = span_L; A.flags = flags; A.sink = SINK_SHARED;
+    A.d_raw = &genome->d_raw; A.raw_off = I.raw_off.data();
+    return fold_engine(ctx, A, out, nullptr);
+}
+
+int mirfold_fold_regions_stream(mirfold_ctx *ctx, const mirfold_genome *genome, const mirfold_genome_region *regions, uint32_t nseq,
+                                int span_L, uint32_t flags, mirfold_chunk_fn fn, void *user, mirfold_stats *stats)
+{
+    if (!fn) return MIRFOLD_ERR_ARG;
+    RegionInput I;
+    const int rc = region_input(ctx, genome, regions, nseq, false, I);
+    if (rc != MIRFOLD_OK) return rc;
+    FoldArgs A;
+    A.seq_off = I.seq_off.data(); A.nseq = nseq; A.span_L = span_L; A.flags = flags; A.sink = SINK_STREAM;
+    A.fn = fn; A.user = user;
+    A.d_raw = &genome->d_raw; A.raw_off = I.raw_off.data();
+    return fold_engine(ctx, A, nullptr, stats);
+}
+
+int mirfold_fold_candidates_regions(mirfold_ctx *ctx, const mirfold_genome *genome, const mirfold_genome_region *regions, uint32_t nseq,
+                                    int span_L, uint32_t flags, const mirfold_mature *matures, const uint64_t *mature_off, int minlen,
+                                    int minloop, int min_mature_len, int max_mature_len, mirfold_candidates **out)
+{
+    if (!out || !mature_off || (!matures && mature_off[nseq])) return MIRFOLD_ERR_ARG;
+    *out = nullptr;
+    RegionInput I;
+    const int rc = region_input(ctx, genome, regions, nseq, true, I);
+    if (rc != MIRFOLD_OK) return rc;
+    FoldArgs A;
+    A.seq_off = I.seq_off.data(); A.nseq = nseq; A.span_L = span_L; A.flags = flags;
+    A.d_raw = &genome->d_raw; A.raw_off = I.raw_off.data();
+    return fold_candidates_engine(ctx, A, I.cand.data(), matures, mature_off, minlen, minloop, min_mature_len, max_mature_len, out);
 }
 
 void mirfold_free_candidates(mirfold_candidates *c)
@@ -1483,7 +1669,7 @@ void mirfold_free_result(mirfold_result *res)
         pool_give(ctx, ctx->arena_pool, R->arena);
         pool_give(ctx, ctx->hits_pool, R->hits);
         ctx->live_results--;
-        del = ctx->closed && ctx->live_results == 0;
+        del = ctx->closed && ctx->live_results == 0 && ctx->live_genomes == 0;
     }
     R->arena.release();
     R->hits.release();

@@ -70,7 +70,7 @@ struct LocusDesc {
     unsigned long long seq_off;   // into codes / F (elements)
     unsigned long long band_off;  // into C / M (elements)
     unsigned long long ring_off;  // into ring scratch (elements)
-    unsigned long long raw_off;   // into the raw ASCII buffer
+    unsigned long long raw_off;   // into the raw ASCII buffer; | MF_RAW_REVERSE: fold the reverse complement
     int n;
     int Ls;      // L* = min(L, n)
     int dmax;    // min(Ls, n-1)
@@ -85,6 +85,8 @@ struct LocusDesc {
     int tile_step;           // rows owned per tile
     unsigned int tile_rcp;   // ceil(2^32 / tile_step): (i-1)/tile_step == __umulhi(i-1, tile_rcp)
 };
+// raw_off flag of a minus-strand genome region (mirfold_fold_regions): k_prepare reads the locus backwards and complements it
+#define MF_RAW_REVERSE (1ULL << 63)
 #define MF_TILE_LEN 608
 #define MF_TILE_LEN_BIG 864   /* the largest shared-memory bucket: one 1024-thread CTA per SM (155 KB of rings) */
 

@@ -69,6 +69,18 @@ class FastaIndex:
             return self.fetch(region, 1, 1 << 62)
         return self.fetch(seqid, start, end)
 
+    def packed(self):
+        """(names, bases, offsets): the contig names in file order, all their bases concatenated (bytes, exactly as
+        stored) and uint64 offsets with contig k at bases[offsets[k]:offsets[k + 1]] -- the upload format of
+        MirFold.upload_genome / mirfold_genome_upload.  fetch(names[k], s, e) == bases[offsets[k] + s - 1:...] after the
+        same clipping."""
+        import numpy as np
+        names = list(self._order)
+        off = np.zeros(len(names) + 1, np.uint64)
+        if names:
+            off[1:] = np.cumsum([len(self._seq[n]) for n in names], dtype=np.uint64)
+        return names, b"".join(self._seq[n] for n in names), off
+
     def extend_region_sequence(self, seqid, extendregion):
         """Sequence of a half-open extend region [start, end) as dump_piece cuts it (:1097-1105)."""
         return self.fetch(seqid, extendregion[0], extendregion[1] - 1)

@@ -75,6 +75,11 @@ class FoldResult:
         (miR_PREFeR.py:1566-1589)."""
         return classify_result(self._lib, self._ptr, self.nseq, self.arena, minlen, minloop)
 
+    def set_inputs(self, buf, off):
+        """The packed sequences the result was folded from, for record_blocks() of a result that was folded from genome
+        coordinates (Genome.fold_regions): the caller extracts them on the host when it wants the RNALfold text."""
+        self._inputs = (np.ascontiguousarray(buf, np.uint8), np.ascontiguousarray(off, np.uint64))
+
     def record_blocks(self):
         """RNALfold's output of every record (hit lines, converted sequence, total line) as one bytes object
         plus nseq+1 offsets -- formatted natively by mirfold_format_records() (include/mirfold.h)."""
@@ -205,6 +210,39 @@ class FoldChunk:
 
 MATURE_DTYPE = np.dtype([("start", "<i4"), ("end", "<i4"), ("strand", "<i4"), ("depth", "<i4")])
 REGION_DTYPE = np.dtype([("start", "<i4"), ("end", "<i4")])
+# mirfold_genome_region: contig index (-1 = not in the FASTA), [start, end) as dump_piece prints it, strand ord('+') / ord('-')
+GENOME_REGION_DTYPE = np.dtype([("contig", "<i4"), ("start", "<i4"), ("end", "<i4"), ("strand", "<i4")])
+
+
+def _mature_array(matures):
+    """MATURE_DTYPE array of matures given as such an array or as (start, end, strand_char, depth) tuples."""
+    if isinstance(matures, np.ndarray) and matures.dtype == MATURE_DTYPE:
+        return np.ascontiguousarray(matures)
+    mat = np.zeros(len(matures), MATURE_DTYPE)
+    for k, m in enumerate(matures):
+        mat[k] = (m[0], m[1], ord(m[2]) if isinstance(m[2], str) else int(m[2]), m[3] if len(m) > 3 else 0)
+    return mat
+
+
+def _stream(callback, call):
+    """Run call(fn, stats) with fn a C trampoline handing FoldChunks to callback; an exception inside the callback
+    aborts the fold (the library returns MIRFOLD_ERR_CALLBACK) and is re-raised here.  Returns (rc, stats dict)."""
+    err = []
+
+    def tramp(_user, cptr):
+        try:
+            callback(FoldChunk(cptr.contents))
+            return 0
+        except BaseException as e:   # noqa: BLE001 -- must not propagate through the C frames
+            err.append(e)
+            return 1
+
+    fn = _lib.CHUNK_FN(tramp)
+    st = _lib.Stats()
+    rc = call(fn, st)
+    if err:
+        raise err[0]
+    return rc, st.as_dict()
 
 
 class Candidates:
@@ -289,6 +327,106 @@ class Batch:
 
     def __exit__(self, *a):
         self.close()
+
+
+class Genome:
+    """A FASTA resident in HBM on every device of its context (mirfold_genome_*): records are given as coordinates
+    (GENOME_REGION_DTYPE rows) and the extend regions are cut, reverse-complemented and encoded on the device -- what
+    dump_piece does with `samtools faidx` per record (miR_PREFeR.py:1097-1108, :1131, :1177), without the strings.
+    Results equal those of the text entry points on FastaIndex.extend_region_sequence + records.fold_sequence."""
+
+    def __init__(self, owner, ptr, index, names, off):
+        self._owner, self._ptr, self.index = owner, ptr, index
+        self.names = list(names)
+        self.lengths = np.diff(off.astype(np.int64))
+        self.contig_ids = {n: k for k, n in enumerate(self.names)}
+
+    def contig_index(self, seqid):
+        """Index of seqid in the upload, -1 for a seqid the FASTA does not have (an empty record, like samtools)."""
+        return self.contig_ids.get(seqid, -1)
+
+    def regions(self, seqids, starts, ends, strands):
+        """GENOME_REGION_DTYPE array from per-record seqids, [start, end) and '+' / '-' strands."""
+        reg = np.zeros(len(seqids), GENOME_REGION_DTYPE)
+        reg["contig"] = [self.contig_ids.get(s, -1) for s in seqids]
+        reg["start"], reg["end"] = starts, ends
+        reg["strand"] = [ord(s) if isinstance(s, str) and len(s) == 1 else 0 for s in strands]
+        return reg
+
+    def sequence(self, contig, start, end, strand):
+        """The folded sequence of one region, extracted on the host (FastaIndex + the reference's reverse complement)."""
+        from .records import get_reverse_complement
+        if contig < 0:
+            return ""
+        s = self.index.extend_region_sequence(self.names[contig], (int(start), int(end)))
+        return get_reverse_complement(s) if strand in (45, "-") else s
+
+    @staticmethod
+    def _table(regions):
+        if isinstance(regions, np.ndarray) and regions.dtype == GENOME_REGION_DTYPE:
+            return np.ascontiguousarray(regions)
+        ra = np.asarray(regions, np.int64).reshape(-1, 4)
+        reg = np.zeros(len(ra), GENOME_REGION_DTYPE)
+        for k, name in enumerate(GENOME_REGION_DTYPE.names):
+            reg[name] = ra[:, k]
+        return reg
+
+    def _args(self, regions):
+        if not self._ptr:
+            raise MirfoldError(-3, "the genome was closed")
+        reg = self._table(regions)
+        return reg, (self._owner._ctx, self._ptr, reg.ctypes.data_as(C.c_void_p), len(reg))
+
+    def fold_regions(self, regions, span, flags=0):
+        """mirfold_fold_regions(): MirFold.fold_packed() of the regions' sequences.  record_blocks() of the result needs
+        the sequences: FoldResult.set_inputs(*MirFold.pack([...Genome.sequence...]))."""
+        reg, head = self._args(regions)
+        res = C.POINTER(_lib.Result)()
+        rc = self._owner._lib.mirfold_fold_regions(*head, int(span), int(flags), C.byref(res))
+        if rc != 0:
+            self._owner._raise(rc)
+        return FoldResult(self._owner._lib, res, len(reg), owner=self._owner)
+
+    def fold_regions_stream(self, regions, span, callback, flags=0):
+        """mirfold_fold_regions_stream(): MirFold.fold_stream() of the regions' sequences.  Returns the stats dict."""
+        reg, head = self._args(regions)
+        rc, st = _stream(callback, lambda fn, st: self._owner._lib.mirfold_fold_regions_stream(
+            *head, int(span), int(flags), fn, None, C.byref(st)))
+        if rc != 0:
+            self._owner._raise(rc)
+        return st
+
+    def fold_candidates(self, regions, span, matures, mature_off, minlen=55, minloop=3, min_mature_len=18, max_mature_len=24,
+                        flags=0):
+        """mirfold_fold_candidates_regions(): MirFold.fold_candidates() of the regions' sequences, with each record's
+        (start, end) as its duplex region."""
+        reg, head = self._args(regions)
+        mat = _mature_array(matures)
+        moff = np.ascontiguousarray(mature_off, np.uint64)
+        res = C.POINTER(_lib.Candidates)()
+        rc = self._owner._lib.mirfold_fold_candidates_regions(*head, int(span), int(flags), mat.ctypes.data_as(C.c_void_p),
+                                                              moff.ctypes.data_as(C.POINTER(C.c_uint64)), int(minlen), int(minloop),
+                                                              int(min_mature_len), int(max_mature_len), C.byref(res))
+        if rc != 0:
+            self._owner._raise(rc)
+        return Candidates(self._owner._lib, res, mat, moff)
+
+    def close(self):
+        if self._ptr:
+            self._owner._lib.mirfold_genome_free(self._ptr)
+            self._ptr = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def plan_shards(lengths, span, n_shards):
@@ -376,25 +514,12 @@ class MirFold:
         FoldChunk.records names the input records.  Returns the call's stats dict."""
         buf = np.ascontiguousarray(buf, np.uint8)
         off = np.ascontiguousarray(off, np.uint64)
-        err = []
-
-        def tramp(_user, cptr):
-            try:
-                callback(FoldChunk(cptr.contents))
-                return 0
-            except BaseException as e:   # noqa: BLE001 -- must not propagate through the C frames
-                err.append(e)
-                return 1
-
-        fn = _lib.CHUNK_FN(tramp)
-        st = _lib.Stats()
-        rc = self._lib.mirfold_fold_stream(self._ctx, buf.ctypes.data_as(C.c_void_p), off.ctypes.data_as(C.POINTER(C.c_uint64)),
-                                           len(off) - 1, int(span), int(flags), fn, None, C.byref(st))
-        if err:
-            raise err[0]
+        rc, st = _stream(callback, lambda fn, st: self._lib.mirfold_fold_stream(
+            self._ctx, buf.ctypes.data_as(C.c_void_p), off.ctypes.data_as(C.POINTER(C.c_uint64)), len(off) - 1, int(span),
+            int(flags), fn, None, C.byref(st)))
         if rc != 0:
             self._raise(rc)
-        return st.as_dict()
+        return st
 
     def fold_candidates(self, buf, off, span, regions, matures, mature_off, minlen=55, minloop=3, min_mature_len=18,
                         max_mature_len=24, flags=0):
@@ -409,12 +534,7 @@ class MirFold:
         if nseq:
             ra = np.asarray(regions, np.int64).reshape(nseq, 2)
             reg["start"], reg["end"] = ra[:, 0], ra[:, 1]
-        if isinstance(matures, np.ndarray) and matures.dtype == MATURE_DTYPE:
-            mat = np.ascontiguousarray(matures)
-        else:
-            mat = np.zeros(len(matures), MATURE_DTYPE)
-            for k, m in enumerate(matures):
-                mat[k] = (m[0], m[1], ord(m[2]) if isinstance(m[2], str) else int(m[2]), m[3] if len(m) > 3 else 0)
+        mat = _mature_array(matures)
         moff = np.ascontiguousarray(mature_off, np.uint64)
         res = C.POINTER(_lib.Candidates)()
         rc = self._lib.mirfold_fold_candidates(self._ctx, buf.ctypes.data_as(C.c_void_p), off.ctypes.data_as(C.POINTER(C.c_uint64)),
@@ -435,6 +555,16 @@ class MirFold:
         if rc != 0:
             self._raise(rc)
         return Batch(self, ptr, len(off) - 1, (buf, off))
+
+    def upload_genome(self, index):
+        """mirfold_genome_upload(): keep the FASTA of `index` (a FastaIndex) in HBM on every device of this context.
+        Returns a Genome (a context manager; close() frees the device copies)."""
+        names, bases, off = index.packed()
+        ptr = C.c_void_p()
+        rc = self._lib.mirfold_genome_upload(self._ctx, bases, off.ctypes.data_as(C.POINTER(C.c_uint64)), len(names), C.byref(ptr))
+        if rc != 0:
+            self._raise(rc)
+        return Genome(self, ptr, index, names, off)
 
     def fold(self, seqs, span, flags=0):
         buf, off = self.pack(seqs)

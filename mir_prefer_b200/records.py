@@ -109,9 +109,10 @@ def write_fasta(records, path):
 class RecordFold:
     """Folded records: structures for the predict stage and, on request, the RNALfold text."""
 
-    def __init__(self, records, result):
+    def __init__(self, records, result, seq_of=None):
         self.records = records
         self.result = result
+        self._seq_of = seq_of or _oriented_sequence   # genome records: extracted on the host (only the text needs it)
 
     def structures(self, minlen, minloop=3, native=True):
         """Generator of (which, peak, [(norm_energy, fold_start, ss, sstype)]) -- one per record,
@@ -133,7 +134,7 @@ class RecordFold:
         out = []
         for r, rec in enumerate(self.records):
             out.append(header_line(rec) + "\n")
-            seq = _oriented_sequence(rec)
+            seq = self._seq_of(rec)
             if seq.split(None, 1)[:1] == []:      # blank line: echoed, not folded
                 out.append(seq + "\n")
             else:
@@ -156,13 +157,49 @@ class RecordFold:
         self.close()
 
 
-def candidates_of_records(mf, records, span, minlen=55, minloop=3, min_mature_len=18, max_mature_len=24):
+_STRAND_CODE = {"+": 43, "-": 45}
+
+
+def region_table(genome, records):
+    """GENOME_REGION_DTYPE rows of the records' (seqid, region, strand) against `genome` (fold.Genome).  A seqid the
+    genome does not have becomes contig -1 (an empty record); a strand other than '+' / '-' is rejected by the library."""
+    import itertools
+    import numpy as np
+    from .fold import GENOME_REGION_DTYPE
+    ids = genome.contig_ids
+    flat = np.fromiter(itertools.chain.from_iterable((ids.get(r.seqid, -1), r.region[0], r.region[1], _STRAND_CODE.get(r.strand, 0))
+                                                     for r in records), np.int32, count=4 * len(records))
+    return flat.view(GENOME_REGION_DTYPE)
+
+
+def _mature_table(records):
+    """MATURE_DTYPE array of all records' matures, in record order, and the nseq+1 offsets."""
+    import itertools
+    import numpy as np
+    from .fold import MATURE_DTYPE
+    moff = np.zeros(len(records) + 1, np.uint64)
+    moff[1:] = np.cumsum(np.fromiter((len(r.matures) for r in records), np.int64, count=len(records)), dtype=np.uint64)
+    n = int(moff[-1])
+    flat = np.fromiter(itertools.chain.from_iterable((m[0], m[1], ord(m[2]), m[3] if len(m) > 3 else 0) for r in records for m in r.matures),
+                       np.int32, count=4 * n)
+    return flat.view(MATURE_DTYPE), moff
+
+
+def candidates_of_records(mf, records, span, minlen=55, minloop=3, min_mature_len=18, max_mature_len=24, genome=None):
     """Records -> (ss_records, DuplexTable) in ONE fused device pass (mirfold_fold_candidates): the fold, the candidate
     structures of get_structures_next_extendregion (miR_PREFeR.py:1566-1589) and get_maturestar_info (:1876-1999) for every
-    (structure, mature) pair.  ss_records is what filter_next_loci consumes: (which, peak, structures) per record."""
+    (structure, mature) pair.  ss_records is what filter_next_loci consumes: (which, peak, structures) per record.
+    genome (fold.Genome, from mf.upload_genome): every record is folded from its coordinates in the resident genome
+    (mirfold_fold_candidates_regions) and its `seq` may be None; the result is the same."""
     import numpy as np
     from .predict import DuplexTable
     records = list(records)
+    if genome is not None:
+        matures, moff = _mature_table(records)
+        cand = genome.fold_candidates(region_table(genome, records), span, matures, moff, minlen, minloop, min_mature_len,
+                                      max_mature_len)
+        ss_records = [(rec.tag, "%s-%s" % (rec.locus[0], rec.locus[1]), cand.structures(k)) for k, rec in enumerate(records)]
+        return ss_records, DuplexTable.from_candidates(cand, records), cand
     seqs = [_oriented_sequence(r) for r in records]
     buf, off = mf.pack(seqs)
     matures, moff = [], [0]
@@ -175,11 +212,15 @@ def candidates_of_records(mf, records, span, minlen=55, minloop=3, min_mature_le
     return ss_records, DuplexTable.from_candidates(cand, records), cand
 
 
-def fold_records(mf, records, span):
+def fold_records(mf, records, span, genome=None):
     """Fold LocusRecords on the device.  Identical oriented sequences (the reference writes
     duplicated records for both-strand L/R loci, SURVEY App. C) are folded once; record count and
-    order are preserved because the predict stage pairs records positionally (:2364-2399)."""
+    order are preserved because the predict stage pairs records positionally (:2364-2399).
+    genome (fold.Genome): every record is folded from its coordinates (mirfold_fold_regions) and its `seq` may be None;
+    records with the same (contig, clipped start, clipped end, strand) are folded once."""
     records = list(records)
+    if genome is not None:
+        return _fold_records_genome(records, span, genome)
     seqs = [_oriented_sequence(r) for r in records]
     first, uniq, index = {}, [], []
     for s in seqs:
@@ -190,12 +231,30 @@ def fold_records(mf, records, span):
     return RecordFold(records, _Replicated(mf.fold(uniq, span), index))
 
 
+def _fold_records_genome(records, span, genome):
+    import numpy as np
+    reg = region_table(genome, records)
+    contig = reg["contig"].astype(np.int64)
+    clen = np.where(contig >= 0, genome.lengths[np.maximum(contig, 0)] if len(genome.lengths) else 0, 0)
+    s = np.maximum(reg["start"].astype(np.int64), 1)
+    e = np.minimum(reg["end"].astype(np.int64) - 1, clen)
+    empty = (contig < 0) | (s > e)
+    key = np.stack([np.where(empty, -1, contig), np.where(empty, 0, s), np.where(empty, 0, e), reg["strand"]], axis=1)
+    _, first, index = np.unique(key, axis=0, return_index=True, return_inverse=True)
+    ureg = reg[first]                   # one representative record per distinct folded sequence
+    res = genome.fold_regions(ureg, span)
+    host = lambda: [genome.sequence(*(int(x) for x in r)) for r in ureg]   # noqa: E731 -- RNALfold text only
+    seq_of = lambda rec: genome.sequence(genome.contig_index(rec.seqid), rec.region[0], rec.region[1], rec.strand)   # noqa: E731
+    return RecordFold(records, _Replicated(res, index.reshape(-1).tolist(), host_seqs=host), seq_of)
+
+
 class _Replicated:
     """View of a FoldResult through a record -> unique-sequence index."""
 
-    def __init__(self, result, index):
+    def __init__(self, result, index, host_seqs=None):
         self._res, self._index = result, index
         self.stats = result.stats
+        self._host_seqs = host_seqs     # genome results: the unique sequences, extracted on the host for record_blocks()
 
     def hits(self, r):
         return self._res.hits(self._index[r])
@@ -204,6 +263,10 @@ class _Replicated:
         return self._res.total(self._index[r])
 
     def record_blocks(self):
+        if self._host_seqs is not None:
+            from .fold import MirFold
+            self._res.set_inputs(*MirFold.pack(self._host_seqs()))
+            self._host_seqs = None
         return self._res.record_blocks()
 
     def classify(self, minlen, minloop=3):

@@ -352,6 +352,36 @@ int mirfold_fold_candidates_regions(mirfold_ctx *ctx, const mirfold_genome *geno
                                     int max_mature_len, mirfold_candidates **out);
 void mirfold_free_candidates(mirfold_candidates *c);
 
+/* ---- MFE significance against shuffled sequences (randfold's test, Bonnet et al. 2004) ----
+ * For every record: its total MFE (the " (%6.2f)" total line) and that of n_shuffles shuffles of it, folded on the
+ * device.  Shuffles act on the sequence as it is folded (upper-case, T -> U) and treat every distinct byte as a symbol:
+ *   MIRFOLD_SHUFFLE_MONO  Fisher-Yates: keeps the multiset of symbols;
+ *   MIRFOLD_SHUFFLE_DI    Altschul-Erickson (uShuffle, k = 2): keeps every dinucleotide count and the first and last
+ *                         symbols, uniform over the sequences that do; at most 16 distinct symbols per record.
+ * Replicate k of record r is a pure function of (seed, r, k) (splitmix64, csrc/shuffle_rng.cuh), so results do not
+ * depend on the devices, chunks or rounds.  span_L = 0 folds every record globally (at a span of at least its length,
+ * so native_dcal == mirfold_fold's total at span_L = n; records must then be at most 4096 nt); otherwise 5..4096.
+ * Records shorter than 5 nt have native 0, every shuffle 0 and n_le = n_shuffles.  The fold stops after the f3 scan
+ * (no traceback) and downloads 4 bytes per folded sequence; stats count every folded nt and cell, natives included.
+ * Derived: p = (n_le + 1) / (n_shuffles + 1), mean = sum / K, sd^2 = sumsq / K - mean^2, z = (native - mean) / sd.
+ * MIRFOLD_ERR_ARG, and no output, for n_shuffles = 0, an unknown mode, a closed context, a span outside the range
+ * above or a record with more than 16 symbols in dinucleotide mode. */
+#define MIRFOLD_SHUFFLE_MONO 1
+#define MIRFOLD_SHUFFLE_DI 2
+typedef struct mirfold_shuffle_stat {
+    int32_t native_dcal;   /* total MFE of the unshuffled record (== mirfold_fold's total at this span) */
+    uint32_t n_le;         /* shuffles whose total MFE <= native_dcal                                  */
+    int64_t sum_dcal;      /* sum of the shuffles' totals                                              */
+    int64_t sumsq_dcal;    /* sum of their squares                                                     */
+} mirfold_shuffle_stat;
+int mirfold_shuffle_test(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq_off, uint32_t nseq, int span_L /* 0 = global */,
+                         uint32_t flags, int mode, uint32_t n_shuffles, uint64_t seed,
+                         mirfold_shuffle_stat *out /* nseq, caller-allocated */, mirfold_stats *stats /* may be NULL */);
+/* Inspection / test hook: replicate `replicate` of every record as mirfold_shuffle_test folds it, generated by the device
+ * kernel on device 0 of ctx.  Record r's shuffle is written to out[seq_off[r] .. seq_off[r+1]) (converted letters). */
+int mirfold_shuffle_sequences(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq_off, uint32_t nseq, int mode,
+                              uint64_t seed, uint32_t replicate, char *out /* seq_off[nseq] bytes */);
+
 #ifdef __cplusplus
 }
 #endif

@@ -88,6 +88,10 @@ class Candidates(C.Structure):
                 ("stats", Stats)]
 
 
+class ShuffleStat(C.Structure):
+    _fields_ = [("native_dcal", C.c_int32), ("n_le", C.c_uint32), ("sum_dcal", C.c_int64), ("sumsq_dcal", C.c_int64)]
+
+
 class FillPlan(C.Structure):
     _fields_ = [("kernel", C.c_int32), ("stride", C.c_int32), ("tile_len", C.c_int32), ("tile_step", C.c_int32),
                 ("n_units", C.c_int32), ("dmax", C.c_int32), ("band_cells", C.c_uint64)]
@@ -100,7 +104,7 @@ EXPORTS = ["mirfold_open", "mirfold_close", "mirfold_fold", "mirfold_fold_device
            "mirfold_classify", "mirfold_free_structures", "mirfold_fold_stream", "mirfold_batch_upload", "mirfold_batch_fold",
            "mirfold_batch_free", "mirfold_plan_shards", "mirfold_int_peak2", "mirfold_fold_candidates", "mirfold_free_candidates", "mirfold_fold_text", "mirfold_plan_fill_units",
            "mirfold_genome_upload", "mirfold_genome_free", "mirfold_fold_regions", "mirfold_fold_regions_stream",
-           "mirfold_fold_candidates_regions"]
+           "mirfold_fold_candidates_regions", "mirfold_shuffle_test", "mirfold_shuffle_sequences"]
 
 _lib = None
 
@@ -193,5 +197,12 @@ def load():
                                                         C.POINTER(C.c_uint64), C.c_int, C.c_int, C.c_int, C.c_int,
                                                         C.POINTER(C.POINTER(Candidates))]
         lib.mirfold_fold_candidates_regions.restype = C.c_int
+    if hasattr(lib, "mirfold_shuffle_test") or not os.environ.get("MIRFOLD_LIB_PATH"):   # an A/B build may predate the shuffle test
+        lib.mirfold_shuffle_test.argtypes = [vp, C.c_void_p, C.POINTER(C.c_uint64), C.c_uint32, C.c_int, C.c_uint32, C.c_int,
+                                             C.c_uint32, C.c_uint64, C.c_void_p, C.POINTER(Stats)]
+        lib.mirfold_shuffle_test.restype = C.c_int
+        lib.mirfold_shuffle_sequences.argtypes = [vp, C.c_void_p, C.POINTER(C.c_uint64), C.c_uint32, C.c_int, C.c_uint64, C.c_uint32,
+                                                  C.c_void_p]
+        lib.mirfold_shuffle_sequences.restype = C.c_int
     _lib = lib
     return lib

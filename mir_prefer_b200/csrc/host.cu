@@ -26,6 +26,7 @@
 
 #include "../../include/mirfold.h"
 #include "mirfold_internal.cuh"
+#include "shuffle_rng.cuh"
 
 #define MIRFOLD_VERSION "0.2.0"
 
@@ -146,11 +147,13 @@ struct Device {
     cudaEvent_t ev_first = nullptr, ev_last = nullptr;
     DBuf duplex_arena, duplex_q, duplex_v;   // mirfold_duplex scratch
     DBuf cand_regions, cand_matures, cand_moff;   // the call's records (mirfold_fold_candidates)
+    DBuf shuf_in, shuf_off, shuf_items, shuf_raw, shuf_scr, shuf_fail;   // mirfold_shuffle_test: records, one round's replicates
     void release()
     {
         lane[0].release(); lane[1].release();
         duplex_arena.release(); duplex_q.release(); duplex_v.release();
         cand_regions.release(); cand_matures.release(); cand_moff.release();
+        shuf_in.release(); shuf_off.release(); shuf_items.release(); shuf_raw.release(); shuf_scr.release(); shuf_fail.release();
         if (ev_first) cudaEventDestroy(ev_first);
         if (ev_last) cudaEventDestroy(ev_last);
         ev_first = ev_last = nullptr;
@@ -227,7 +230,9 @@ struct SharedOut {
     }
 };
 
-enum { SINK_NONE = 0, SINK_SHARED = 1, SINK_STREAM = 2, SINK_CAND = 3 };
+// SINK_TOTALS: the totals-only pass of mirfold_shuffle_test -- prepare, fill and f3, then only F[seq_off + 1] per locus
+// (4 bytes) leaves the device; no emission plan, traceback or pack
+enum { SINK_NONE = 0, SINK_SHARED = 1, SINK_STREAM = 2, SINK_CAND = 3, SINK_TOTALS = 4 };
 
 // fused stage 1 + 3: what the chunks of all devices append to (small: a few percent of the hit text)
 struct CandCollector {
@@ -260,6 +265,7 @@ struct Job {   // one fold call; shared read-only by the device threads (sinks a
     std::atomic<int> *cb_abort = nullptr;
     const CandArgs *cand = nullptr;
     CandCollector *collect = nullptr;
+    int32_t *totals = nullptr;         // SINK_TOTALS: per record of the call
 };
 
 struct DevOut {
@@ -365,6 +371,11 @@ __global__ void k_gather_bounds(const unsigned long long *tb_base, const unsigne
 {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k <= nl) out[k] = hitidx[tb_base[k]];
+    if (k < nl) totals[k] = F[loci[k].seq_off + 1];
+}
+__global__ void k_gather_totals(const LocusDesc *loci, const int *F, int *totals, int nl)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k < nl) totals[k] = F[loci[k].seq_off + 1];
 }
 
@@ -581,7 +592,7 @@ struct DevicePipeline {
         chunks.push_back({b, loci.size()});
         // The download of a device's LAST chunk is the only one nothing overlaps (154 MB per device take 11.6 ms when eight GPUs
         // write into host memory at once): cut the last chunk 80 : 20 so that only the small tail's download is exposed.
-        if (J.sink != SINK_NONE) {
+        if (J.sink != SINK_NONE && J.sink != SINK_TOTALS) {
             const Chunk last = chunks.back();
             uint64_t cells = 0;
             for (size_t k = last.begin; k < last.end; k++) cells += loci[k].cells;
@@ -672,7 +683,7 @@ struct DevicePipeline {
         // The two lanes' fills normally share the SMs and finish together, which is what hides wave tails -- but it also means the
         // small last chunk (plan_chunks cuts it 80 : 20) would be done before the previous chunk's download even starts.  Its fill
         // therefore waits for the previous chunk's fill to END: it then runs next to that chunk's traceback and under its download.
-        if (J.sink != SINK_NONE && nlanes_ == 2 && ci > 0 && ci + 1 == chunks.size())
+        if (J.sink != SINK_NONE && J.sink != SINK_TOTALS && nlanes_ == 2 && ci > 0 && ci + 1 == chunks.size())
             CK(cudaStreamWaitEvent(lo, D.lane[(ci + 1) % 2].ev[3], 0));
         // ---- K1, K2 on the low-priority stream
         const LocusDesc *dl = Ln.loci.as<LocusDesc>();
@@ -693,6 +704,7 @@ struct DevicePipeline {
             out.st.kernel_launches += 1 + nfill + (P.n_long > 0 ? 1 : 0) + (P.n_long < nl ? 1 : 0);
         }
         CK(cudaEventRecord(Ln.ev[4], hi));
+        if (J.sink == SINK_TOTALS) return front_totals(Ln, ci + 1 == chunks.size());
         TraceBuffers &tb = Ln.tb;
         tb = TraceBuffers{};
         tb.loci = dl; tb.nloci = nl; tb.codes = Ln.codes.as<unsigned char>();
@@ -711,9 +723,31 @@ struct DevicePipeline {
         return true;
     }
 
+    // ---- SINK_TOTALS: the chunk ends after f3 with the download of its total lines (retire publishes them)
+    bool front_totals(Lane &Ln, bool last_chunk)
+    {
+        cudaStream_t hi = Ln.s_hi;
+        const int nl = Ln.prep.nl;
+        CK(Ln.totals.ensure((size_t)nl * 4 + 4));
+        CK(Ln.h_out.ensure((size_t)nl * 4 + 64));
+        k_gather_totals<<<(nl + 255) / 256, 256, 0, hi>>>(Ln.loci.as<LocusDesc>(), Ln.F.as<int>(), Ln.totals.as<int>(), nl);
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(Ln.ev[5], hi));
+        if (last_chunk) CK(cudaEventRecord(D.ev_last, hi));
+        CK(cudaMemcpyAsync(Ln.h_out.p, Ln.totals.p, (size_t)nl * 4, cudaMemcpyDeviceToHost, hi));
+        CK(cudaEventRecord(Ln.ev[6], hi));
+        CK(cudaStreamWaitEvent(Ln.s_lo, Ln.ev[6], 0));   // the lane's next upload waits for this chunk to leave the device
+        out.st.kernel_launches += 1;
+        out.st.d2h_bytes += (uint64_t)nl * 4;
+        Ln.pending = true;
+        ht.mark("front (descriptors, uploads, K1-K3, totals enqueue)");
+        return true;
+    }
+
     // ---- middle: tracebacks, emission decisions, output sizes (second host sync)
     bool middle(Lane &Ln)
     {
+        if (J.sink == SINK_TOTALS) return true;
         cudaStream_t hi = Ln.s_hi;
         TraceBuffers &tb = Ln.tb;
         const Prep &P = Ln.prep;
@@ -762,6 +796,7 @@ struct DevicePipeline {
     // ---- back: pack the printed structures and start the download into the sink (asynchronous; see retire)
     bool back(Lane &Ln, bool last_chunk)
     {
+        if (J.sink == SINK_TOTALS) return true;
         cudaStream_t hi = Ln.s_hi;
         TraceBuffers &tb = Ln.tb;
         const Prep &P = Ln.prep;
@@ -944,6 +979,11 @@ struct DevicePipeline {
         }
         if (J.sink == SINK_NONE) return true;
         if (J.sink == SINK_CAND) { retire_candidates(Ln); return true; }
+        if (J.sink == SINK_TOTALS) {
+            const int *h = Ln.h_out.as<int>();
+            for (int k = 0; k < nl; k++) J.totals[loci[P.cb + k].rec] = h[k];
+            return true;
+        }
         const unsigned long long *h_bounds = Ln.h_out.as<unsigned long long>();
         const int *h_total = (const int *)(h_bounds + nl + 1);
         if (J.sink == SINK_SHARED) {
@@ -1056,6 +1096,7 @@ struct FoldArgs {
     const CandArgs *cand = nullptr;      // SINK_CAND
     CandCollector *collect = nullptr;
     uint64_t *nhits_out = nullptr;
+    int32_t *totals = nullptr;           // SINK_TOTALS: nseq entries, records shorter than 5 nt are left as they are
 };
 
 int fold_engine(mirfold_ctx *ctx, const FoldArgs &A, mirfold_result **out, mirfold_stats *stats_out)
@@ -1086,12 +1127,12 @@ int fold_engine(mirfold_ctx *ctx, const FoldArgs &A, mirfold_result **out, mirfo
     std::mutex cb_mu;
     std::atomic<int> cb_abort{0};
     J.fn = A.fn; J.user = A.user; J.cb_mu = &cb_mu; J.cb_abort = &cb_abort;
-    J.cand = A.cand; J.collect = A.collect;
+    J.cand = A.cand; J.collect = A.collect; J.totals = A.totals;
 
     std::unique_ptr<ResultOwner> R;
     SharedOut S;
     const uint64_t nt_total = nseq ? A.seq_off[nseq] - A.seq_off[0] : 0;
-    if (A.sink != SINK_STREAM && A.sink != SINK_CAND) {
+    if (A.sink == SINK_SHARED || A.sink == SINK_NONE) {
         R.reset(new ResultOwner());
         R->ctx = ctx;
         R->hit_begin.assign((size_t)nseq + 1, 0);
@@ -1143,7 +1184,7 @@ int fold_engine(mirfold_ctx *ctx, const FoldArgs &A, mirfold_result **out, mirfo
     for (int g = 0; g < G; g++) { add_stats(st, parts[g].st); nhits += parts[g].nhits; abytes += parts[g].arena_bytes; }
     st.n_devices = G;
 
-    if (A.sink == SINK_CAND) {
+    if (A.sink == SINK_CAND || A.sink == SINK_TOTALS) {
         st.ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
         if (stats_out) *stats_out = st;
         if (A.nhits_out) *A.nhits_out = nhits;
@@ -1627,6 +1668,208 @@ int mirfold_fold_candidates_regions(mirfold_ctx *ctx, const mirfold_genome *geno
 void mirfold_free_candidates(mirfold_candidates *c)
 {
     if (c) delete reinterpret_cast<CandOwner *>(c);
+}
+
+}  // extern "C"
+
+namespace {
+// ---- MFE significance against shuffles (mirfold_shuffle_test / mirfold_shuffle_sequences)
+int shuffle_args(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq_off, uint32_t nseq, int mode)
+{
+    if (!ctx || ctx->closed || !seq_off || (!seqs && nseq)) return MIRFOLD_ERR_ARG;
+    if (mode != MIRFOLD_SHUFFLE_MONO && mode != MIRFOLD_SHUFFLE_DI) { ctx->last_error = "unknown shuffle mode"; return MIRFOLD_ERR_ARG; }
+    const int rc = validate_offsets(ctx, seq_off, nseq);
+    if (rc != MIRFOLD_OK) return rc;
+    if (mode == MIRFOLD_SHUFFLE_DI)
+        for (uint32_t r = 0; r < nseq; r++) {
+            bool seen[256] = {};
+            int ns = 0;
+            for (uint64_t t = seq_off[r]; t < seq_off[r + 1]; t++) {
+                unsigned char c = (unsigned char)seqs[t];
+                if (c >= 'a' && c <= 'z') c -= 32;
+                if (c == 'T') c = 'U';
+                if (!seen[c]) { seen[c] = true; ns++; }
+            }
+            if (ns > MF_SHUF_MAX_SYMBOLS) {
+                char msg[128];
+                snprintf(msg, sizeof msg, "record %u has %d distinct symbols; dinucleotide shuffles allow %d", r, ns, MF_SHUF_MAX_SYMBOLS);
+                ctx->last_error = msg;
+                return MIRFOLD_ERR_ARG;
+            }
+        }
+    return MIRFOLD_OK;
+}
+
+// the records, rebased to offset 0 (off), onto device D
+cudaError_t shuffle_upload(Device &D, const char *seqs, const std::vector<uint64_t> &off)
+{
+    const size_t nseq = off.size() - 1, bytes = (size_t)off.back();
+    cudaError_t e = cudaSetDevice(D.id);
+    if (e == cudaSuccess) e = D.shuf_in.ensure(bytes + 16);
+    if (e == cudaSuccess) e = D.shuf_off.ensure(8 * (nseq + 1));
+    if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(D.shuf_in.p, seqs, bytes, cudaMemcpyHostToDevice, D.lane[0].s_lo);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(D.shuf_off.p, off.data(), 8 * (nseq + 1), cudaMemcpyHostToDevice, D.lane[0].s_lo);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(D.lane[0].s_lo);
+    return e;
+}
+
+// the round's replicates into D.shuf_raw (bytes in all); *bad = a record with too many symbols (checked on the host before)
+cudaError_t shuffle_generate(Device &D, const std::vector<ShuffleItem> &items, uint64_t bytes, uint64_t seed, int mode, int *bad)
+{
+    cudaStream_t st = D.lane[0].s_lo;
+    cudaError_t e = cudaSetDevice(D.id);
+    if (e == cudaSuccess) e = D.shuf_items.ensure(sizeof(ShuffleItem) * items.size() + 16);
+    if (e == cudaSuccess) e = D.shuf_raw.ensure(bytes + 16);
+    if (e == cudaSuccess) e = D.shuf_scr.ensure(bytes + 16);
+    if (e == cudaSuccess) e = D.shuf_fail.ensure(4);
+    if (e == cudaSuccess) e = cudaMemsetAsync(D.shuf_fail.p, 0, 4, st);
+    if (e == cudaSuccess && !items.empty())
+        e = cudaMemcpyAsync(D.shuf_items.p, items.data(), sizeof(ShuffleItem) * items.size(), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess)
+        e = launch_shuffle(D.shuf_in.as<char>(), D.shuf_off.as<unsigned long long>(), D.shuf_items.as<ShuffleItem>(), (unsigned)items.size(),
+                           D.shuf_raw.as<char>(), D.shuf_scr.as<unsigned char>(), seed, mode, D.shuf_fail.as<int>(), st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(bad, D.shuf_fail.p, 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    return e;
+}
+
+void add_stats_sequential(mirfold_stats &a, const mirfold_stats &b)   // engine calls that ran one after the other
+{
+    a.ms_h2d += b.ms_h2d; a.ms_fill += b.ms_fill; a.ms_f3 += b.ms_f3; a.ms_trace += b.ms_trace; a.ms_d2h += b.ms_d2h;
+    a.ms_device += b.ms_device;
+    a.nt += b.nt; a.cells += b.cells; a.tracebacks += b.tracebacks; a.kernel_launches += b.kernel_launches;
+    a.h2d_bytes += b.h2d_bytes; a.d2h_bytes += b.d2h_bytes; a.n_chunks += b.n_chunks; a.fill_units += b.fill_units;
+}
+
+int cuda_fail(mirfold_ctx *ctx, cudaError_t e, const char *what)
+{
+    ctx->last_error = std::string(what) + ": " + cudaGetErrorString(e);
+    cudaGetLastError();
+    return e == cudaErrorMemoryAllocation ? MIRFOLD_ERR_NOMEM : MIRFOLD_ERR_CUDA;
+}
+}  // namespace
+
+extern "C" {
+
+// Rounds: the (record, replicate) pairs of records of at least 5 nt, replicate-major, are cut into rounds of at most
+// MIRFOLD_SHUFFLE_ROUND_NT nucleotides (default 2^27; a single longer pair is a round of its own).  Every device generates
+// the whole round into its own raw buffer (cheaper than moving it), and the round is folded as a device-resident batch
+// through the engine (LPT shards, chunks and lanes unchanged) with the totals-only sink.  The natives are folded once the
+// same way.  The tally is integer arithmetic on the host, so it is exact and independent of the order of the rounds.
+int mirfold_shuffle_test(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq_off, uint32_t nseq, int span_L, uint32_t flags,
+                         int mode, uint32_t n_shuffles, uint64_t seed, mirfold_shuffle_stat *out, mirfold_stats *stats)
+{
+    if (!out || n_shuffles == 0) return MIRFOLD_ERR_ARG;
+    int rc = shuffle_args(ctx, seqs, seq_off, nseq, mode);
+    if (rc != MIRFOLD_OK) return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    std::vector<uint64_t> off((size_t)nseq + 1);
+    uint64_t max_n = 0;
+    for (uint32_t r = 0; r <= nseq; r++) off[r] = seq_off[r] - seq_off[0];
+    for (uint32_t r = 0; r < nseq; r++) max_n = std::max(max_n, off[r + 1] - off[r]);
+    int L = span_L;
+    if (span_L == 0) {   // global: L* = min(L, n) = n for every record
+        if (max_n > MF_MAX_SPAN) { ctx->last_error = "span_L = 0 (global) needs records of at most 4096 nt"; return MIRFOLD_ERR_ARG; }
+        L = (int)std::max<uint64_t>(max_n, 5);
+    } else if (span_L < 5 || span_L > MF_MAX_SPAN) { ctx->last_error = "span_L out of range [5, 4096] (or 0)"; return MIRFOLD_ERR_ARG; }
+    const char *base = nseq ? seqs + seq_off[0] : seqs;
+    mirfold_stats st{};
+    for (Device &D : ctx->devs) {
+        const cudaError_t e = shuffle_upload(D, base, off);
+        if (e != cudaSuccess) return cuda_fail(ctx, e, "shuffle upload");
+        st.h2d_bytes += off.back() + 8 * ((uint64_t)nseq + 1);
+    }
+    std::vector<void *> d_in, d_round;
+    for (Device &D : ctx->devs) d_in.push_back(D.shuf_in.p);
+    // natives
+    std::vector<int32_t> native((size_t)nseq + 1, 0);
+    {
+        FoldArgs A;
+        A.seq_off = off.data(); A.nseq = nseq; A.span_L = L; A.flags = flags; A.sink = SINK_TOTALS;
+        A.d_raw = &d_in; A.raw_off = off.data(); A.totals = native.data();
+        mirfold_stats s{};
+        rc = fold_engine(ctx, A, nullptr, &s);
+        if (rc != MIRFOLD_OK) return rc;
+        add_stats_sequential(st, s);
+    }
+    std::vector<mirfold_shuffle_stat> res((size_t)nseq);
+    std::vector<uint32_t> recs;
+    for (uint32_t r = 0; r < nseq; r++) {
+        res[r] = mirfold_shuffle_stat{native[r], 0, 0, 0};
+        if (off[r + 1] - off[r] >= 5) recs.push_back(r);
+        else res[r].n_le = n_shuffles;   // nothing to fold: every shuffle totals 0 == native
+    }
+    const char *env = getenv("MIRFOLD_SHUFFLE_ROUND_NT");
+    const uint64_t round_nt = std::max<uint64_t>(env ? strtoull(env, nullptr, 10) : (1ull << 27), 1);
+    std::vector<ShuffleItem> items;
+    std::vector<uint64_t> roff;
+    std::vector<int32_t> tot;
+    size_t cursor = 0;
+    const size_t npairs = recs.size() * (size_t)n_shuffles;
+    while (cursor < npairs) {
+        items.clear(); roff.assign(1, 0);
+        for (; cursor < npairs; cursor++) {
+            const uint32_t r = recs[cursor % recs.size()];
+            const uint64_t n = off[r + 1] - off[r];
+            if (!items.empty() && roff.back() + n > round_nt) break;
+            items.push_back(ShuffleItem{r, (uint32_t)(cursor / recs.size()), roff.back()});
+            roff.push_back(roff.back() + n);
+        }
+        d_round.clear();
+        for (Device &D : ctx->devs) {
+            int bad = 0;
+            const cudaError_t e = shuffle_generate(D, items, roff.back(), seed, mode, &bad);
+            if (e != cudaSuccess) return cuda_fail(ctx, e, "shuffle kernel");
+            if (bad) { ctx->last_error = "a record has too many distinct symbols"; return MIRFOLD_ERR_ARG; }
+            d_round.push_back(D.shuf_raw.p);
+            st.h2d_bytes += sizeof(ShuffleItem) * items.size();
+            st.kernel_launches += 1;
+        }
+        tot.assign(items.size(), 0);
+        FoldArgs A;
+        A.seq_off = roff.data(); A.nseq = (uint32_t)items.size(); A.span_L = L; A.flags = flags; A.sink = SINK_TOTALS;
+        A.d_raw = &d_round; A.raw_off = roff.data(); A.totals = tot.data();
+        mirfold_stats s{};
+        rc = fold_engine(ctx, A, nullptr, &s);
+        if (rc != MIRFOLD_OK) return rc;
+        add_stats_sequential(st, s);
+        for (size_t i = 0; i < items.size(); i++) {
+            mirfold_shuffle_stat &o = res[items[i].rec];
+            const int64_t t = tot[i];
+            o.n_le += t <= (int64_t)o.native_dcal;
+            o.sum_dcal += t;
+            o.sumsq_dcal += t * t;
+        }
+    }
+    if (nseq) memcpy(out, res.data(), sizeof(mirfold_shuffle_stat) * nseq);
+    st.n_devices = (int32_t)ctx->devs.size();
+    st.ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = st;
+    return MIRFOLD_OK;
+}
+
+int mirfold_shuffle_sequences(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq_off, uint32_t nseq, int mode, uint64_t seed,
+                              uint32_t replicate, char *out)
+{
+    if (!out) return MIRFOLD_ERR_ARG;
+    const int rc = shuffle_args(ctx, seqs, seq_off, nseq, mode);
+    if (rc != MIRFOLD_OK) return rc;
+    std::vector<uint64_t> off((size_t)nseq + 1);
+    for (uint32_t r = 0; r <= nseq; r++) off[r] = seq_off[r] - seq_off[0];
+    std::vector<ShuffleItem> items((size_t)nseq);
+    for (uint32_t r = 0; r < nseq; r++) items[r] = ShuffleItem{r, replicate, off[r]};
+    Device &D = ctx->devs[0];
+    int bad = 0;
+    cudaError_t e = shuffle_upload(D, nseq ? seqs + seq_off[0] : seqs, off);
+    if (e == cudaSuccess) e = shuffle_generate(D, items, off.back(), seed, mode, &bad);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "shuffle kernel");
+    if (bad) { ctx->last_error = "a record has too many distinct symbols"; return MIRFOLD_ERR_ARG; }
+    if (off.back()) {
+        e = cudaMemcpyAsync(out + seq_off[0], D.shuf_raw.p, (size_t)off.back(), cudaMemcpyDeviceToHost, D.lane[0].s_lo);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(D.lane[0].s_lo);
+        if (e != cudaSuccess) return cuda_fail(ctx, e, "shuffle download");
+    }
+    return MIRFOLD_OK;
 }
 
 int mirfold_plan_shards(const uint64_t *seq_off, uint32_t nseq, int span_L, int n_shards, uint32_t *shard_of, uint64_t *shard_cells)

@@ -220,6 +220,16 @@ struct CandLaunch {
 cudaError_t launch_cand_classify(const CandLaunch &a, int pass, cudaStream_t st);
 cudaError_t launch_cand_finish(const CandLaunch &a, int max_len, cudaStream_t st);
 cudaError_t run_int_peak(cudaStream_t st, int sm_count, double *addmin, double *dpx, double *s16x2);
+// shuffled replicates of the significance test (shuffle.cu): item t writes replicate `rep` of input record `rec` (n bytes,
+// converted letters) to out + dst, using scr + dst as n bytes of scratch
+#define MF_SHUFFLE_MONO 1   /* == MIRFOLD_SHUFFLE_MONO */
+#define MF_SHUFFLE_DI 2     /* == MIRFOLD_SHUFFLE_DI   */
+struct ShuffleItem {
+    unsigned int rec, rep;
+    unsigned long long dst;
+};
+cudaError_t launch_shuffle(const char *in, const unsigned long long *in_off, const ShuffleItem *items, unsigned int nitems,
+                           char *out, unsigned char *scr, unsigned long long seed, int mode, int *fail, cudaStream_t st);
 struct mirfold_duplex_query;
 struct mirfold_duplex_verdict;
 cudaError_t launch_duplex(const char *arena, const mirfold_duplex_query *qs, unsigned long long nq,

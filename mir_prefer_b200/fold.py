@@ -214,6 +214,29 @@ REGION_DTYPE = np.dtype([("start", "<i4"), ("end", "<i4")])
 GENOME_REGION_DTYPE = np.dtype([("contig", "<i4"), ("start", "<i4"), ("end", "<i4"), ("strand", "<i4")])
 
 
+# mirfold_shuffle_stat plus the fields derived from it (shuffle_test)
+SHUFFLE_MODES = {"mono": 1, "di": 2}   # MIRFOLD_SHUFFLE_MONO / MIRFOLD_SHUFFLE_DI
+SHUFFLE_STAT_DTYPE = np.dtype([("native_dcal", "<i4"), ("n_le", "<u4"), ("sum_dcal", "<i8"), ("sumsq_dcal", "<i8")])
+SHUFFLE_DTYPE = np.dtype(SHUFFLE_STAT_DTYPE.descr + [("p_value", "<f8"), ("mean", "<f8"), ("sd", "<f8"), ("z", "<f8")])
+
+
+def shuffle_fields(stat, n_shuffles):
+    """SHUFFLE_DTYPE rows from SHUFFLE_STAT_DTYPE rows of a test with K = n_shuffles shuffles: p = (n_le + 1) / (K + 1),
+    mean and population sd of the shuffles' totals (dcal), z = (native - mean) / sd (NaN when sd == 0).  The variance is
+    taken from the integer sums exactly (K * sumsq - sum^2 in Python integers), so sd is 0 exactly when all shuffles tie."""
+    K = int(n_shuffles)
+    out = np.zeros(len(stat), SHUFFLE_DTYPE)
+    for f in SHUFFLE_STAT_DTYPE.names:
+        out[f] = stat[f]
+    out["p_value"] = (out["n_le"].astype(np.float64) + 1.0) / (K + 1)
+    out["mean"] = out["sum_dcal"] / K
+    var = [(K * q - s * s) / (K * K) for s, q in zip(stat["sum_dcal"].tolist(), stat["sumsq_dcal"].tolist())]
+    out["sd"] = np.sqrt(np.asarray(var, np.float64)) if len(var) else 0.0
+    with np.errstate(divide="ignore", invalid="ignore"):
+        out["z"] = np.where(out["sd"] > 0, (out["native_dcal"] - out["mean"]) / out["sd"], np.nan)
+    return out
+
+
 def _mature_array(matures):
     """MATURE_DTYPE array of matures given as such an array or as (start, end, strand_char, depth) tuples."""
     if isinstance(matures, np.ndarray) and matures.dtype == MATURE_DTYPE:
@@ -579,6 +602,41 @@ class MirFold:
         if rc != 0:
             self._raise(rc)
         return FoldResult(self._lib, res, len(off) - 1, owner=self)
+
+    @staticmethod
+    def _shuffle_mode(mode):
+        if mode not in SHUFFLE_MODES:
+            raise MirfoldError(-3, "shuffle mode must be one of %s, not %r" % (sorted(SHUFFLE_MODES), mode))
+        return SHUFFLE_MODES[mode]
+
+    def shuffle_test(self, seqs, n_shuffles, seed=0, mode="di", span=0, flags=0, with_stats=False):
+        """mirfold_shuffle_test(): the MFE of every sequence against n_shuffles shuffles of it (randfold's test), folded on
+        the device.  mode "di" keeps dinucleotide counts (Altschul-Erickson), "mono" the base composition; span 0 folds
+        globally (sequences up to 4096 nt).  Returns a SHUFFLE_DTYPE array, one row per sequence (energies in dcal), and
+        with with_stats=True also the call's stats dict."""
+        buf, off = self.pack(seqs)
+        stat = np.zeros(len(off) - 1, SHUFFLE_STAT_DTYPE)
+        st = _lib.Stats()
+        rc = self._lib.mirfold_shuffle_test(self._ctx, buf.ctypes.data_as(C.c_void_p), off.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                            len(off) - 1, int(span), int(flags), self._shuffle_mode(mode), int(n_shuffles),
+                                            int(seed) & 0xFFFFFFFFFFFFFFFF, stat.ctypes.data_as(C.c_void_p), C.byref(st))
+        if rc != 0:
+            self._raise(rc)
+        out = shuffle_fields(stat, n_shuffles)
+        return (out, st.as_dict()) if with_stats else out
+
+    def shuffle_sequences(self, seqs, replicate, seed=0, mode="di"):
+        """mirfold_shuffle_sequences(): shuffle number `replicate` of every sequence exactly as shuffle_test folds it
+        (upper-case, T -> U), generated by the device kernel.  Returns a list of str."""
+        buf, off = self.pack(seqs)
+        out = np.zeros(max(len(buf), 1), np.uint8)
+        rc = self._lib.mirfold_shuffle_sequences(self._ctx, buf.ctypes.data_as(C.c_void_p), off.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                 len(off) - 1, self._shuffle_mode(mode), int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                                 int(replicate), out.ctypes.data_as(C.c_void_p))
+        if rc != 0:
+            self._raise(rc)
+        raw = out.tobytes()
+        return [raw[int(off[r]):int(off[r + 1])].decode("latin-1") for r in range(len(off) - 1)]
 
     def int_peak2(self):
         """(add+min, DPX s32, VIADDMNMX.S16x2) min-plus terms/s on this context's device."""

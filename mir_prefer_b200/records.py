@@ -212,6 +212,63 @@ def candidates_of_records(mf, records, span, minlen=55, minloop=3, min_mature_le
     return ss_records, DuplexTable.from_candidates(cand, records), cand
 
 
+def candidate_precursors(cand, records, genome=None, only_passing=True):
+    """The precursors hairpin_significance scores: (distinct precursor strings in order of first appearance, indices of the
+    scored structures of cand, and for each of them the index of its precursor in the first list)."""
+    import numpy as np
+    st = cand.structs
+    code0 = cand.verdicts["code"] == 0 if cand.nverdicts else np.zeros(0, bool)
+    fs_all, ln_all = st["fold_start"].tolist(), st["len"].tolist()
+    vb_all, vc_all = cand.verdict_begin.tolist(), cand.verdict_count.tolist()
+    first, uniq, rows, which = {}, [], [], []
+    for r in range(cand.nseq):
+        b, c = int(cand.struct_begin[r]), int(cand.struct_count[r])
+        seq = None
+        for k in range(b, b + c):
+            if only_passing and not code0[vb_all[k]:vb_all[k] + vc_all[k]].any():
+                continue
+            if seq is None:
+                rec = records[r]
+                seq = (genome.sequence(genome.contig_index(rec.seqid), rec.region[0], rec.region[1], rec.strand) if genome is not None
+                       else _oriented_sequence(rec))
+            p = seq[fs_all[k] - 1:fs_all[k] - 1 + ln_all[k]]
+            if p not in first:
+                first[p] = len(uniq)
+                uniq.append(p)
+            rows.append(k)
+            which.append(first[p])
+    return uniq, np.asarray(rows, np.int64), np.asarray(which, np.int64)
+
+
+def hairpin_significance(mf, cand, records, n_shuffles, seed=0, mode="di", genome=None, only_passing=True, span=0):
+    """MFE significance of the candidate precursors of `cand` (candidates_of_records' Candidates over `records`) against
+    n_shuffles shuffles each (MirFold.shuffle_test; randfold's test).  The precursor of a structure is its record's folded
+    sequence [fold_start - 1, fold_start - 1 + len); with genome= it is extracted on the host through Genome.sequence.
+    only_passing=True scores only structures with at least one code-0 duplex verdict.  Identical precursors are folded
+    once, so their rows are equal.  Returns one row per structure of cand, in cand's order: rec, struct (index within the
+    record), fold_start, len, scored, then the SHUFFLE_DTYPE fields (zero counts and NaN statistics where not scored).
+    Results depend on (seed, the distinct precursors in order of first appearance)."""
+    import numpy as np
+    from .fold import SHUFFLE_DTYPE
+    dt = np.dtype([("rec", "<u4"), ("struct", "<u4"), ("fold_start", "<i4"), ("len", "<i4"), ("scored", "?")] + SHUFFLE_DTYPE.descr)
+    out = np.zeros(cand.nstructs, dt)
+    if cand.nstructs:   # structures of record r: structs[struct_begin[r] .. +struct_count[r])
+        cnt = cand.struct_count.astype(np.int64)
+        k = np.concatenate([np.arange(b, b + c, dtype=np.int64) for b, c in zip(cand.struct_begin.tolist(), cnt.tolist())])
+        out["rec"][k] = np.repeat(np.arange(cand.nseq, dtype=np.int64), cnt)
+        out["struct"][k] = k - np.repeat(cand.struct_begin.astype(np.int64), cnt)
+    out["fold_start"], out["len"] = cand.structs["fold_start"], cand.structs["len"]
+    for f in ("p_value", "mean", "sd", "z"):
+        out[f] = np.nan
+    uniq, rows, which = candidate_precursors(cand, list(records), genome, only_passing)
+    if len(rows):
+        res = mf.shuffle_test(uniq, n_shuffles, seed=seed, mode=mode, span=span)
+        out["scored"][rows] = True
+        for f in SHUFFLE_DTYPE.names:
+            out[f][rows] = res[f][which]
+    return out
+
+
 def fold_records(mf, records, span, genome=None):
     """Fold LocusRecords on the device.  Identical oriented sequences (the reference writes
     duplicated records for both-strand L/R loci, SURVEY App. C) are folded once; record count and

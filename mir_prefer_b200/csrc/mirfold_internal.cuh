@@ -83,12 +83,25 @@ struct LocusDesc {
     // min((i-1)/tile_step, tile_last), which holds all of (i, i+4..i+dmax).  Untiled: tile_last = 0.
     int tile_last;           // number of tiles - 1
     int tile_step;           // rows owned per tile
-    unsigned int tile_rcp;   // ceil(2^32 / tile_step): (i-1)/tile_step == __umulhi(i-1, tile_rcp)
+    unsigned int tile_rcp;   // ceil(2^32 / tile_step): __umulhi(i-1, tile_rcp) is (i-1)/tile_step or one more (tile_of_row)
 };
 // raw_off flag of a minus-strand genome region (mirfold_fold_regions): k_prepare reads the locus backwards and complements it
 #define MF_RAW_REVERSE (1ULL << 63)
 #define MF_TILE_LEN 608
 #define MF_TILE_LEN_BIG 864   /* the largest shared-memory bucket: one 1024-thread CTA per SM (155 KB of rings) */
+
+// owner tile of row i (1 <= i < 2^30) of a tiled locus: min((i-1)/tile_step, tile_last).  With x = i-1, S = tile_step and
+// e = tile_rcp*S - 2^32 < S, __umulhi(x, tile_rcp) = floor(x/S + x*e/(S*2^32)); for x < 2^30 the second term is below 1/4,
+// so the estimate is x/S or, when x mod S is near S-1, x/S + 1, and one compare corrects it.  Without the correction rows
+// go wrong from x = 7 615 399 on (S = 580, L = 28).  tests/test_long_loci.py::test_owner_tile_is_exact checks a mirror of this expression
+// for every S in [MF_TILE_MIN_STEP, MF_TILE_LEN_BIG] at the worst x < 2^30 of every residue class.
+__device__ __forceinline__ int tile_of_row(int i, unsigned int tile_rcp, int tile_step, int tile_last)
+{
+    const unsigned int x = (unsigned int)(i - 1);
+    unsigned int t = __umulhi(x, tile_rcp);
+    t -= (t * (unsigned int)tile_step > x) ? 1u : 0u;
+    return min((int)t, tile_last);
+}
 
 // element offset (relative to the locus' band_off) of row i's owner-tile origin, i.e. of cell
 // (i, i+4); cell (i, i+d) sits (d-4)*stride further.  Any cell (i', j') with i <= i' and
@@ -96,7 +109,7 @@ struct LocusDesc {
 __device__ __forceinline__ unsigned long long band_row_base(const LocusDesc &L, int i)
 {
     if (L.tile_last == 0) return (unsigned long long)(i - 1);
-    const int t = min((int)__umulhi((unsigned)(i - 1), L.tile_rcp), L.tile_last);
+    const int t = tile_of_row(i, L.tile_rcp, L.tile_step, L.tile_last);
     const int a = min(t * L.tile_step, L.n - L.stride);   // tiled: stride == tile length
     return (unsigned long long)t * ((unsigned long long)(L.dmax - 3) * L.stride) + (unsigned long long)(i - 1 - a);
 }

@@ -51,10 +51,11 @@ cudaError_t launch_plan(const TraceBuffers &b, cudaStream_t st)
 // band offset of cell (i, i+d) of a tiled long locus (LocusDesc::tile_*, see band_row_base)
 __device__ __noinline__ unsigned long long tb_tiled_off(int i, int d, unsigned int tile_rcp, int tile_last, int tile_step, int n, int dmax)
 {
-    const int t = min((int)__umulhi((unsigned)(i - 1), tile_rcp), tile_last);
+    const int t = tile_of_row(i, tile_rcp, tile_step, tile_last);
     const int TL = tile_step + dmax;   // tile length == the locus' band stride (608 or 864)
-    const int a = min(t * tile_step, n - TL);
-    return (unsigned long long)t * ((unsigned long long)(dmax - 3) * TL) + (unsigned)((d - 4) * TL + (i - 1 - a));
+    const int a = min(t * tile_step, n - TL);   // tile t's first row - 1: a <= t * tile_step <= i - 1
+    // tile t, diagonal d >= 4, local row i-1-a >= 0: every term is non-negative
+    return ((unsigned long long)t * (unsigned)(dmax - 3) + (unsigned)(d - 4)) * (unsigned)TL + (unsigned)(i - 1 - a);
 }
 
 struct Fold {

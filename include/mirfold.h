@@ -108,6 +108,10 @@ void mirfold_close(mirfold_ctx *ctx);
  *   seq_off : nseq+1 offsets into seqs.
  * With n_devices > 1 the records are sharded by DP work across the devices (no collectives)
  * and gathered back in input order. */
+/* span_L is 5..4096 for every fold entry point.  A record may have up to 2^30 - 1 nt.  At span_L > 800 a record longer
+ * than 864 nt is filled as one unit (mirfold_plan_fill_units: kernel 0), which must hold fewer than 2^31 band cells,
+ * (min(span_L, n-1) - 3) * stride < 2^31: records up to 2 691 072 nt at span_L = 801, 524 672 nt at 4096.  A batch
+ * with a longer record is rejected as a whole with MIRFOLD_ERR_ARG before anything is allocated. */
 int mirfold_fold(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq_off, uint32_t nseq,
                  int span_L, uint32_t flags, mirfold_result **out);
 
@@ -207,7 +211,8 @@ int mirfold_plan_shards(const uint64_t *seq_off, uint32_t nseq, int span_L, int 
  * overlapping tiles of tile_len bases: tile t covers bases a_t+1 .. a_t+tile_len, a_t = min(t*tile_step, n-tile_len),
  * and owns rows a_t+1 .. a_t+tile_step (the last tile: all its remaining rows); every cell (i, j <= i+span) of an owned
  * row lies inside the tile.  kernel: 0 = generic global-memory kernel, else the shared-memory bucket's stride
- * (160 / 352 / 608 / 864).  band_cells = cells the band arrays hold (stride * diagonals * n_units). */
+ * (160 / 352 / 608 / 864).  band_cells = cells the band arrays hold (stride * diagonals * n_units).  MIRFOLD_ERR_ARG for an
+ * untiled unit of 2^31 band cells or more, which the fold entry points reject (see mirfold_fold). */
 typedef struct mirfold_fill_plan {
     int32_t kernel;
     int32_t stride;

@@ -1125,8 +1125,9 @@ __global__ void __launch_bounds__(NT, MINB) k_fill_s16(FillLaunch a)
 
 // ------------------------------------------------------------------------------------ K2 (generic: any n)
 // Same algorithm with the Cm window in a global-memory ring (for loci longer than the largest
-// shared-memory bucket).  Dynamic smem: sS[npad] | sS1[npad] | pairtab[64] | list[n] (int)
-template <int NT>
+// shared-memory bucket).  Scratch sS[npad] | sS1[npad] | pairtab[64] | list[n] (int), generic_scratch_bytes():
+// dynamic shared memory, or (GSCR) global memory after the unit's Cm ring when the launch's longest unit does not fit
+template <int NT, bool GSCR>
 __global__ void __launch_bounds__(NT) k_fill_generic(FillLaunch a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -1134,7 +1135,9 @@ __global__ void __launch_bounds__(NT) k_fill_generic(FillLaunch a)
     const int n = L.n, Ls = L.Ls, dmax = L.dmax, NS = L.stride;
     const DevParams *__restrict__ P = a.P;
     const int npad = (n + 3 + 15) & ~15;
-    unsigned char *sS = smem_raw;
+    int *rD = a.ring + L.ring_off;                              // [MF_RING_DML][NS]
+    int *rCm = rD + (unsigned long long)MF_RING_DML * NS;       // [MF_RING_CM][NS]
+    unsigned char *sS = GSCR ? (unsigned char *)(rCm + (unsigned long long)MF_RING_CM * NS) : smem_raw;
     unsigned char *sS1 = sS + npad;
     unsigned char *sPair = sS1 + npad;
     int *sList = (int *)(sPair + 64);
@@ -1152,8 +1155,6 @@ __global__ void __launch_bounds__(NT) k_fill_generic(FillLaunch a)
 
     int *Cb = a.C + L.band_off;
     int *Mb = a.M + L.band_off;
-    int *rD = a.ring + L.ring_off;                              // [MF_RING_DML][NS]
-    int *rCm = rD + (unsigned long long)MF_RING_DML * NS;       // [MF_RING_CM][NS]
     for (long long k = tid; k < (long long)(dmax - 3) * (NS / 4); k += NT) ((unsigned int *)(a.Ib + L.band_off))[k] = 0x01010101u;   // no traceback hint
     for (int k = tid; k < MF_RING_DML * NS; k += NT) rD[k] = MF_INF;
     __syncthreads();
@@ -1250,7 +1251,7 @@ cudaError_t fill_configure_device()
     if ((e = configure_fill_bucket<608, MF_B608_NT, 2>()) != cudaSuccess) return e;
     if ((e = configure_fill_bucket<352, MF_B352_NT, MF_B352_MINB>()) != cudaSuccess) return e;
     if ((e = configure_fill_bucket<160, 256, 4>()) != cudaSuccess) return e;
-    return cudaFuncSetAttribute(k_fill_generic<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    return cudaFuncSetAttribute(k_fill_generic<512, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MF_GENERIC_SMEM_MAX);
 }
 
 template <int NS, int NT, int MINB>
@@ -1293,13 +1294,12 @@ cudaError_t launch_fill(const FillLaunch &a, cudaStream_t st, cudaStream_t side,
     const int ng = a.bucket_first[1] - a.bucket_first[0];
     if (ng > 0) {
         constexpr int NT = 512;
-        const int npad = (a.max_n + 3 + 15) & ~15;
-        const size_t smem = (size_t)2 * npad + 64 + (size_t)a.max_n * sizeof(int) + 16;
-        if (smem > 200 * 1024) return cudaErrorInvalidValue;   // n > ~33 000 nt
+        const size_t smem = generic_scratch_bytes(a.max_n);
         FillLaunch b = a;
         b.loci = a.loci + a.bucket_first[0];
         b.nloci = ng;
-        k_fill_generic<NT><<<ng, NT, smem, st>>>(b);
+        if (smem <= MF_GENERIC_SMEM_MAX) k_fill_generic<NT, false><<<ng, NT, smem, st>>>(b);
+        else k_fill_generic<NT, true><<<ng, NT, 0, st>>>(b);   // a unit of more than about 34 100 nt
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }
     if ((e = launch_fill_bucket<MF_TILE_LEN_BIG, MF_B864_NT, 1>(a, a.bucket_first[1], a.bucket_first[2] - a.bucket_first[1], st)) != cudaSuccess) return e;

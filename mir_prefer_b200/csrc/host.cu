@@ -425,9 +425,17 @@ unsigned long long shape_locus(LocusDesc &d, int n, int L)
     }
     return band_elems(d.stride, d.dmax);
 }
+// ring scratch of one fill unit: the DML ring; a generic unit adds its Cm ring and room for the kernel's scratch, which
+// k_fill_generic keeps there when it does not fit shared memory (rounded to 128 B so that the next unit's rings stay aligned)
 unsigned long long unit_ring_elems(int stride)
 {
-    return (unsigned long long)stride * (is_bucket_stride(stride) ? MF_RING_DML : MF_RING_PER_STRIDE);
+    if (is_bucket_stride(stride)) return (unsigned long long)stride * MF_RING_DML;
+    return (unsigned long long)stride * MF_RING_PER_STRIDE + (generic_scratch_bytes(stride) + 127) / 128 * 32;
+}
+// an untiled unit of 2^31 band cells or more overflows the kernels' 32-bit band offsets (MF_MAX_UNIT_BAND_CELLS)
+static bool band_offsets_fit(const LocusDesc &d)
+{
+    return d.tile_last > 0 || band_elems(d.stride, d.dmax) < MF_MAX_UNIT_BAND_CELLS;
 }
 static int unit_bucket(const LocusDesc &u)   // index into FillLaunch::bucket_first
 {
@@ -1069,11 +1077,25 @@ void add_stats(mirfold_stats &a, const mirfold_stats &b)
     a.h2d_bytes += b.h2d_bytes; a.d2h_bytes += b.d2h_bytes; a.n_chunks += b.n_chunks; a.fill_units += b.fill_units;
 }
 
-int validate_offsets(mirfold_ctx *ctx, const uint64_t *seq_off, uint32_t nseq)
+// span_L > 0: also every record the engine would fill as one unit of 2^31 band cells or more (band_offsets_fit), so
+// that such a batch is refused before anything is allocated.  Those need n * (min(span_L, n) - 3) >= 2^31, so n > 2^19.
+int validate_offsets(mirfold_ctx *ctx, const uint64_t *seq_off, uint32_t nseq, int span_L)
 {
     for (uint32_t r = 0; r < nseq; r++) {
         if (seq_off[r + 1] < seq_off[r]) { ctx->last_error = "seq_off is not non-decreasing"; return MIRFOLD_ERR_ARG; }
-        if (seq_off[r + 1] - seq_off[r] > (uint64_t)0x3fffffff) { ctx->last_error = "a sequence is longer than 2^30 - 1 nt"; return MIRFOLD_ERR_ARG; }
+        const uint64_t len = seq_off[r + 1] - seq_off[r];
+        if (len > (uint64_t)0x3fffffff) { ctx->last_error = "a sequence is longer than 2^30 - 1 nt"; return MIRFOLD_ERR_ARG; }
+        if (span_L > 0 && len > (1u << 19)) {
+            LocusDesc d{};
+            shape_locus(d, (int)len, span_L);
+            if (!band_offsets_fit(d)) {
+                char msg[160];
+                snprintf(msg, sizeof msg, "record %u: %llu nt at span %d is one fill unit of %llu band cells (at most 2^31 - 1)", r,
+                         (unsigned long long)len, span_L, band_elems(d.stride, d.dmax));
+                ctx->last_error = msg;
+                return MIRFOLD_ERR_ARG;
+            }
+        }
     }
     return MIRFOLD_OK;
 }
@@ -1107,7 +1129,7 @@ int fold_engine(mirfold_ctx *ctx, const FoldArgs &A, mirfold_result **out, mirfo
     if (ctx->closed) return MIRFOLD_ERR_ARG;
     if (A.span_L < 5 || A.span_L > MF_MAX_SPAN) { ctx->last_error = "span_L out of range [5, 4096]"; return MIRFOLD_ERR_ARG; }
     if (out) *out = nullptr;
-    int rc = validate_offsets(ctx, A.seq_off, A.nseq);
+    int rc = validate_offsets(ctx, A.seq_off, A.nseq, A.span_L);
     if (rc != MIRFOLD_OK) return rc;
     const auto t0 = std::chrono::steady_clock::now();
     HostTimer ht;
@@ -1403,7 +1425,7 @@ int mirfold_batch_upload(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq
     if (!ctx || !out || !seq_off || (!seqs && nseq) || ctx->closed) return MIRFOLD_ERR_ARG;
     *out = nullptr;
     if (span_L < 5 || span_L > MF_MAX_SPAN) { ctx->last_error = "span_L out of range [5, 4096]"; return MIRFOLD_ERR_ARG; }
-    int rc = validate_offsets(ctx, seq_off, nseq);
+    int rc = validate_offsets(ctx, seq_off, nseq, span_L);
     if (rc != MIRFOLD_OK) return rc;
     std::unique_ptr<mirfold_batch> B(new mirfold_batch());
     B->ctx = ctx; B->nseq = nseq; B->span_L = span_L;
@@ -1678,7 +1700,7 @@ int shuffle_args(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq_off, ui
 {
     if (!ctx || ctx->closed || !seq_off || (!seqs && nseq)) return MIRFOLD_ERR_ARG;
     if (mode != MIRFOLD_SHUFFLE_MONO && mode != MIRFOLD_SHUFFLE_DI) { ctx->last_error = "unknown shuffle mode"; return MIRFOLD_ERR_ARG; }
-    const int rc = validate_offsets(ctx, seq_off, nseq);
+    const int rc = validate_offsets(ctx, seq_off, nseq, 0);   // the span is checked by mirfold_shuffle_test
     if (rc != MIRFOLD_OK) return rc;
     if (mode == MIRFOLD_SHUFFLE_DI)
         for (uint32_t r = 0; r < nseq; r++) {
@@ -1772,6 +1794,7 @@ int mirfold_shuffle_test(mirfold_ctx *ctx, const char *seqs, const uint64_t *seq
         if (max_n > MF_MAX_SPAN) { ctx->last_error = "span_L = 0 (global) needs records of at most 4096 nt"; return MIRFOLD_ERR_ARG; }
         L = (int)std::max<uint64_t>(max_n, 5);
     } else if (span_L < 5 || span_L > MF_MAX_SPAN) { ctx->last_error = "span_L out of range [5, 4096] (or 0)"; return MIRFOLD_ERR_ARG; }
+    if ((rc = validate_offsets(ctx, seq_off, nseq, L)) != MIRFOLD_OK) return rc;
     const char *base = nseq ? seqs + seq_off[0] : seqs;
     mirfold_stats st{};
     for (Device &D : ctx->devs) {
@@ -1891,6 +1914,7 @@ int mirfold_plan_fill_units(uint32_t n, int span_L, mirfold_fill_plan *out)
     if (!out || n < 1 || n > 0x7fffffffu || span_L < 5) return MIRFOLD_ERR_ARG;
     LocusDesc d{};
     const unsigned long long be = shape_locus(d, (int)n, span_L);
+    if (!band_offsets_fit(d)) return MIRFOLD_ERR_ARG;
     out->kernel = is_bucket_stride(d.stride) ? d.stride : 0;
     out->stride = d.stride;
     out->tile_len = d.tile_last ? d.stride : (int)n;
@@ -1935,6 +1959,7 @@ int mirfold_debug_matrices(mirfold_ctx *ctx, const char *seq, uint32_t n, int sp
     cudaStream_t st = Ln.s_lo;
     LocusDesc d{};
     const unsigned long long cells = shape_locus(d, (int)n, span_L);
+    if (!band_offsets_fit(d)) { ctx->last_error = "one fill unit of 2^31 band cells or more"; return MIRFOLD_ERR_ARG; }
     std::vector<LocusDesc> units;
     int bucket_first[6], max_n = 0;
     const unsigned long long ring_elems = build_fill_units(&d, 1, units, bucket_first, max_n);

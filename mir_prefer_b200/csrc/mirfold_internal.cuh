@@ -138,6 +138,17 @@ __host__ __device__ __forceinline__ int band_stride_for(int n, bool big)
 #define MF_RING_CM 64  /* generic kernel: Cm window ring in global memory (needs >= 33 diagonals) */
 #define MF_RING_DML 16 /* DML ring (needs >= 9 diagonals)                                         */
 #define MF_RING_PER_STRIDE (MF_RING_CM + MF_RING_DML)
+// generic kernel scratch of an n-nt unit: sS[npad] | sS1[npad] | pair table[64] | typed-cell list[n] (int), 16 B slack.
+// In dynamic shared memory while the launch's longest unit fits MF_GENERIC_SMEM_MAX (about 34 100 nt), else in the
+// unit's ring region after its Cm ring (unit_ring_elems in host.cu reserves it for every generic unit)
+#define MF_GENERIC_SMEM_MAX (200 * 1024)
+__host__ __device__ __forceinline__ unsigned long long generic_scratch_bytes(int n)
+{
+    return 2ULL * (unsigned long long)((n + 3 + 15) & ~15) + 64 + 4ULL * (unsigned long long)n + 16;
+}
+// An untiled unit addresses its band with 32-bit offsets (d-4)*stride + i-1 (k_fill_generic, the f3 kernels, the
+// traceback): its band must hold fewer than 2^31 cells.  Tiled units (stride <= 864) are far below.
+#define MF_MAX_UNIT_BAND_CELLS (1ULL << 31)
 
 // ---- kernel launchers (each defined next to its kernels) -------------------------------
 struct FillLaunch {

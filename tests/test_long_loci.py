@@ -96,18 +96,29 @@ def test_owner_tile_estimate_alone_is_wrong_on_long_loci():
     assert min((first_wrong_row(S) or MAX_ROW, S) for S in range(MIN_STEP, 605)) == (7_158_607, 604)
 
 
-def test_planned_tile_steps_are_in_the_checked_range():
+def test_planned_tile_steps_are_in_the_checked_range_or_untiled():
     """Every span the engine accepts up to the 864-nt bucket tiles a 2^30 - 1 nt locus with a step test_owner_tile_is_exact
-    covers, or does not tile it; the step and rcp pairing is the one the mirror assumes."""
+    covers, or does not tile it; the step and rcp pairing is the one the mirror assumes.  A span that does not tile (L > 800)
+    plans longer loci as one generic unit, and a 2^30 - 1 nt locus is then rejected: its unit would hold more than 2^31
+    band cells, beyond the kernels' 32-bit band offsets (tests/test_wide_spans.py)."""
     steps = set()
+    untiled = []
     for L in range(5, MAX_STEP + 1):
-        p = plan_fill_units(MAX_ROW - 1, L)
+        try:
+            p = plan_fill_units(MAX_ROW - 1, L)
+        except mp.MirfoldError as e:
+            assert e.code == -3, L
+            g = plan_fill_units(MAX_STEP + 1, L)
+            assert g["kernel"] == 0 and g["n_units"] == 1, (L, g)
+            untiled.append(L)
+            continue
         if p["n_units"] > 1:
             assert MIN_STEP <= p["tile_step"] <= MAX_STEP, (L, p)
             assert p["tile_step"] == p["tile_len"] - p["dmax"]
             steps.add(p["tile_step"])
         else:
             assert p["kernel"] == 0, (L, p)   # a span too wide to tile: the generic kernel, untiled
+    assert untiled == list(range(801, MAX_STEP + 1))
     # spans 5..800 give 540 distinct steps; the first row any of them gets wrong without the correction is x = 7 615 399
     assert len(steps) == 540
     assert min(first_wrong_row(S) for S in steps if first_wrong_row(S)) == 7_615_399

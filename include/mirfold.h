@@ -108,7 +108,8 @@ void mirfold_close(mirfold_ctx *ctx);
  *   seq_off : nseq+1 offsets into seqs.
  * With n_devices > 1 the records are sharded by DP work across the devices (no collectives)
  * and gathered back in input order. */
-/* span_L is 5..4096 for every fold entry point.  A record may have up to 2^30 - 1 nt.  At span_L > 800 a record longer
+/* span_L is 5..4096 for every fold entry point.  A record may have up to 2^30 - 1 nt, whatever the device's memory: a
+ * tiled record larger than the device budget is folded in segments (mirfold_plan_segments), with the same result.  At span_L > 800 a record longer
  * than 864 nt is filled as one unit (mirfold_plan_fill_units: kernel 0), which must hold fewer than 2^31 band cells,
  * (min(span_L, n-1) - 3) * stride < 2^31: records up to 2 691 072 nt at span_L = 801, 524 672 nt at 4096.  A batch
  * with a longer record is rejected as a whole with MIRFOLD_ERR_ARG before anything is allocated. */
@@ -223,6 +224,26 @@ typedef struct mirfold_fill_plan {
     uint64_t band_cells;
 } mirfold_fill_plan;
 int mirfold_plan_fill_units(uint32_t n, int span_L, mirfold_fill_plan *out);
+
+/* How the fold runs one locus of n bases at span span_L when its device entry may use budget_bytes for it.  A tiled locus
+ * (mirfold_plan_fill_units: n_units > 1) that needs more than the budget is folded in segments from its 3' end, so a
+ * record's length is not bounded by device memory: a segment owns the tiles tile_first .. tile_last (rows row_first ..
+ * row_last) and also fills the halo_tiles tiles above them, which own the rows up to row_last + min(span_L, n) + 1 that
+ * its f3 and tracebacks read.  The sequence-sized arrays (about 16 bytes per nt) stay whole; device_bytes is what the
+ * segment needs with them.  Segments take as many owned tiles as fit the budget, at least one.  A locus that fits, or is
+ * one unit, is one segment.  The engine uses this plan with budget_bytes = a lane's share of the device entry's budget
+ * (MIRFOLD_MEM_BUDGET_MB, or a share of free memory at mirfold_open) for every locus larger than the whole budget.
+ * Host-only.  *n_segments = the number of segments; the first min(cap, *n_segments) are written to segs, in the order
+ * they run.  MIRFOLD_ERR_ARG as mirfold_plan_fill_units, and for n >= 2^30. */
+typedef struct mirfold_segment {
+    int32_t tile_first, tile_last;   /* owned tiles */
+    int32_t halo_tiles;              /* tiles tile_last+1 .. tile_last+halo_tiles, filled but not owned */
+    int32_t row_first, row_last;     /* owned rows (1-based) */
+    int32_t reserved;
+    uint64_t device_bytes;
+} mirfold_segment;
+int mirfold_plan_segments(uint32_t n, int span_L, uint64_t budget_bytes, mirfold_segment *segs, uint32_t cap,
+                          uint32_t *n_segments);
 
 /* Replaces: what RNALfold's main() prints per record (RLF .rodata "%s (%6.2f) %4d\n" / "%s\n (%6.2f)\n",
  * SURVEY A.6) -- the text miR_PREFeR.py collects at :3085-3098 and parses at :1541-1599.  For every record r

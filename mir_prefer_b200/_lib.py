@@ -97,6 +97,11 @@ class FillPlan(C.Structure):
                 ("n_units", C.c_int32), ("dmax", C.c_int32), ("band_cells", C.c_uint64)]
 
 
+class Segment(C.Structure):
+    _fields_ = [("tile_first", C.c_int32), ("tile_last", C.c_int32), ("halo_tiles", C.c_int32), ("row_first", C.c_int32),
+                ("row_last", C.c_int32), ("reserved", C.c_int32), ("device_bytes", C.c_uint64)]
+
+
 # every symbol include/mirfold.h declares
 EXPORTS = ["mirfold_open", "mirfold_close", "mirfold_fold", "mirfold_fold_device", "mirfold_debug_matrices",
            "mirfold_free_result", "mirfold_strerror", "mirfold_last_error", "mirfold_version", "mirfold_duplex",
@@ -104,7 +109,7 @@ EXPORTS = ["mirfold_open", "mirfold_close", "mirfold_fold", "mirfold_fold_device
            "mirfold_classify", "mirfold_free_structures", "mirfold_fold_stream", "mirfold_batch_upload", "mirfold_batch_fold",
            "mirfold_batch_free", "mirfold_plan_shards", "mirfold_int_peak2", "mirfold_fold_candidates", "mirfold_free_candidates", "mirfold_fold_text", "mirfold_plan_fill_units",
            "mirfold_genome_upload", "mirfold_genome_free", "mirfold_fold_regions", "mirfold_fold_regions_stream",
-           "mirfold_fold_candidates_regions", "mirfold_shuffle_test", "mirfold_shuffle_sequences"]
+           "mirfold_fold_candidates_regions", "mirfold_shuffle_test", "mirfold_shuffle_sequences", "mirfold_plan_segments"]
 
 _lib = None
 
@@ -172,6 +177,9 @@ def load():
     if hasattr(lib, "mirfold_plan_fill_units"):
         lib.mirfold_plan_fill_units.argtypes = [C.c_uint32, C.c_int, C.POINTER(FillPlan)]
         lib.mirfold_plan_fill_units.restype = C.c_int
+    if hasattr(lib, "mirfold_plan_segments"):
+        lib.mirfold_plan_segments.argtypes = [C.c_uint32, C.c_int, C.c_uint64, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]
+        lib.mirfold_plan_segments.restype = C.c_int
     if os.environ.get("MIRFOLD_LIB_PATH") and not all(hasattr(lib, x) for x in ("mirfold_fold_candidates", "mirfold_fold_text")):
         _lib = lib      # an older A/B build of the library: the entry points below are not in it
         return lib

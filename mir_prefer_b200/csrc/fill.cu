@@ -1515,6 +1515,98 @@ __global__ void __launch_bounds__(NW * 32) k_f3_cta(const LocusDesc *__restrict_
     }
 }
 
+// k_f3_cta over rows row_hi down to row_lo of one segment of a segmented locus (host.cu, fold_segmented), below rows whose
+// f3 earlier segments left in F.  The descriptor is the locus' suffix from the segment's first tile on, so every band offset
+// is relative to the segment's buffer.  A copy of k_f3_cta rather than a shared body: k_f3_cta keeps its exact code.
+template <int NW>
+__global__ void __launch_bounds__(NW * 32) k_f3_seg(const LocusDesc *__restrict__ loci, const unsigned char *__restrict__ codes,
+                                                    const int *__restrict__ Call, int *__restrict__ Fall,
+                                                    const DevParams *__restrict__ P, int win, int row_hi, int row_lo)
+{
+    __shared__ unsigned char sPair[64];
+    __shared__ int sD3[40], sD5[40];
+    __shared__ int sG[NW][32];
+    extern __shared__ __align__(16) unsigned char f3_dyn[];
+    int *sF = (int *)f3_dyn;                              // f3(ilo + k), k < win
+    unsigned char *sC = (unsigned char *)(sF + win);      // codes(ilo + k)
+    constexpr int NT = NW * 32;
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    if (tid < 64) sPair[tid] = P->pair[tid];
+    if (tid < 40) { sD3[tid] = P->dangle3[tid]; sD5[tid] = P->dangle5[tid]; }
+    const LocusDesc L = loci[blockIdx.x];
+    const int n = L.n, Ls = L.Ls, NS = L.stride;
+    const unsigned char *__restrict__ cd = codes + L.seq_off;
+    const int *__restrict__ C = Call + L.band_off;
+    int *F = Fall + L.seq_off;
+    const int AUp = P->TerminalAU;
+    constexpr int DS = 31;
+    const int slice = (max(Ls - DS + 1, 0) + NW - 1) / NW;
+    for (int ihi = row_hi; ihi >= row_lo; ihi -= 32) {
+        const int ilo = max(row_lo, ihi - 31);
+        __syncthreads();   // previous block's f3 stores (warp 0) are visible; sF/sC/sG free again
+        for (int k = tid; k < win; k += NT) {
+            const int pos = ilo + k;
+            sF[k] = (pos <= n + 2) ? F[pos] : 0;
+            sC[k] = (pos <= n + 2) ? cd[pos] : 0;
+        }
+        __syncthreads();
+        // ---- phase P: warp w takes spans [d0, d1]
+        int gout = MF_INF;
+        {
+            const int i = ilo + lane;
+            if (i <= ihi && slice > 0) {
+                const int dend = min(Ls, n - 1 - i);
+                const int d0 = DS + w * slice, d1 = min(dend, d0 + slice - 1);
+                if (d0 <= d1) {
+                    const int ci = sC[lane], si = ci & 7, s1i = ci >> 4, si1 = sC[lane + 1] & 7;
+                    const int *pa = C + band_row_base(L, i) + (d0 - 4) * NS;
+                    int jl = lane + d0;   // j - ilo
+#pragma unroll 4
+                    for (int d = d0; d <= d1; d++, jl++, pa += NS) {
+                        const int cA = pa[0], cB = pa[1 - NS];
+                        gout = min(gout, dev_f3_term(sPair, sD3, sD5, AUp, si, s1i, si1, sC[jl] & 7, sC[jl + 1] >> 4, d, Ls, cA, cB,
+                                                     sF[jl + 1], sF[jl + 2]));
+                    }
+                }
+            }
+        }
+        sG[w][lane] = gout;
+        __syncthreads();
+        if (w == 0) {
+#pragma unroll
+            for (int k = 1; k < NW; k++) gout = min(gout, sG[k][lane]);
+            // ---- phase S (as k_f3)
+            int Fw = sF[ihi + 1 - ilo + lane];
+            for (int i = ihi; i >= ilo; i--) {
+                const int d = lane, j = i + d;
+                const int *Ci = C + band_row_base(L, i);
+                const int f2 = __shfl_down_sync(0xffffffffu, Fw, 1);
+                const int ci = sC[i - ilo], si = ci & 7, s1i = ci >> 4, si1 = sC[i + 1 - ilo] & 7;
+                int best = MF_INF;
+                if (d >= 4 && d < DS && d <= Ls && j <= n - 1) {
+                    const int cA = Ci[(d - 4) * NS];
+                    const int cB = (d >= 5) ? Ci[(d - 5) * NS + 1] : MF_INF;
+                    best = dev_f3_term(sPair, sD3, sD5, AUp, si, s1i, si1, sC[j - ilo] & 7, sC[j + 1 - ilo] >> 4, d, Ls, cA, cB, Fw, f2);
+                }
+                if (lane == 31 && n <= i + Ls) {   // j == n: no f3 / dangle3 terms
+                    const int dn = n - i, sj = cd[n] & 7;
+                    int t = (dn < Ls) ? sPair[si * 8 + sj] : 0;
+                    if (t) best = min(best, Ci[(dn - 4) * NS] + (t > 2 ? AUp : 0));
+                    t = (dn - 1 >= 4) ? sPair[si1 * 8 + sj] : 0;
+                    if (t) best = min(best, Ci[(dn - 5) * NS + 1] + sD5[t * 5 + s1i] + (t > 2 ? AUp : 0));
+                }
+                best = warp_min(best);
+                const int g = __shfl_sync(0xffffffffu, gout, i - ilo);
+                const int fnext = __shfl_sync(0xffffffffu, Fw, 0);   // f3(i+1)
+                const int fi = min(fnext, min(best, g));
+                if (lane == 0) F[i] = fi;
+                Fw = __shfl_up_sync(0xffffffffu, Fw, 1);
+                if (lane == 0) Fw = fi;
+            }
+        }
+    }
+}
+
 // loci are sorted by descending length: the first n_long (n > MF_TILE_LEN) get a CTA each
 cudaError_t launch_f3(const LocusDesc *loci, int nloci, int n_long, int max_Ls, const unsigned char *codes, const int *C, int *F,
                       const DevParams *P, cudaStream_t st)
@@ -1532,5 +1624,15 @@ cudaError_t launch_f3(const LocusDesc *loci, int nloci, int n_long, int max_Ls, 
         const int warps_per_block = 4;
         k_f3<<<(rest + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, st>>>(loci + n_long, rest, codes, C, F, P);
     }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_f3_rows(const LocusDesc *locus, int Ls, int row_hi, int row_lo, const unsigned char *codes, const int *C, int *F,
+                           const DevParams *P, cudaStream_t st)
+{
+    if (row_hi < row_lo) return cudaSuccess;
+    constexpr int NW = 8;
+    const int win = (std::max(Ls, 32) + 40 + 3) & ~3;
+    k_f3_seg<NW><<<1, NW * 32, (size_t)win * 5, st>>>(locus, codes, C, F, P, win, row_hi, row_lo);
     return cudaGetLastError();
 }

@@ -98,6 +98,7 @@ struct Lane {
     cudaStream_t side = nullptr;   // small fill buckets run here, concurrently with the big one
     DBuf units, raw, loci, codes, F, C, M, Mp, Ib, ring, fillflags, tbcount, tbbase, listoff, startlist, scan_in, scan_out, scan_tmp;
     DBuf slots, tblen, tbstart, tblocus, tbflag, tbenergy, stackscr, fail, ssoff, hitidx;
+    DBuf segstate;   // segmented loci: the emission plan's state carried from segment to segment (k_plan_seg)
     DBuf o_hits, o_arena, bounds, totals;
     DBuf c_counts, c_soff, c_structs, c_nq, c_sbytes, c_voff, c_aoff, c_lsb, c_verd, c_vmat, c_arena, c_sout;   // fused stage 1 + 3
     HBuf hc_structs, hc_arena, hc_verd, hc_vmat, hc_voff, hc_lsb;
@@ -126,7 +127,7 @@ struct Lane {
         DBuf *all[] = {&units, &raw, &loci, &codes, &F, &C, &M, &Mp, &Ib, &ring, &fillflags, &tbcount, &tbbase, &listoff, &startlist, &scan_in,
                        &scan_out, &scan_tmp, &slots, &tblen, &tbstart, &tblocus, &tbflag, &tbenergy, &stackscr, &fail,
                        &ssoff, &hitidx, &o_hits, &o_arena, &bounds, &totals, &c_counts, &c_soff, &c_structs, &c_nq, &c_sbytes,
-                       &c_voff, &c_aoff, &c_lsb, &c_verd, &c_vmat, &c_arena, &c_sout};
+                       &c_voff, &c_aoff, &c_lsb, &c_verd, &c_vmat, &c_arena, &c_sout, &segstate};
         for (DBuf *b : all) b->release();
         HBuf *hall[] = {&h_raw, &h_loci, &h_units, &h_listoff, &h_small, &h_out, &h_hits, &h_arena, &hc_structs, &hc_arena, &hc_verd,
                         &hc_vmat, &hc_voff, &hc_lsb};
@@ -441,6 +442,18 @@ static int unit_bucket(const LocusDesc &u)   // index into FillLaunch::bucket_fi
 {
     return !is_bucket_stride(u.stride) ? 0 : u.stride == MF_TILE_LEN_BIG ? 1 : u.stride == MF_TILE_LEN ? 2 : u.stride == 352 ? 3 : 4;
 }
+// fill unit of tile t of a tiled locus: TL bases from a_t + 1, band at the locus' band_off + t tiles
+LocusDesc tile_unit(const LocusDesc &d, int t)
+{
+    LocusDesc u = d;
+    const int TL = d.stride;
+    const int a = std::min(t * d.tile_step, d.n - TL);
+    u.n = TL; u.Ls = std::min(d.Ls, TL); u.dmax = d.dmax;
+    u.seq_off = d.seq_off + (unsigned long long)a;
+    u.band_off = d.band_off + (unsigned long long)t * band_elems(TL, d.dmax);
+    u.tile_last = 0;
+    return u;
+}
 // Fill units of a chunk: one per untiled locus, one per tile otherwise, sorted by (bucket, descending n)
 // so that the stride buckets are contiguous.  Assigns ring offsets; returns ring elements.
 unsigned long long build_fill_units(const LocusDesc *loci, int nl, std::vector<LocusDesc> &units, int bucket_first[6], int &max_n)
@@ -451,16 +464,7 @@ unsigned long long build_fill_units(const LocusDesc *loci, int nl, std::vector<L
         const LocusDesc &d = loci[k];
         if (d.dmax < 4) continue;   // n < 5 never reaches here; keeps the kernels' assumptions explicit
         if (d.tile_last == 0) { units.push_back(d); continue; }
-        for (int t = 0; t <= d.tile_last; t++) {
-            LocusDesc u = d;
-            const int TL = d.stride;
-            const int a = std::min(t * d.tile_step, d.n - TL);
-            u.n = TL; u.Ls = std::min(d.Ls, TL); u.dmax = d.dmax;
-            u.seq_off = d.seq_off + (unsigned long long)a;
-            u.band_off = d.band_off + (unsigned long long)t * band_elems(TL, d.dmax);
-            u.tile_last = 0;
-            units.push_back(u);
-        }
+        for (int t = 0; t <= d.tile_last; t++) units.push_back(tile_unit(d, t));
     }
     std::stable_sort(units.begin(), units.end(), [](const LocusDesc &a, const LocusDesc &b) {
         const int ba = unit_bucket(a), bb = unit_bucket(b);
@@ -482,15 +486,55 @@ unsigned long long build_fill_units(const LocusDesc *loci, int nl, std::vector<L
     return ring_acc;
 }
 
+// estimated device bytes of one traceback (slot, stack, per-traceback ints)
+static size_t traceback_bytes(int n, int L)
+{
+    return (size_t)((std::min(L, n) + 8) & ~3) + (size_t)(std::min(L, n) / 4 + 16) * 8 + 64;
+}
 // device bytes one locus needs on a lane: band (C, M, Mp), ring, descriptors, sequence-sized arrays and an
 // estimate of the per-traceback buffers (slots, stacks, per-traceback ints: about one traceback per 8 nt)
 size_t locus_bytes(int n, int L)
 {
     LocusDesc d{};
     const unsigned long long be = shape_locus(d, n, L);
-    const size_t per_tb = (size_t)((std::min(L, n) + 8) & ~3) + (size_t)(std::min(L, n) / 4 + 16) * 8 + 64;
     return (size_t)be * 13 + (size_t)(d.tile_last + 1) * unit_ring_elems(d.stride) * 4 +
-           (size_t)(d.tile_last + 2) * sizeof(LocusDesc) + (size_t)n * 16 + (size_t)(n / 8 + 2) * per_tb + 4096;
+           (size_t)(d.tile_last + 2) * sizeof(LocusDesc) + (size_t)n * 16 + (size_t)(n / 8 + 2) * traceback_bytes(n, L) + 4096;
+}
+
+// ---- segmented loci.  A tiled locus larger than the device budget is folded in segments from its 3' end: a segment owns
+// the tiles [t0, t1] and also holds `halo` tiles above t1, those owning rows up to (its last owned row + L* + 1) -- what f3
+// (row i reads only row i's owner tile) and a traceback from a start in its owned rows or the row above them can read.
+// The sequence-sized arrays (codes, F, raw) stay whole; band, rings and traceback scratch are per segment.
+struct SegPlan {
+    int t0, t1, halo;      // owned tiles [t0, t1], tiles t1+1 .. t1+halo above
+    int row_lo, row_hi;    // owned rows
+    size_t bytes;          // device bytes while the segment runs (the locus' sequence-sized arrays included)
+};
+static int64_t tile_last_row(const LocusDesc &d, int t) { return t == d.tile_last ? d.n : (int64_t)(t + 1) * d.tile_step; }
+static size_t segment_bytes(const LocusDesc &d, int L, int t0, int t1, int halo)
+{
+    const size_t tiles = (size_t)(t1 + halo - t0 + 1);
+    const int64_t rows = tile_last_row(d, t1) - (int64_t)t0 * d.tile_step;
+    return tiles * band_elems(d.stride, d.dmax) * 13 + tiles * unit_ring_elems(d.stride) * 4 + (tiles + 2) * sizeof(LocusDesc) +
+           (size_t)d.n * 16 + (size_t)(rows / 8 + 2) * traceback_bytes(d.n, L) + 4096;
+}
+// Segments in the order they run (3' end first).  A locus that fits `budget` (or is one unit) is one segment; otherwise each
+// segment takes as many owned tiles as fit, at least one.
+void plan_segments(int n, int L, size_t budget, std::vector<SegPlan> &out)
+{
+    out.clear();
+    LocusDesc d{};
+    shape_locus(d, n, L);
+    const size_t whole = locus_bytes(n, L);
+    if (d.tile_last == 0 || whole <= budget) { out.push_back(SegPlan{0, d.tile_last, 0, 1, n, whole}); return; }
+    for (int t1 = d.tile_last; t1 >= 0;) {
+        const int64_t hi = tile_last_row(d, t1), reach = std::min<int64_t>(n, hi + d.Ls + 1);
+        const int halo = (int)std::min<int64_t>((reach - 1) / d.tile_step, d.tile_last) - t1;
+        int t0 = t1;
+        while (t0 > 0 && segment_bytes(d, L, t0 - 1, t1, halo) <= budget) t0--;
+        out.push_back(SegPlan{t0, t1, halo, t0 * d.tile_step + 1, (int)hi, segment_bytes(d, L, t0, t1, halo)});
+        t1 = t0 - 1;
+    }
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -502,7 +546,7 @@ struct DevicePipeline {
     const uint64_t *raw_off;      // ... at these per-record offsets
     DevOut &out;
     std::vector<Locus> loci;      // descending DP cells
-    struct Chunk { size_t begin, end; };
+    struct Chunk { size_t begin, end; bool segmented; };
     std::vector<Chunk> chunks;
     int nlanes_ = 1;
     HostTimer ht;
@@ -546,12 +590,16 @@ struct DevicePipeline {
         bool ok = true;
         if (!chunks.empty()) {
             CK(cudaEventRecord(D.ev_first, D.lane[0].s_lo));
-            ok = front(D.lane[0], 0);
+            ok = chunks[0].segmented || front(D.lane[0], 0);
             for (size_t k = 0; ok && k < chunks.size(); k++) {
                 Lane &Ln = D.lane[k % nlanes];
-                if (nlanes == 2 && k + 1 < chunks.size()) ok = front(D.lane[(k + 1) % 2], k + 1);   // its fill overlaps everything below
-                ok = ok && middle(Ln) && back(Ln, k + 1 == chunks.size());
-                if (nlanes == 1 && ok && k + 1 < chunks.size()) ok = front(Ln, k + 1);
+                const bool pre = k + 1 < chunks.size() && !chunks[k + 1].segmented;   // a segmented chunk has no front
+                if (chunks[k].segmented) ok = fold_segmented(Ln, k) && (!pre || front(D.lane[(k + 1) % nlanes], k + 1));
+                else {
+                    if (nlanes == 2 && pre) ok = front(D.lane[(k + 1) % 2], k + 1);   // its fill overlaps everything below
+                    ok = ok && middle(Ln) && back(Ln, k + 1 == chunks.size());
+                    if (nlanes == 1 && ok && pre) ok = front(Ln, k + 1);
+                }
                 if (J.cb_abort && J.cb_abort->load()) { out.err = MIRFOLD_ERR_CALLBACK; out.errmsg = "chunk callback returned non-zero"; ok = false; }
             }
             for (int l = 0; ok && l < nlanes; l++) ok = retire(D.lane[l]);
@@ -587,17 +635,17 @@ struct DevicePipeline {
             if (loci[k].n != last_n) { last_n = loci[k].n; last_b = locus_bytes(last_n, J.L); }
             lb[k] = last_b; total += last_b;
         }
-        const size_t lane_budget = std::max<size_t>(D.mem_budget / (J.serial ? 1 : 2), 1);
+        const size_t lane_budget = lane_bytes();
         size_t nch = (total + lane_budget - 1) / lane_budget;
         if (J.sink != SINK_NONE || nch > 1) nch = std::max<size_t>(nch, std::min<size_t>(64, (size_t)(total_cells / cells_per_chunk)));
         nch = std::max<size_t>(nch, 1);
         const size_t target = std::min(lane_budget, total / nch + 1);
         size_t b = 0, acc = 0;
         for (size_t k = 0; k < loci.size(); k++) {
-            if (k > b && acc + lb[k] > target) { chunks.push_back({b, k}); b = k; acc = 0; }
+            if (k > b && acc + lb[k] > target) { chunks.push_back({b, k, false}); b = k; acc = 0; }
             acc += lb[k];
         }
-        chunks.push_back({b, loci.size()});
+        chunks.push_back({b, loci.size(), false});
         // The download of a device's LAST chunk is the only one nothing overlaps (154 MB per device take 11.6 ms when eight GPUs
         // write into host memory at once): cut the last chunk 80 : 20 so that only the small tail's download is exposed.
         if (J.sink != SINK_NONE && J.sink != SINK_TOTALS) {
@@ -610,11 +658,20 @@ struct DevicePipeline {
                 while (cut < last.end && acc2 < cells - cells / 5) acc2 += loci[cut++].cells;
                 if (cut > last.begin && cut < last.end) {
                     chunks.back().end = cut;
-                    chunks.push_back({cut, last.end});
+                    chunks.push_back({cut, last.end, false});
                 }
             }
         }
+        // a tiled locus over the device's whole budget (always a chunk of its own: it exceeds the target) runs in segments
+        for (Chunk &c : chunks)
+            if (c.end == c.begin + 1 && lb[c.begin] > D.mem_budget) {
+                LocusDesc d{};
+                shape_locus(d, loci[c.begin].n, J.L);
+                c.segmented = d.tile_last > 0;
+            }
     }
+
+    size_t lane_bytes() const { return std::max<size_t>(D.mem_budget / (J.serial ? 1 : 2), 1); }
 
     // ---- front: descriptors, upload, encode, band fill, f3, emission plan (everything up to the first host sync)
     bool front(Lane &Ln, size_t ci)
@@ -873,7 +930,7 @@ struct DevicePipeline {
     }
 
     // ---- fused stages 1 + 3 on the chunk's packed hits (still in HBM): classify, duplex verdicts, compact download
-    bool back_candidates(Lane &Ln, bool last_chunk)
+    bool back_candidates(Lane &Ln, bool last_chunk, bool bounds_ready = false)
     {
         cudaStream_t hi = Ln.s_hi;
         TraceBuffers &tb = Ln.tb;
@@ -882,7 +939,8 @@ struct DevicePipeline {
         const uint64_t nhits = Ln.nhits;
         const CandArgs &ca = *J.cand;
         unsigned long long *hs = Ln.h_small.as<unsigned long long>();
-        if (tb.ntb) {
+        if (bounds_ready) {   // a segmented locus: its staged hits, bounds and total were uploaded
+        } else if (tb.ntb) {
             k_gather_bounds<<<(nl + 1 + 255) / 256, 256, 0, hi>>>(tb.tb_base, Ln.hitidx.as<unsigned long long>(), tb.loci, tb.F,
                                                                   Ln.bounds.as<unsigned long long>(), Ln.totals.as<int>(), nl);
             CK(cudaGetLastError());
@@ -939,6 +997,278 @@ struct DevicePipeline {
         CK(cudaMemcpyAsync(Ln.hc_voff.p, Ln.c_voff.p, (ns + 1) * 8, cudaMemcpyDeviceToHost, hi));
         CK(cudaMemcpyAsync(Ln.hc_lsb.p, Ln.c_lsb.p, (size_t)(nl + 1) * 8, cudaMemcpyDeviceToHost, hi));
         out.st.d2h_bytes += ns * sizeof(mirfold_structure) + nb + nv * (sizeof(mirfold_duplex_verdict) + 4) + (ns + 1) * 8 + (uint64_t)(nl + 1) * 8 + 64;
+        return true;
+    }
+
+    // ---- a segmented locus (plan_segments): every segment fills its tiles, runs f3 over its owned rows, the emission plan
+    // from the state the segment above left, the tracebacks from its starts and the emission decisions, then packs and
+    // downloads its hits.  Each segment is addressed as the locus' suffix from its first tile's origin on (the same tiles,
+    // rows and f3 shifted by that origin), so the band buffer starts at the segment's first tile.  The last traceback of a
+    // segment is decided against the first one of the next: its slot, start and length are carried over, not traced again.
+    // The record's hits are staged on the host and published as one record once its last segment is done.
+    bool fold_segmented(Lane &Ln, size_t ci)
+    {
+        if (!retire(Ln)) return false;
+        cudaStream_t st = Ln.s_lo;
+        const Locus &l = loci[chunks[ci].begin];
+        const int n = l.n;
+        const bool last_chunk = ci + 1 == chunks.size();
+        Prep &P = Ln.prep;
+        P = Prep{};
+        P.cb = chunks[ci].begin; P.ce = chunks[ci].end; P.nl = 1;
+        LocusDesc d{};
+        shape_locus(d, n, J.L);
+        d.rec = (int)l.rec;
+        d.raw_off = d_raw ? raw_off[l.rec] : 0;
+        P.max_Ls = d.Ls;
+        const int S = d.tile_step, TL = d.stride;
+        std::vector<SegPlan> segs;
+        plan_segments(n, J.L, lane_bytes(), segs);
+        // whole-locus arrays: raw, codes, F; descriptors [0] = the locus, [1] = the running segment's suffix
+        CK(Ln.h_loci.ensure(2 * sizeof(LocusDesc)));
+        CK(Ln.loci.ensure(2 * sizeof(LocusDesc)));
+        CK(Ln.codes.ensure((size_t)n + 3));
+        CK(Ln.F.ensure(((size_t)n + 3) * 4));
+        CK(Ln.segstate.ensure(16));
+        CK(Ln.fail.ensure(4));
+        CK(Ln.listoff.ensure(8));
+        CK(Ln.tbbase.ensure(16));
+        CK(Ln.tbcount.ensure(4));
+        CK(Ln.h_small.ensure(256));
+        LocusDesc *hl = Ln.h_loci.as<LocusDesc>();
+        hl[0] = d;
+        const LocusDesc *dl = Ln.loci.as<LocusDesc>();
+        CK(cudaEventRecord(Ln.ev[0], st));
+        const char *raw_dev = d_raw;
+        if (!d_raw) {
+            CK(Ln.raw.ensure((size_t)n));
+            CK(cudaMemcpyAsync(Ln.raw.p, J.seqs + J.h_off[l.rec], (size_t)n, cudaMemcpyHostToDevice, st));
+            out.st.h2d_bytes += (uint64_t)n;
+            raw_dev = Ln.raw.as<char>();
+        }
+        CK(cudaMemcpyAsync(Ln.loci.p, hl, sizeof(LocusDesc), cudaMemcpyHostToDevice, st));
+        CK(cudaMemsetAsync(Ln.segstate.p, 0, 16, st));   // fnext = f3(n-3) = 0, do_bt = have_prev = 0
+        CK(cudaMemsetAsync(Ln.fail.p, 0, 4, st));
+        CK(cudaMemsetAsync(Ln.listoff.p, 0, 8, st));
+        CK(cudaEventRecord(Ln.ev[1], st));
+        CK(launch_prepare(raw_dev, dl, 1, (unsigned long long)n + 3, Ln.codes.as<unsigned char>(), Ln.F.as<int>(), st));
+        out.st.kernel_launches += 1;
+        std::vector<mirfold_hit> hits;   // the record's hits in print order; ss_off into `arena`
+        std::vector<char> arena;
+        std::vector<char> carry_slot;    // the last traceback of the segment above: slot, length, absolute start
+        int carry_len = 0, carry_start = 0;
+        bool carry = false;
+        const int slot_stride = (d.Ls + 4 + 3) & ~3, stack_cap = d.Ls / 4 + 16;
+        unsigned long long *hs = Ln.h_small.as<unsigned long long>();
+        for (size_t sg = 0; sg < segs.size(); sg++) {
+            const SegPlan &g = segs[sg];
+            const bool last = sg + 1 == segs.size();
+            const int t_hi = g.t1 + g.halo, ntiles = t_hi - g.t0 + 1;
+            const int a = std::min(g.t0 * S, n - TL);   // the first tile's origin: suffix row k is locus row a + k
+            LocusDesc ds = d;
+            ds.n = n - a; ds.seq_off = d.seq_off + (unsigned long long)a; ds.band_off = 0; ds.tile_last = d.tile_last - g.t0;
+            hl[1] = ds;
+            // ---- fill of the segment's tiles (one bucket), f3 over its owned rows
+            const size_t be = (size_t)ntiles * band_elems(TL, d.dmax);
+            CK(Ln.h_units.ensure(sizeof(LocusDesc) * (size_t)ntiles + 64));
+            LocusDesc *hu = Ln.h_units.as<LocusDesc>();
+            for (int t = g.t0; t <= t_hi; t++) {
+                LocusDesc u = tile_unit(d, t);
+                u.band_off = (unsigned long long)(t - g.t0) * band_elems(TL, d.dmax);
+                u.ring_off = (unsigned long long)(t - g.t0) * unit_ring_elems(TL);
+                hu[t - g.t0] = u;
+            }
+            CK(Ln.C.ensure(be * 4));
+            CK(Ln.M.ensure(be * 4));
+            CK(Ln.Ib.ensure(be + 256));
+            if (!J.force_wide) CK(Ln.Mp.ensure(be * 4 + 4096));
+            CK(Ln.ring.ensure((size_t)ntiles * unit_ring_elems(TL) * 4));
+            CK(Ln.units.ensure(sizeof(LocusDesc) * (size_t)ntiles + 64));
+            CK(Ln.fillflags.ensure((size_t)ntiles * 4 + 4));
+            CK(cudaMemcpyAsync(Ln.units.p, hu, sizeof(LocusDesc) * (size_t)ntiles, cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(Ln.loci.as<LocusDesc>() + 1, &hl[1], sizeof(LocusDesc), cudaMemcpyHostToDevice, st));
+            CK(cudaMemsetAsync(Ln.fillflags.p, 0, (size_t)ntiles * 4 + 4, st));
+            out.st.h2d_bytes += sizeof(LocusDesc) * (uint64_t)(ntiles + 1);
+            out.st.fill_units += (uint64_t)ntiles;
+            CK(cudaEventRecord(Ln.ev[2], st));
+            FillLaunch fa{Ln.units.as<LocusDesc>(), ntiles, TL, Ln.codes.as<unsigned char>(), Ln.C.as<int>(), Ln.M.as<int>(), Ln.ring.as<int>(),
+                          Ln.Ib.as<unsigned char>(), Ln.Mp.as<unsigned int>(), D.dP, {0, 0, 0, 0, 0, 0}, Ln.fillflags.as<int>(), J.force_wide ? 1 : 0,
+                          env_opts() | (J.L >= MF_DYNW_MIN_SPAN ? 8 : 0)};
+            const int bucket = unit_bucket(hu[0]);
+            for (int b = 0; b < 6; b++) fa.bucket_first[b] = b <= bucket ? 0 : ntiles;
+            CK(launch_fill(fa, st));
+            CK(cudaEventRecord(Ln.ev[3], st));
+            const int row_lo = g.row_lo - a, row_hi = std::min(g.row_hi, n - 4) - a;   // owned rows with an f3 / plan step
+            CK(launch_f3_rows(dl + 1, d.Ls, row_hi, row_lo, Ln.codes.as<unsigned char>(), Ln.C.as<int>(), Ln.F.as<int>(), D.dP, st));
+            CK(cudaEventRecord(Ln.ev[4], st));
+            out.st.kernel_launches += (J.force_wide ? 1 : 2) + (row_hi >= row_lo ? 1 : 0);
+            if (J.sink == SINK_TOTALS) {
+                CK(cudaEventRecord(Ln.ev[5], st));
+                CK(cudaEventRecord(Ln.ev[6], st));
+                CK(cudaStreamSynchronize(st));
+                segment_times(Ln);
+                continue;
+            }
+            // ---- emission plan over the owned rows, resumed from the segment above
+            const int *Fs = Ln.F.as<int>() + ds.seq_off;
+            CK(Ln.startlist.ensure(((size_t)(g.row_hi - g.row_lo + 1) / 2 + 4) * 4));
+            CK(launch_plan_seg(Fs, row_hi, row_lo, g.row_lo == 1 ? 1 : 0, Ln.segstate.as<int>(), Ln.startlist.as<int>(),
+                               Ln.tbbase.as<unsigned long long>(), Ln.tbcount.as<int>(), st));
+            CK(cudaMemcpyAsync(&hs[0], Ln.tbbase.as<unsigned long long>() + 1, 8, cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            const int nc = carry ? 1 : 0;
+            const unsigned long long m = hs[0], ntb = m + (unsigned long long)nc;
+            out.st.tracebacks += m;
+            // ---- tracebacks of the segment's starts behind the carried entry 0
+            CK(Ln.slots.ensure((size_t)ntb * slot_stride + 16));
+            CK(Ln.tblen.ensure((size_t)ntb * 4 + 16)); CK(Ln.tbstart.ensure((size_t)ntb * 4 + 16));
+            CK(Ln.tblocus.ensure((size_t)ntb * 4 + 16)); CK(Ln.tbflag.ensure((size_t)ntb * 4 + 16));
+            CK(Ln.tbenergy.ensure((size_t)ntb * 4 + 16));
+            CK(Ln.stackscr.ensure((size_t)ntb * stack_cap * 8 + 16));
+            CK(Ln.ssoff.ensure((size_t)(ntb + 1) * 8)); CK(Ln.hitidx.ensure((size_t)(ntb + 1) * 8));
+            CK(Ln.scan_in.ensure((size_t)(ntb + 1) * 8)); CK(Ln.scan_out.ensure((size_t)(ntb + 1) * 8));
+            TraceBuffers tb{};
+            tb.loci = dl + 1; tb.nloci = 1; tb.codes = Ln.codes.as<unsigned char>();
+            tb.C = Ln.C.as<int>(); tb.M = Ln.M.as<int>(); tb.F = Ln.F.as<int>(); tb.Ib = Ln.Ib.as<unsigned char>(); tb.P = D.dP;
+            tb.tb_count = Ln.tbcount.as<int>(); tb.tb_base = Ln.tbbase.as<unsigned long long>();
+            tb.list_off = Ln.listoff.as<unsigned long long>(); tb.tb_start_list = Ln.startlist.as<int>();
+            tb.fail_flag = Ln.fail.as<int>();
+            tb.slot_stride = slot_stride; tb.stack_cap = stack_cap; tb.code_win = (d.Ls + 8 + 15) & ~15;
+            tb.slots = Ln.slots.as<char>(); tb.tb_len = Ln.tblen.as<int>(); tb.tb_start = Ln.tbstart.as<int>();
+            tb.tb_locus = Ln.tblocus.as<int>(); tb.tb_flag = Ln.tbflag.as<int>(); tb.tb_energy = Ln.tbenergy.as<int>();
+            tb.stack_scratch = Ln.stackscr.as<int>();
+            if (carry) {
+                CK(cudaMemcpyAsync(tb.slots, carry_slot.data(), (size_t)slot_stride, cudaMemcpyHostToDevice, st));
+                CK(cudaMemcpyAsync(tb.tb_len, &carry_len, 4, cudaMemcpyHostToDevice, st));
+                CK(cudaMemcpyAsync(tb.tb_start, &carry_start, 4, cudaMemcpyHostToDevice, st));
+            }
+            TraceBuffers tv = tb;   // the segment's own tracebacks: entries nc .. ntb-1
+            tv.ntb = m;
+            tv.slots += (size_t)nc * slot_stride; tv.tb_len += nc; tv.tb_start += nc; tv.tb_locus += nc; tv.tb_flag += nc; tv.tb_energy += nc;
+            tv.stack_scratch += (size_t)nc * stack_cap * 2;
+            CK(launch_traceback(tv, st));
+            tb.ntb = ntb;
+            int *abs_start = Ln.tblocus.as<int>();
+            CK(launch_emit_seg(tb, nc, a, last ? 1 : 0, Ln.F.as<int>() + d.seq_off, n, abs_start, st));
+            uint64_t nhits = 0, abytes = 0;
+            if (ntb) {
+                k_emit_sizes<<<(unsigned)((ntb + 1 + 255) / 256), 256, 0, st>>>(tb.tb_flag, tb.tb_len, Ln.scan_in.as<unsigned long long>(),
+                                                                              Ln.scan_out.as<unsigned long long>(), ntb);
+                CK(cudaGetLastError());
+                CK(exclusive_scan(Ln, Ln.scan_in.as<unsigned long long>(), Ln.ssoff.as<unsigned long long>(), (size_t)ntb + 1, st));
+                CK(exclusive_scan(Ln, Ln.scan_out.as<unsigned long long>(), Ln.hitidx.as<unsigned long long>(), (size_t)ntb + 1, st));
+                CK(cudaMemcpyAsync(&hs[1], Ln.ssoff.as<unsigned long long>() + ntb, 8, cudaMemcpyDeviceToHost, st));
+                CK(cudaMemcpyAsync(&hs[2], Ln.hitidx.as<unsigned long long>() + ntb, 8, cudaMemcpyDeviceToHost, st));
+                out.st.kernel_launches += 8;
+            }
+            CK(cudaMemcpyAsync(&hs[3], Ln.fail.p, 4, cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            if (*(int *)&hs[3]) { out.err = MIRFOLD_ERR_BACKTRACK; out.errmsg = "traceback found no decomposition"; return false; }
+            if (ntb) { abytes = hs[1]; nhits = hs[2]; }
+            // ---- pack and download the printed hits; carry the undecided last traceback to the next segment
+            CK(Ln.o_hits.ensure(nhits * sizeof(mirfold_hit) + 16));
+            CK(Ln.o_arena.ensure(abytes + 16));
+            CK(Ln.h_hits.ensure(nhits * sizeof(mirfold_hit) + 16));
+            CK(Ln.h_arena.ensure(abytes + 16));
+            TraceBuffers tp = tb;
+            tp.tb_start = abs_start;
+            CK(launch_pack(tp, Ln.ssoff.as<unsigned long long>(), Ln.hitidx.as<unsigned long long>(), Ln.o_arena.as<char>(),
+                           Ln.o_hits.as<mirfold_hit>(), (unsigned long long)arena.size(), st));
+            CK(cudaEventRecord(Ln.ev[5], st));
+            if (nhits) CK(cudaMemcpyAsync(Ln.h_hits.p, Ln.o_hits.p, nhits * sizeof(mirfold_hit), cudaMemcpyDeviceToHost, st));
+            if (abytes) CK(cudaMemcpyAsync(Ln.h_arena.p, Ln.o_arena.p, abytes, cudaMemcpyDeviceToHost, st));
+            carry = !last && ntb > 0;
+            if (carry) {
+                carry_slot.resize((size_t)slot_stride);
+                CK(cudaMemcpyAsync(carry_slot.data(), tb.slots + (ntb - 1) * slot_stride, (size_t)slot_stride, cudaMemcpyDeviceToHost, st));
+                CK(cudaMemcpyAsync(&carry_len, tb.tb_len + (ntb - 1), 4, cudaMemcpyDeviceToHost, st));
+                CK(cudaMemcpyAsync(&carry_start, abs_start + (ntb - 1), 4, cudaMemcpyDeviceToHost, st));
+            }
+            CK(cudaEventRecord(Ln.ev[6], st));
+            CK(cudaStreamSynchronize(st));
+            out.st.kernel_launches += 1 + (m ? 1 : 0) + (ntb ? 2 : 0);   // k_plan_seg, k_traceback, k_emit_seg, k_pack
+            out.st.d2h_bytes += nhits * sizeof(mirfold_hit) + abytes + 32;
+            hits.insert(hits.end(), Ln.h_hits.as<mirfold_hit>(), Ln.h_hits.as<mirfold_hit>() + nhits);
+            arena.insert(arena.end(), Ln.h_arena.as<char>(), Ln.h_arena.as<char>() + abytes);
+            segment_times(Ln);
+        }
+        int total = 0;
+        CK(cudaMemcpyAsync(&total, Ln.F.as<int>() + d.seq_off + 1, 4, cudaMemcpyDeviceToHost, st));
+        if (last_chunk) CK(cudaEventRecord(D.ev_last, st));
+        CK(cudaStreamSynchronize(st));
+        out.st.d2h_bytes += 4;
+        ht.mark("segmented locus");
+        return publish_segmented(Ln, l.rec, hits, arena, total, last_chunk);
+    }
+
+    void segment_times(Lane &Ln)
+    {
+        float ms = 0;
+        cudaEventElapsedTime(&ms, Ln.ev[2], Ln.ev[3]); out.st.ms_fill += ms;
+        cudaEventElapsedTime(&ms, Ln.ev[3], Ln.ev[4]); out.st.ms_f3 += ms;
+        cudaEventElapsedTime(&ms, Ln.ev[4], Ln.ev[5]); out.st.ms_trace += ms;
+        cudaEventElapsedTime(&ms, Ln.ev[5], Ln.ev[6]); out.st.ms_d2h += ms;
+    }
+
+    // the segmented record's staged hits (ss_off relative to its own arena) into the call's sink, as one record
+    bool publish_segmented(Lane &Ln, uint32_t r, const std::vector<mirfold_hit> &hits, const std::vector<char> &arena, int total,
+                           bool last_chunk)
+    {
+        const uint64_t nh = hits.size(), ab = arena.size();
+        float ms = 0;
+        cudaEventElapsedTime(&ms, Ln.ev[0], Ln.ev[1]); out.st.ms_h2d += ms;
+        if (J.sink == SINK_TOTALS) { J.totals[r] = total; return true; }
+        out.nhits += nh;
+        out.arena_bytes += ab;
+        if (J.sink == SINK_SHARED) {
+            SharedOut &S = *J.shared;
+            uint64_t hb = 0, abase = 0;
+            mirfold_hit *dh;
+            char *da;
+            std::unique_ptr<OverflowChunk> O;
+            if (S.reserve(nh, ab, hb, abase)) { dh = S.hits.as<mirfold_hit>() + hb; da = S.arena.as<char>() + abase; }
+            else {
+                O.reset(new OverflowChunk());
+                CK(O->hits.ensure(nh * sizeof(mirfold_hit) + 16));
+                CK(O->arena.ensure(ab + 16));
+                O->nhits = nh; O->abytes = ab;
+                O->recs = {r}; O->begin = {0}; O->count = {(uint32_t)nh};
+                dh = O->hits.as<mirfold_hit>(); da = O->arena.as<char>();
+            }
+            for (uint64_t k = 0; k < nh; k++) { dh[k] = hits[k]; dh[k].ss_off += abase; }
+            if (ab) memcpy(da, arena.data(), ab);
+            S.totals[r] = total;
+            if (O) { std::lock_guard<std::mutex> lk(S.mu); S.overflow.push_back(std::move(O)); }
+            else { S.hit_begin[r] = hb; S.hit_count[r] = (uint32_t)nh; }
+        } else if (J.sink == SINK_STREAM) {
+            uint64_t begin = 0;
+            uint32_t count = (uint32_t)nh;
+            mirfold_chunk c{};
+            c.n_records = 1; c.device = D.id;
+            c.record = &r; c.hit_begin = &begin; c.hit_count = &count; c.total_mfe_dcal = &total;
+            c.nhits = nh; c.hits = hits.data(); c.ss_arena = arena.data(); c.ss_bytes = ab;
+            std::lock_guard<std::mutex> lk(*J.cb_mu);
+            if (!J.cb_abort->load() && J.fn(J.user, &c) != 0) J.cb_abort->store(1);
+        } else if (J.sink == SINK_CAND) {   // stages 1 + 3 on the record's hits, uploaded again as a chunk of one locus
+            cudaStream_t hi = Ln.s_hi;
+            const unsigned long long bounds[2] = {0, nh};
+            CK(Ln.o_hits.ensure(nh * sizeof(mirfold_hit) + 16));
+            CK(Ln.o_arena.ensure(ab + 16));
+            CK(Ln.bounds.ensure(16));
+            CK(Ln.totals.ensure(8));
+            if (nh) CK(cudaMemcpyAsync(Ln.o_hits.p, hits.data(), nh * sizeof(mirfold_hit), cudaMemcpyHostToDevice, hi));
+            if (ab) CK(cudaMemcpyAsync(Ln.o_arena.p, arena.data(), ab, cudaMemcpyHostToDevice, hi));
+            CK(cudaMemcpyAsync(Ln.bounds.p, bounds, 16, cudaMemcpyHostToDevice, hi));
+            CK(cudaMemcpyAsync(Ln.totals.p, &total, 4, cudaMemcpyHostToDevice, hi));
+            out.st.h2d_bytes += nh * sizeof(mirfold_hit) + ab + 20;
+            Ln.tb = TraceBuffers{};
+            Ln.tb.loci = Ln.loci.as<LocusDesc>(); Ln.tb.nloci = 1;
+            Ln.nhits = nh; Ln.abytes = ab; Ln.arena_base = 0;
+            if (!back_candidates(Ln, last_chunk, true)) return false;
+            CK(cudaEventRecord(Ln.ev[6], hi));
+            CK(cudaEventSynchronize(Ln.ev[6]));
+            retire_candidates(Ln);
+        }
         return true;
     }
 
@@ -1922,6 +2252,22 @@ int mirfold_plan_fill_units(uint32_t n, int span_L, mirfold_fill_plan *out)
     out->n_units = d.dmax >= 4 ? d.tile_last + 1 : 0;   // n < 5: nothing to fill
     out->dmax = d.dmax;
     out->band_cells = be;
+    return MIRFOLD_OK;
+}
+
+int mirfold_plan_segments(uint32_t n, int span_L, uint64_t budget_bytes, mirfold_segment *segs, uint32_t cap, uint32_t *n_segments)
+{
+    if (!n_segments || n < 1 || n > 0x3fffffffu || span_L < 5 || span_L > MF_MAX_SPAN || (!segs && cap)) return MIRFOLD_ERR_ARG;
+    LocusDesc d{};
+    shape_locus(d, (int)n, span_L);
+    if (!band_offsets_fit(d)) return MIRFOLD_ERR_ARG;
+    std::vector<SegPlan> plan;
+    plan_segments((int)n, span_L, (size_t)budget_bytes, plan);
+    *n_segments = (uint32_t)plan.size();
+    for (uint32_t k = 0; k < cap && k < plan.size(); k++) {
+        const SegPlan &g = plan[k];
+        segs[k] = mirfold_segment{g.t0, g.t1, g.halo, g.row_lo, g.row_hi, 0, (uint64_t)g.bytes};
+    }
     return MIRFOLD_OK;
 }
 

@@ -201,6 +201,12 @@ struct TraceBuffers {
     int *fail_flag;                // 1 int
 };
 cudaError_t launch_plan(const TraceBuffers &b, cudaStream_t st);
+// segmented loci (host.cu, fold_segmented): f3 of a row range, the resumable plan, emission across segment edges
+cudaError_t launch_f3_rows(const LocusDesc *locus, int Ls, int row_hi, int row_lo, const unsigned char *codes, const int *C, int *F,
+                           const DevParams *P, cudaStream_t st);
+cudaError_t launch_plan_seg(const int *F, int row_hi, int row_lo, int bottom, int *state, int *list, unsigned long long *tb_base,
+                            int *tb_count, cudaStream_t st);
+cudaError_t launch_emit_seg(const TraceBuffers &b, int n_carry, int shift, int last, const int *F, int n, int *abs_start, cudaStream_t st);
 cudaError_t launch_traceback(const TraceBuffers &b, cudaStream_t st);
 cudaError_t launch_emit(const TraceBuffers &b, cudaStream_t st);
 struct mirfold_hit;

@@ -47,6 +47,37 @@ cudaError_t launch_plan(const TraceBuffers &b, cudaStream_t st)
     return cudaGetLastError();
 }
 
+// k_plan over rows row_hi .. row_lo of one segment of a segmented locus (host.cu, fold_segmented), resumed from the state
+// the segment above left in state[0..2] (fnext, do_bt, have_prev; all 0 at the top: f3(n-3) == 0) and left there for the
+// segment below.  The row loop produces the starts i + 1 of rows row_lo .. row_hi, so every start lies in the segment's
+// owned rows or the first row above them, whose traceback the segment's halo holds.  F and the starts are relative to the
+// segment's suffix descriptor; `bottom`: the segment holds row 1 of the locus (the final backtrack(1, L*)).
+__global__ void k_plan_seg(const int *__restrict__ F, int row_hi, int row_lo, int bottom, int *state, int *list,
+                           unsigned long long *tb_base, int *tb_count)
+{
+    int cnt = 0, fnext = state[0], do_bt = state[1], have_prev = state[2];
+    for (int i = row_hi; i >= row_lo; i--) {
+        const int fi = F[i];
+        if (fi != fnext) do_bt = 1;
+        else if (do_bt) { list[cnt++] = i + 1; have_prev = 1; do_bt = 0; }
+        if (bottom && i == 1) {
+            if (!have_prev) do_bt = 1;
+            if (do_bt) list[cnt++] = 1;
+        }
+        fnext = fi;
+    }
+    state[0] = fnext; state[1] = do_bt; state[2] = have_prev;
+    tb_base[0] = 0; tb_base[1] = (unsigned long long)cnt;
+    tb_count[0] = cnt;
+}
+
+cudaError_t launch_plan_seg(const int *F, int row_hi, int row_lo, int bottom, int *state, int *list, unsigned long long *tb_base,
+                            int *tb_count, cudaStream_t st)
+{
+    k_plan_seg<<<1, 1, 0, st>>>(F, row_hi, row_lo, bottom, state, list, tb_base, tb_count);
+    return cudaGetLastError();
+}
+
 // ------------------------------------------------------------------------------------ traceback
 // band offset of cell (i, i+d) of a tiled long locus (LocusDesc::tile_*, see band_row_base)
 __device__ __noinline__ unsigned long long tb_tiled_off(int i, int d, unsigned int tile_rcp, int tile_last, int tile_step, int n, int dmax)
@@ -510,6 +541,58 @@ cudaError_t launch_emit(const TraceBuffers &b, cudaStream_t st)
     if (b.ntb == 0) return cudaSuccess;
     const unsigned long long blocks = (b.ntb + 3) / 4;
     k_emit<<<(unsigned)blocks, 128, 0, st>>>(b);
+    return cudaGetLastError();
+}
+
+// k_emit over one segment of a segmented locus.  Its tracebacks are, in print order, the one carried over from the segment
+// above (n_carry = 1: entry 0, start already absolute, traced there) and the segment's own (starts relative to the
+// segment's suffix, which begins after base `shift`).  Every entry is decided against the next one; the last entry of a
+// segment that is not the last waits for the first traceback of the segment below (the host carries it over and it is
+// not printed here).  In the last segment the final entries are printed as k_emit prints them.  Writes the absolute start
+// of every entry to abs_start (k_pack's tb_start); F is the whole locus' f3, n its length.
+__global__ void __launch_bounds__(128) k_emit_seg(TraceBuffers b, int n_carry, int shift, int last, const int *__restrict__ F, int n,
+                                                  int *__restrict__ abs_start)
+{
+    const unsigned long long g = ((unsigned long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (g >= b.ntb) return;
+    const unsigned long long ntb = b.ntb;
+    auto start_of = [&](unsigned long long k) { return b.tb_start[k] + (k < (unsigned long long)n_carry ? 0 : shift); };
+    const int start = start_of(g), len = b.tb_len[g];
+    bool printed;
+    const int last_regular = (int)ntb - ((start_of(ntb - 1) == 1) ? 2 : 1);
+    if (last && (long long)g >= last_regular) printed = true;   // last "prev" at i==1, and the final backtrack(1,L*)
+    else if (g + 1 == ntb) printed = false;                       // carried: decided in the segment below
+    else {
+        const unsigned long long gn = g + 1;
+        const int i = start_of(gn) - 1, ls = b.tb_len[gn];
+        const char *ss = b.slots + gn * (unsigned long long)b.slot_stride;
+        const char *prev = b.slots + g * (unsigned long long)b.slot_stride;
+        if (i + ls < start + len) printed = true;
+        else {
+            const int off = start - i;
+            bool diff = false;
+            for (int kb = 0; kb < len && !diff; kb += 32) {
+                const int k = kb + lane;
+                const bool dneq = (k < len) && (ss[off + k] != prev[k]);
+                diff = __any_sync(FULL, dneq);
+            }
+            printed = diff;
+        }
+    }
+    if (lane == 0) {
+        b.tb_flag[g] = printed ? 1 : 0;
+        const int e2 = (start + len <= n + 2) ? F[start + len] : 0;
+        b.tb_energy[g] = F[start] - e2;
+        abs_start[g] = start;
+    }
+}
+
+cudaError_t launch_emit_seg(const TraceBuffers &b, int n_carry, int shift, int last, const int *F, int n, int *abs_start, cudaStream_t st)
+{
+    if (b.ntb == 0) return cudaSuccess;
+    const unsigned long long blocks = (b.ntb + 3) / 4;
+    k_emit_seg<<<(unsigned)blocks, 128, 0, st>>>(b, n_carry, shift, last, F, n, abs_start);
     return cudaGetLastError();
 }
 

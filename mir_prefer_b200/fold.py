@@ -479,6 +479,27 @@ def plan_fill_units(n, span):
     return {k: int(getattr(fp, k)) for k, _ in _lib.FillPlan._fields_}
 
 
+SEGMENT_DTYPE = np.dtype([("tile_first", np.int32), ("tile_last", np.int32), ("halo_tiles", np.int32), ("row_first", np.int32),
+                          ("row_last", np.int32), ("reserved", np.int32), ("device_bytes", np.uint64)])
+
+
+def plan_segments(n, span, budget_bytes):
+    """How the fold runs a locus of n bases at this span with budget_bytes of device memory (mirfold_plan_segments;
+    host-only): a structured array (SEGMENT_DTYPE) of segments in the order they run, 3' end first -- owned tiles
+    tile_first..tile_last, halo_tiles more above them, owned rows row_first..row_last and device_bytes.  One segment when
+    the locus fits the budget or is one fill unit."""
+    lib = _lib.load()
+    cnt = C.c_uint32(0)
+    rc = lib.mirfold_plan_segments(int(n), int(span), int(budget_bytes), None, 0, C.byref(cnt))
+    if rc != 0:
+        raise MirfoldError(rc, lib.mirfold_strerror(rc).decode())
+    out = np.zeros(cnt.value, SEGMENT_DTYPE)
+    rc = lib.mirfold_plan_segments(int(n), int(span), int(budget_bytes), out.ctypes.data, cnt.value, C.byref(cnt))
+    if rc != 0:
+        raise MirfoldError(rc, lib.mirfold_strerror(rc).decode())
+    return out
+
+
 class MirFold:
     """A libmirfold context (one per process; `devices` = CUDA ordinals, default current device)."""
 

@@ -91,6 +91,12 @@ struct OverflowChunk {   // a chunk that did not fit the shared result buffers (
     std::vector<uint64_t> begin;
 };
 
+// Lane::ev: the events a chunk (or a segment) records, in stream order; side fork / join are launch_fill's
+enum { EV_H2D, EV_KERNELS, EV_FILL, EV_FILL_END, EV_F3_END, EV_PACK_END, EV_D2H_END, EV_SIDE_FORK, EV_SIDE_JOIN, EV_COUNT };
+// Lane::h_small: what a lane downloads before a host sync -- tracebacks (plan), printed bytes and hits (emission), the fail
+// flag (an int) and, for SINK_CAND, the candidate structures, their verdicts and string bytes
+enum { HS_NTB, HS_ABYTES, HS_NHITS, HS_FAIL, HS_NSTRUCTS, HS_NVERDICTS, HS_SBYTES };
+
 // A lane = one complete set of pipeline buffers and streams; a device alternates chunks between two lanes.
 struct Lane {
     cudaStream_t s_lo = nullptr;   // uploads, encode, band fill
@@ -103,8 +109,9 @@ struct Lane {
     DBuf c_counts, c_soff, c_structs, c_nq, c_sbytes, c_voff, c_aoff, c_lsb, c_verd, c_vmat, c_arena, c_sout;   // fused stage 1 + 3
     HBuf hc_structs, hc_arena, hc_verd, hc_vmat, hc_voff, hc_lsb;
     uint64_t c_ns = 0, c_nv = 0, c_nb = 0;
-    HBuf h_raw, h_loci, h_units, h_listoff, h_small, h_out, h_hits, h_arena;
-    cudaEvent_t ev[12] = {};   // 0 h2d begin, 1 kernels begin, 2 fill begin, 3 fill end, 4 f3 end, 5 pack end, 6 d2h end, 7 done, 10/11 side fork/join
+    HBuf h_raw, h_loci, h_units, h_listoff, h_small, h_hits, h_arena;
+    HBuf h_out;   // the chunk's per-locus tables: nl + 1 first-hit bounds (u64), then nl totals (int)
+    cudaEvent_t ev[EV_COUNT] = {};
     // chunk in flight
     bool pending = false;
     Prep prep;
@@ -388,6 +395,16 @@ cudaError_t exclusive_scan(Lane &Ln, const unsigned long long *in, unsigned long
     e = Ln.scan_tmp.ensure(tmp);
     if (e != cudaSuccess) return e;
     return cub::DeviceScan::ExclusiveSum(Ln.scan_tmp.p, tmp, in, out, n, st);
+}
+
+// the band fill of the nu units in Ln.units (sorted into buckets as bucket_first says) on the lane's buffers, at span L
+FillLaunch fill_launch(const Lane &Ln, const DevParams *dP, int nu, int max_n, const int bucket_first[6], bool force_wide, int L)
+{
+    FillLaunch fa{Ln.units.as<LocusDesc>(), nu, max_n, Ln.codes.as<unsigned char>(), Ln.C.as<int>(), Ln.M.as<int>(), Ln.ring.as<int>(),
+                  Ln.Ib.as<unsigned char>(), Ln.Mp.as<unsigned int>(), dP, {0, 0, 0, 0, 0, 0}, Ln.fillflags.as<int>(), force_wide ? 1 : 0,
+                  env_opts() | (L >= MF_DYNW_MIN_SPAN ? 8 : 0)};
+    for (int b = 0; b < 6; b++) fa.bucket_first[b] = bucket_first[b];
+    return fa;
 }
 
 // Band shape of one locus: stride bucket or, for a longer locus with a span that leaves at least
@@ -727,7 +744,7 @@ struct DevicePipeline {
         CK(Ln.h_small.ensure(256));
         // ---- upload
         cudaStream_t lo = Ln.s_lo, hi = Ln.s_hi;
-        CK(cudaEventRecord(Ln.ev[0], lo));
+        CK(cudaEventRecord(Ln.ev[EV_H2D], lo));
         const char *raw_dev = d_raw;
         if (!d_raw) {
             CK(Ln.h_raw.ensure(P.raw_acc));
@@ -744,39 +761,32 @@ struct DevicePipeline {
         out.st.h2d_bytes += (sizeof(LocusDesc) + 8) * (uint64_t)nl + sizeof(LocusDesc) * (uint64_t)nu;
         CK(cudaMemsetAsync(Ln.fail.p, 0, 4, lo));
         CK(cudaMemsetAsync(Ln.fillflags.p, 0, (size_t)nu * 4 + 4, lo));
-        CK(cudaEventRecord(Ln.ev[1], lo));
+        CK(cudaEventRecord(Ln.ev[EV_KERNELS], lo));
         // The two lanes' fills normally share the SMs and finish together, which is what hides wave tails -- but it also means the
         // small last chunk (plan_chunks cuts it 80 : 20) would be done before the previous chunk's download even starts.  Its fill
         // therefore waits for the previous chunk's fill to END: it then runs next to that chunk's traceback and under its download.
         if (J.sink != SINK_NONE && J.sink != SINK_TOTALS && nlanes_ == 2 && ci > 0 && ci + 1 == chunks.size())
-            CK(cudaStreamWaitEvent(lo, D.lane[(ci + 1) % 2].ev[3], 0));
+            CK(cudaStreamWaitEvent(lo, D.lane[(ci + 1) % 2].ev[EV_FILL_END], 0));
         // ---- K1, K2 on the low-priority stream
         const LocusDesc *dl = Ln.loci.as<LocusDesc>();
         CK(launch_prepare(raw_dev, dl, nl, P.seq_acc, Ln.codes.as<unsigned char>(), Ln.F.as<int>(), lo));
-        CK(cudaEventRecord(Ln.ev[2], lo));
-        FillLaunch fa{Ln.units.as<LocusDesc>(), nu, P.max_n, Ln.codes.as<unsigned char>(), Ln.C.as<int>(), Ln.M.as<int>(), Ln.ring.as<int>(),
-                      Ln.Ib.as<unsigned char>(), Ln.Mp.as<unsigned int>(), D.dP, {0, 0, 0, 0, 0, 0}, Ln.fillflags.as<int>(), J.force_wide ? 1 : 0, env_opts() | (J.L >= MF_DYNW_MIN_SPAN ? 8 : 0)};
-        for (int b = 0; b < 6; b++) fa.bucket_first[b] = P.bucket_first[b];
+        CK(cudaEventRecord(Ln.ev[EV_FILL], lo));
         static const bool no_side = getenv("MIRFOLD_NO_SIDE_STREAM") != nullptr;   // A/B runs
-        CK(launch_fill(fa, lo, no_side ? nullptr : Ln.side, Ln.ev[10], Ln.ev[11]));
-        CK(cudaEventRecord(Ln.ev[3], lo));
+        CK(launch_fill(fill_launch(Ln, D.dP, nu, P.max_n, P.bucket_first, J.force_wide, J.L), lo, no_side ? nullptr : Ln.side,
+                       Ln.ev[EV_SIDE_FORK], Ln.ev[EV_SIDE_JOIN]));
+        CK(cudaEventRecord(Ln.ev[EV_FILL_END], lo));
         // ---- K3 + emission plan on the high-priority stream
-        CK(cudaStreamWaitEvent(hi, Ln.ev[3], 0));
+        CK(cudaStreamWaitEvent(hi, Ln.ev[EV_FILL_END], 0));
         CK(launch_f3(dl, nl, P.n_long, P.max_Ls, Ln.codes.as<unsigned char>(), Ln.C.as<int>(), Ln.F.as<int>(), D.dP, hi));
         {   // kernels launched so far: k_prepare, the fill kernels (16-bit + 32-bit redo per non-empty bucket, generic), k_f3 / k_f3_cta
             int nfill = P.bucket_first[1] > P.bucket_first[0] ? 1 : 0;
             for (int b = 1; b < 5; b++) if (P.bucket_first[b + 1] > P.bucket_first[b]) nfill += J.force_wide ? 1 : 2;
             out.st.kernel_launches += 1 + nfill + (P.n_long > 0 ? 1 : 0) + (P.n_long < nl ? 1 : 0);
         }
-        CK(cudaEventRecord(Ln.ev[4], hi));
+        CK(cudaEventRecord(Ln.ev[EV_F3_END], hi));
         if (J.sink == SINK_TOTALS) return front_totals(Ln, ci + 1 == chunks.size());
         TraceBuffers &tb = Ln.tb;
-        tb = TraceBuffers{};
-        tb.loci = dl; tb.nloci = nl; tb.codes = Ln.codes.as<unsigned char>();
-        tb.C = Ln.C.as<int>(); tb.M = Ln.M.as<int>(); tb.F = Ln.F.as<int>(); tb.Ib = Ln.Ib.as<unsigned char>(); tb.P = D.dP;
-        tb.tb_count = Ln.tbcount.as<int>(); tb.tb_base = Ln.tbbase.as<unsigned long long>();
-        tb.list_off = Ln.listoff.as<unsigned long long>(); tb.tb_start_list = Ln.startlist.as<int>();
-        tb.fail_flag = Ln.fail.as<int>();
+        tb = trace_buffers(Ln, dl, nl);
         CK(launch_plan(tb, hi));
         k_widen_counts<<<(nl + 1 + 255) / 256, 256, 0, hi>>>(tb.tb_count, Ln.scan_in.as<unsigned long long>(), nl);
         CK(cudaGetLastError());
@@ -794,14 +804,14 @@ struct DevicePipeline {
         cudaStream_t hi = Ln.s_hi;
         const int nl = Ln.prep.nl;
         CK(Ln.totals.ensure((size_t)nl * 4 + 4));
-        CK(Ln.h_out.ensure((size_t)nl * 4 + 64));
+        CK(Ln.h_out.ensure((size_t)(nl + 1) * 8 + (size_t)nl * 4 + 64));
         k_gather_totals<<<(nl + 255) / 256, 256, 0, hi>>>(Ln.loci.as<LocusDesc>(), Ln.F.as<int>(), Ln.totals.as<int>(), nl);
         CK(cudaGetLastError());
-        CK(cudaEventRecord(Ln.ev[5], hi));
+        CK(cudaEventRecord(Ln.ev[EV_PACK_END], hi));
         if (last_chunk) CK(cudaEventRecord(D.ev_last, hi));
-        CK(cudaMemcpyAsync(Ln.h_out.p, Ln.totals.p, (size_t)nl * 4, cudaMemcpyDeviceToHost, hi));
-        CK(cudaEventRecord(Ln.ev[6], hi));
-        CK(cudaStreamWaitEvent(Ln.s_lo, Ln.ev[6], 0));   // the lane's next upload waits for this chunk to leave the device
+        CK(cudaMemcpyAsync(Ln.h_out.as<unsigned long long>() + nl + 1, Ln.totals.p, (size_t)nl * 4, cudaMemcpyDeviceToHost, hi));
+        CK(cudaEventRecord(Ln.ev[EV_D2H_END], hi));
+        CK(cudaStreamWaitEvent(Ln.s_lo, Ln.ev[EV_D2H_END], 0));   // the lane's next upload waits for this chunk to leave the device
         out.st.kernel_launches += 1;
         out.st.d2h_bytes += (uint64_t)nl * 4;
         Ln.pending = true;
@@ -815,60 +825,83 @@ struct DevicePipeline {
         if (J.sink == SINK_TOTALS) return true;
         cudaStream_t hi = Ln.s_hi;
         TraceBuffers &tb = Ln.tb;
-        const Prep &P = Ln.prep;
-        const int nl = P.nl;
-        unsigned long long *hs = Ln.h_small.as<unsigned long long>();
         CK(cudaStreamSynchronize(hi));
-        const unsigned long long ntb = hs[0];
+        const unsigned long long ntb = Ln.h_small.as<unsigned long long>()[HS_NTB];
         out.st.tracebacks += ntb;
         ht.mark("plan sync");
+        if (!trace_scratch(Ln, tb, ntb, Ln.prep.max_Ls)) return false;
+        CK(launch_traceback(tb, hi));
+        CK(launch_emit(tb, hi));
+        if (ntb) out.st.kernel_launches += 2;
+        if (!emission_sizes(Ln, tb, hi)) return false;
+        ht.mark("traceback sync");
+        return true;
+    }
+
+    // the plan's buffers of the lane for nl descriptors at dl; per-traceback scratch comes from trace_scratch
+    TraceBuffers trace_buffers(Lane &Ln, const LocusDesc *dl, int nl) const
+    {
+        TraceBuffers tb{};
+        tb.loci = dl; tb.nloci = nl; tb.codes = Ln.codes.as<unsigned char>();
+        tb.C = Ln.C.as<int>(); tb.M = Ln.M.as<int>(); tb.F = Ln.F.as<int>(); tb.Ib = Ln.Ib.as<unsigned char>(); tb.P = D.dP;
+        tb.tb_count = Ln.tbcount.as<int>(); tb.tb_base = Ln.tbbase.as<unsigned long long>();
+        tb.list_off = Ln.listoff.as<unsigned long long>(); tb.tb_start_list = Ln.startlist.as<int>();
+        tb.fail_flag = Ln.fail.as<int>();
+        return tb;
+    }
+
+    // scratch of ntb tracebacks of at most max_Ls nt: slots, per-traceback ints, stacks and the emission scans
+    bool trace_scratch(Lane &Ln, TraceBuffers &tb, unsigned long long ntb, int max_Ls)
+    {
         tb.ntb = ntb;
-        tb.slot_stride = (P.max_Ls + 4 + 3) & ~3;
-        tb.stack_cap = P.max_Ls / 4 + 16;
-        tb.code_win = (P.max_Ls + 8 + 15) & ~15;
+        tb.slot_stride = (max_Ls + 4 + 3) & ~3;
+        tb.stack_cap = max_Ls / 4 + 16;
+        tb.code_win = (max_Ls + 8 + 15) & ~15;
         CK(Ln.slots.ensure((size_t)ntb * tb.slot_stride + 16));
         CK(Ln.tblen.ensure((size_t)ntb * 4 + 16)); CK(Ln.tbstart.ensure((size_t)ntb * 4 + 16));
         CK(Ln.tblocus.ensure((size_t)ntb * 4 + 16)); CK(Ln.tbflag.ensure((size_t)ntb * 4 + 16));
         CK(Ln.tbenergy.ensure((size_t)ntb * 4 + 16));
         CK(Ln.stackscr.ensure((size_t)ntb * tb.stack_cap * 8 + 16));
         CK(Ln.ssoff.ensure((size_t)(ntb + 1) * 8)); CK(Ln.hitidx.ensure((size_t)(ntb + 1) * 8));
-        CK(Ln.scan_in.ensure((size_t)(ntb + 1) * 8 + (size_t)(nl + 1) * 8));
+        CK(Ln.scan_in.ensure((size_t)(ntb + 1) * 8 + (size_t)(tb.nloci + 1) * 8));
         CK(Ln.scan_out.ensure((size_t)(ntb + 1) * 8));
         tb.slots = Ln.slots.as<char>(); tb.tb_len = Ln.tblen.as<int>(); tb.tb_start = Ln.tbstart.as<int>();
         tb.tb_locus = Ln.tblocus.as<int>(); tb.tb_flag = Ln.tbflag.as<int>(); tb.tb_energy = Ln.tbenergy.as<int>();
         tb.stack_scratch = Ln.stackscr.as<int>();
-        CK(launch_traceback(tb, hi));
-        CK(launch_emit(tb, hi));
-        if (ntb) {
-            k_emit_sizes<<<(unsigned)((ntb + 1 + 255) / 256), 256, 0, hi>>>(tb.tb_flag, tb.tb_len, Ln.scan_in.as<unsigned long long>(),
-                                                                             Ln.scan_out.as<unsigned long long>(), ntb);
-            CK(cudaGetLastError());
-            CK(exclusive_scan(Ln, Ln.scan_in.as<unsigned long long>(), Ln.ssoff.as<unsigned long long>(), (size_t)ntb + 1, hi));
-            CK(exclusive_scan(Ln, Ln.scan_out.as<unsigned long long>(), Ln.hitidx.as<unsigned long long>(), (size_t)ntb + 1, hi));
-            CK(cudaMemcpyAsync(&hs[1], Ln.ssoff.as<unsigned long long>() + ntb, 8, cudaMemcpyDeviceToHost, hi));
-            CK(cudaMemcpyAsync(&hs[2], Ln.hitidx.as<unsigned long long>() + ntb, 8, cudaMemcpyDeviceToHost, hi));
-            out.st.kernel_launches += 7;
-        }
-        CK(cudaMemcpyAsync(&hs[3], Ln.fail.p, 4, cudaMemcpyDeviceToHost, hi));
-        CK(cudaStreamSynchronize(hi));
-        if (*(int *)&hs[3]) { out.err = MIRFOLD_ERR_BACKTRACK; out.errmsg = "traceback found no decomposition"; return false; }
-        Ln.abytes = ntb ? hs[1] : 0;
-        Ln.nhits = ntb ? hs[2] : 0;
-        ht.mark("traceback sync");
         return true;
     }
 
-    // ---- back: pack the printed structures and start the download into the sink (asynchronous; see retire)
-    bool back(Lane &Ln, bool last_chunk)
+    // after the emission decisions: the printed bytes (ssoff) and hit indices (hitidx) of the tb.ntb tracebacks, their
+    // totals into Ln.abytes / Ln.nhits, and the fail flag (host sync)
+    bool emission_sizes(Lane &Ln, const TraceBuffers &tb, cudaStream_t st)
     {
-        if (J.sink == SINK_TOTALS) return true;
-        cudaStream_t hi = Ln.s_hi;
-        TraceBuffers &tb = Ln.tb;
-        const Prep &P = Ln.prep;
-        const int nl = P.nl;
+        const unsigned long long ntb = tb.ntb;
+        unsigned long long *hs = Ln.h_small.as<unsigned long long>();
+        if (ntb) {
+            k_emit_sizes<<<(unsigned)((ntb + 1 + 255) / 256), 256, 0, st>>>(tb.tb_flag, tb.tb_len, Ln.scan_in.as<unsigned long long>(),
+                                                                             Ln.scan_out.as<unsigned long long>(), ntb);
+            CK(cudaGetLastError());
+            CK(exclusive_scan(Ln, Ln.scan_in.as<unsigned long long>(), Ln.ssoff.as<unsigned long long>(), (size_t)ntb + 1, st));
+            CK(exclusive_scan(Ln, Ln.scan_out.as<unsigned long long>(), Ln.hitidx.as<unsigned long long>(), (size_t)ntb + 1, st));
+            CK(cudaMemcpyAsync(&hs[HS_ABYTES], Ln.ssoff.as<unsigned long long>() + ntb, 8, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(&hs[HS_NHITS], Ln.hitidx.as<unsigned long long>() + ntb, 8, cudaMemcpyDeviceToHost, st));
+            out.st.kernel_launches += 5;   // k_emit_sizes, two cub scans (init + scan each)
+        }
+        CK(cudaMemcpyAsync(&hs[HS_FAIL], Ln.fail.p, 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (*(int *)&hs[HS_FAIL]) { out.err = MIRFOLD_ERR_BACKTRACK; out.errmsg = "traceback found no decomposition"; return false; }
+        Ln.abytes = ntb ? hs[HS_ABYTES] : 0;
+        Ln.nhits = ntb ? hs[HS_NHITS] : 0;
+        return true;
+    }
+
+    // where the lane's Ln.nhits hits and Ln.abytes string bytes go on the host: a reservation in the shared result buffers,
+    // else an overflow chunk of their own (Ln.ovf); the stream sink's buffers; nowhere for the other sinks
+    bool pick_destination(Lane &Ln, mirfold_hit *&dst_hits, char *&dst_arena)
+    {
         const uint64_t nhits = Ln.nhits, abytes = Ln.abytes;
-        mirfold_hit *dst_hits = nullptr;
-        char *dst_arena = nullptr;
+        dst_hits = nullptr;
+        dst_arena = nullptr;
         Ln.hit_base = Ln.arena_base = 0;
         if (J.sink == SINK_SHARED) {
             if (J.shared->reserve(nhits, abytes, Ln.hit_base, Ln.arena_base)) {
@@ -888,6 +921,40 @@ struct DevicePipeline {
             dst_hits = Ln.h_hits.as<mirfold_hit>();
             dst_arena = Ln.h_arena.as<char>();
         }
+        return true;
+    }
+
+    // Ln.bounds / Ln.totals of the chunk: every locus' first hit and total, or all zero when the chunk has no traceback
+    // (hitidx was never scanned)
+    bool gather_bounds(Lane &Ln)
+    {
+        cudaStream_t hi = Ln.s_hi;
+        const TraceBuffers &tb = Ln.tb;
+        const int nl = Ln.prep.nl;
+        if (tb.ntb) {
+            k_gather_bounds<<<(nl + 1 + 255) / 256, 256, 0, hi>>>(tb.tb_base, Ln.hitidx.as<unsigned long long>(), tb.loci, tb.F,
+                                                                  Ln.bounds.as<unsigned long long>(), Ln.totals.as<int>(), nl);
+            CK(cudaGetLastError());
+            out.st.kernel_launches += 1;
+        } else {
+            CK(cudaMemsetAsync(Ln.bounds.p, 0, (size_t)(nl + 1) * 8, hi));
+            CK(cudaMemsetAsync(Ln.totals.p, 0, (size_t)nl * 4, hi));
+        }
+        return true;
+    }
+
+    // ---- back: pack the printed structures and start the download into the sink (asynchronous; see retire)
+    bool back(Lane &Ln, bool last_chunk)
+    {
+        if (J.sink == SINK_TOTALS) return true;
+        cudaStream_t hi = Ln.s_hi;
+        TraceBuffers &tb = Ln.tb;
+        const Prep &P = Ln.prep;
+        const int nl = P.nl;
+        const uint64_t nhits = Ln.nhits, abytes = Ln.abytes;
+        mirfold_hit *dst_hits;
+        char *dst_arena;
+        if (!pick_destination(Ln, dst_hits, dst_arena)) return false;
         CK(Ln.o_hits.ensure(nhits * sizeof(mirfold_hit) + 16));
         CK(Ln.o_arena.ensure(abytes + 16));
         CK(Ln.bounds.ensure((size_t)(nl + 1) * 8));
@@ -895,34 +962,25 @@ struct DevicePipeline {
         CK(launch_pack(tb, Ln.ssoff.as<unsigned long long>(), Ln.hitidx.as<unsigned long long>(), Ln.o_arena.as<char>(),
                        Ln.o_hits.as<mirfold_hit>(), Ln.arena_base, hi));
         out.st.kernel_launches += 1;
-        if (J.sink == SINK_CAND) { if (!back_candidates(Ln, last_chunk)) return false; }
-        else {
-        CK(cudaEventRecord(Ln.ev[5], hi));
-        if (last_chunk) CK(cudaEventRecord(D.ev_last, hi));
-        }
         if (J.sink == SINK_CAND) {
-        } else if (J.sink != SINK_NONE) {
-            if (tb.ntb) {
-                k_gather_bounds<<<(nl + 1 + 255) / 256, 256, 0, hi>>>(tb.tb_base, Ln.hitidx.as<unsigned long long>(), tb.loci, tb.F,
-                                                                      Ln.bounds.as<unsigned long long>(), Ln.totals.as<int>(), nl);
-                CK(cudaGetLastError());
-                out.st.kernel_launches += 1;
-            } else {
-                CK(cudaMemsetAsync(Ln.bounds.p, 0, (size_t)(nl + 1) * 8, hi));
-                CK(cudaMemsetAsync(Ln.totals.p, 0, (size_t)nl * 4, hi));
-            }
-            CK(Ln.h_out.ensure((size_t)(nl + 1) * 8 + (size_t)nl * 4 + 64));
-            unsigned long long *h_bounds = Ln.h_out.as<unsigned long long>();
-            int *h_total = (int *)(h_bounds + nl + 1);
-            if (nhits) CK(cudaMemcpyAsync(dst_hits, Ln.o_hits.p, nhits * sizeof(mirfold_hit), cudaMemcpyDeviceToHost, hi));
-            if (abytes) CK(cudaMemcpyAsync(dst_arena, Ln.o_arena.p, abytes, cudaMemcpyDeviceToHost, hi));
-            CK(cudaMemcpyAsync(h_bounds, Ln.bounds.p, (size_t)(nl + 1) * 8, cudaMemcpyDeviceToHost, hi));
-            CK(cudaMemcpyAsync(h_total, Ln.totals.p, (size_t)nl * 4, cudaMemcpyDeviceToHost, hi));
-            out.st.d2h_bytes += nhits * sizeof(mirfold_hit) + (uint64_t)(nl + 1) * 8 + (uint64_t)nl * 4 + abytes + 32;
-        } else out.st.d2h_bytes += 32;
-        CK(cudaEventRecord(Ln.ev[6], hi));
+            if (!back_candidates(Ln, last_chunk)) return false;
+        } else {
+            CK(cudaEventRecord(Ln.ev[EV_PACK_END], hi));
+            if (last_chunk) CK(cudaEventRecord(D.ev_last, hi));
+            if (J.sink != SINK_NONE) {
+                if (!gather_bounds(Ln)) return false;
+                CK(Ln.h_out.ensure((size_t)(nl + 1) * 8 + (size_t)nl * 4 + 64));
+                unsigned long long *h_bounds = Ln.h_out.as<unsigned long long>();
+                if (nhits) CK(cudaMemcpyAsync(dst_hits, Ln.o_hits.p, nhits * sizeof(mirfold_hit), cudaMemcpyDeviceToHost, hi));
+                if (abytes) CK(cudaMemcpyAsync(dst_arena, Ln.o_arena.p, abytes, cudaMemcpyDeviceToHost, hi));
+                CK(cudaMemcpyAsync(h_bounds, Ln.bounds.p, (size_t)(nl + 1) * 8, cudaMemcpyDeviceToHost, hi));
+                CK(cudaMemcpyAsync(h_bounds + nl + 1, Ln.totals.p, (size_t)nl * 4, cudaMemcpyDeviceToHost, hi));
+                out.st.d2h_bytes += nhits * sizeof(mirfold_hit) + (uint64_t)(nl + 1) * 8 + (uint64_t)nl * 4 + abytes + 32;
+            } else out.st.d2h_bytes += 32;
+        }
+        CK(cudaEventRecord(Ln.ev[EV_D2H_END], hi));
         // the lane's next chunk (uploads on s_lo) may only start once this one has left the device
-        CK(cudaStreamWaitEvent(Ln.s_lo, Ln.ev[6], 0));
+        CK(cudaStreamWaitEvent(Ln.s_lo, Ln.ev[EV_D2H_END], 0));
         out.nhits += nhits;
         out.arena_bytes += abytes;
         ht.mark("back (pack + download enqueue)");
@@ -939,15 +997,7 @@ struct DevicePipeline {
         const uint64_t nhits = Ln.nhits;
         const CandArgs &ca = *J.cand;
         unsigned long long *hs = Ln.h_small.as<unsigned long long>();
-        if (bounds_ready) {   // a segmented locus: its staged hits, bounds and total were uploaded
-        } else if (tb.ntb) {
-            k_gather_bounds<<<(nl + 1 + 255) / 256, 256, 0, hi>>>(tb.tb_base, Ln.hitidx.as<unsigned long long>(), tb.loci, tb.F,
-                                                                  Ln.bounds.as<unsigned long long>(), Ln.totals.as<int>(), nl);
-            CK(cudaGetLastError());
-        } else {   // a hairpin-free chunk: hitidx was never scanned, every locus has no hits (as in back())
-            CK(cudaMemsetAsync(Ln.bounds.p, 0, (size_t)(nl + 1) * 8, hi));
-            CK(cudaMemsetAsync(Ln.totals.p, 0, (size_t)nl * 4, hi));
-        }
+        if (!bounds_ready && !gather_bounds(Ln)) return false;   // bounds_ready: a segmented locus' staged bounds were uploaded
         CK(Ln.c_counts.ensure((nhits + 2) * 8)); CK(Ln.c_soff.ensure((nhits + 2) * 8));
         CK(Ln.c_lsb.ensure((size_t)(nl + 1) * 8));
         CandLaunch c{};
@@ -961,11 +1011,11 @@ struct DevicePipeline {
         c.fail_flag = Ln.fail.as<int>();
         CK(launch_cand_classify(c, 0, hi));
         CK(exclusive_scan(Ln, c.counts, Ln.c_soff.as<unsigned long long>(), (size_t)nhits + 1, hi));
-        CK(cudaMemcpyAsync(&hs[4], Ln.c_soff.as<unsigned long long>() + nhits, 8, cudaMemcpyDeviceToHost, hi));
-        CK(cudaMemcpyAsync(&hs[3], Ln.fail.p, 4, cudaMemcpyDeviceToHost, hi));
+        CK(cudaMemcpyAsync(&hs[HS_NSTRUCTS], Ln.c_soff.as<unsigned long long>() + nhits, 8, cudaMemcpyDeviceToHost, hi));
+        CK(cudaMemcpyAsync(&hs[HS_FAIL], Ln.fail.p, 4, cudaMemcpyDeviceToHost, hi));
         CK(cudaStreamSynchronize(hi));
-        if (*(int *)&hs[3]) { out.err = MIRFOLD_ERR_ARG; out.errmsg = "a hit on which the reference's classifier raises (no pair / unbalanced)"; return false; }
-        const uint64_t ns = Ln.c_ns = hs[4];
+        if (*(int *)&hs[HS_FAIL]) { out.err = MIRFOLD_ERR_ARG; out.errmsg = "a hit on which the reference's classifier raises (no pair / unbalanced)"; return false; }
+        const uint64_t ns = Ln.c_ns = hs[HS_NSTRUCTS];
         CK(Ln.c_structs.ensure(ns * sizeof(mirfold_structure) + 16)); CK(Ln.c_sout.ensure(ns * sizeof(mirfold_structure) + 16));
         CK(Ln.c_nq.ensure((ns + 2) * 8)); CK(Ln.c_sbytes.ensure((ns + 2) * 8));
         CK(Ln.c_voff.ensure((ns + 2) * 8)); CK(Ln.c_aoff.ensure((ns + 2) * 8));
@@ -975,17 +1025,17 @@ struct DevicePipeline {
         CK(launch_cand_classify(c, 1, hi));
         CK(exclusive_scan(Ln, c.nq, Ln.c_voff.as<unsigned long long>(), (size_t)ns + 1, hi));
         CK(exclusive_scan(Ln, c.sbytes, Ln.c_aoff.as<unsigned long long>(), (size_t)ns + 1, hi));
-        CK(cudaMemcpyAsync(&hs[5], Ln.c_voff.as<unsigned long long>() + ns, 8, cudaMemcpyDeviceToHost, hi));
-        CK(cudaMemcpyAsync(&hs[6], Ln.c_aoff.as<unsigned long long>() + ns, 8, cudaMemcpyDeviceToHost, hi));
+        CK(cudaMemcpyAsync(&hs[HS_NVERDICTS], Ln.c_voff.as<unsigned long long>() + ns, 8, cudaMemcpyDeviceToHost, hi));
+        CK(cudaMemcpyAsync(&hs[HS_SBYTES], Ln.c_aoff.as<unsigned long long>() + ns, 8, cudaMemcpyDeviceToHost, hi));
         CK(cudaStreamSynchronize(hi));
-        const uint64_t nv = Ln.c_nv = hs[5], nb = Ln.c_nb = hs[6];
+        const uint64_t nv = Ln.c_nv = hs[HS_NVERDICTS], nb = Ln.c_nb = hs[HS_SBYTES];
         CK(Ln.c_verd.ensure(nv * sizeof(mirfold_duplex_verdict) + 16)); CK(Ln.c_vmat.ensure(nv * 4 + 16)); CK(Ln.c_arena.ensure(nb + 16));
         c.voff = Ln.c_voff.as<unsigned long long>(); c.aoff = Ln.c_aoff.as<unsigned long long>();
         c.verdicts = Ln.c_verd.as<mirfold_duplex_verdict>(); c.verdict_mature = Ln.c_vmat.as<unsigned int>();
         c.out_arena = Ln.c_arena.as<char>(); c.out_base = 0; c.structs_out = Ln.c_sout.as<mirfold_structure>();
         CK(launch_cand_finish(c, P.max_Ls + 4, hi));
-        out.st.kernel_launches += tb.ntb ? 11 : 10;   // gather (if any traceback), 2 x classify, locus bounds, 3 x cub scan (2 kernels each), duplex, strings
-        CK(cudaEventRecord(Ln.ev[5], hi));
+        out.st.kernel_launches += 10;   // 2 x classify, locus bounds, 3 x cub scan (2 kernels each), duplex, strings
+        CK(cudaEventRecord(Ln.ev[EV_PACK_END], hi));
         if (last_chunk) CK(cudaEventRecord(D.ev_last, hi));
         CK(Ln.hc_structs.ensure(ns * sizeof(mirfold_structure) + 16)); CK(Ln.hc_arena.ensure(nb + 16));
         CK(Ln.hc_verd.ensure(nv * sizeof(mirfold_duplex_verdict) + 16)); CK(Ln.hc_vmat.ensure(nv * 4 + 16));
@@ -1038,7 +1088,7 @@ struct DevicePipeline {
         LocusDesc *hl = Ln.h_loci.as<LocusDesc>();
         hl[0] = d;
         const LocusDesc *dl = Ln.loci.as<LocusDesc>();
-        CK(cudaEventRecord(Ln.ev[0], st));
+        CK(cudaEventRecord(Ln.ev[EV_H2D], st));
         const char *raw_dev = d_raw;
         if (!d_raw) {
             CK(Ln.raw.ensure((size_t)n));
@@ -1050,7 +1100,7 @@ struct DevicePipeline {
         CK(cudaMemsetAsync(Ln.segstate.p, 0, 16, st));   // fnext = f3(n-3) = 0, do_bt = have_prev = 0
         CK(cudaMemsetAsync(Ln.fail.p, 0, 4, st));
         CK(cudaMemsetAsync(Ln.listoff.p, 0, 8, st));
-        CK(cudaEventRecord(Ln.ev[1], st));
+        CK(cudaEventRecord(Ln.ev[EV_KERNELS], st));
         CK(launch_prepare(raw_dev, dl, 1, (unsigned long long)n + 3, Ln.codes.as<unsigned char>(), Ln.F.as<int>(), st));
         out.st.kernel_launches += 1;
         std::vector<mirfold_hit> hits;   // the record's hits in print order; ss_off into `arena`
@@ -1058,7 +1108,6 @@ struct DevicePipeline {
         std::vector<char> carry_slot;    // the last traceback of the segment above: slot, length, absolute start
         int carry_len = 0, carry_start = 0;
         bool carry = false;
-        const int slot_stride = (d.Ls + 4 + 3) & ~3, stack_cap = d.Ls / 4 + 16;
         unsigned long long *hs = Ln.h_small.as<unsigned long long>();
         for (size_t sg = 0; sg < segs.size(); sg++) {
             const SegPlan &g = segs[sg];
@@ -1090,23 +1139,21 @@ struct DevicePipeline {
             CK(cudaMemsetAsync(Ln.fillflags.p, 0, (size_t)ntiles * 4 + 4, st));
             out.st.h2d_bytes += sizeof(LocusDesc) * (uint64_t)(ntiles + 1);
             out.st.fill_units += (uint64_t)ntiles;
-            CK(cudaEventRecord(Ln.ev[2], st));
-            FillLaunch fa{Ln.units.as<LocusDesc>(), ntiles, TL, Ln.codes.as<unsigned char>(), Ln.C.as<int>(), Ln.M.as<int>(), Ln.ring.as<int>(),
-                          Ln.Ib.as<unsigned char>(), Ln.Mp.as<unsigned int>(), D.dP, {0, 0, 0, 0, 0, 0}, Ln.fillflags.as<int>(), J.force_wide ? 1 : 0,
-                          env_opts() | (J.L >= MF_DYNW_MIN_SPAN ? 8 : 0)};
+            CK(cudaEventRecord(Ln.ev[EV_FILL], st));
             const int bucket = unit_bucket(hu[0]);
-            for (int b = 0; b < 6; b++) fa.bucket_first[b] = b <= bucket ? 0 : ntiles;
-            CK(launch_fill(fa, st));
-            CK(cudaEventRecord(Ln.ev[3], st));
+            int bucket_first[6];
+            for (int b = 0; b < 6; b++) bucket_first[b] = b <= bucket ? 0 : ntiles;
+            CK(launch_fill(fill_launch(Ln, D.dP, ntiles, TL, bucket_first, J.force_wide, J.L), st));
+            CK(cudaEventRecord(Ln.ev[EV_FILL_END], st));
             const int row_lo = g.row_lo - a, row_hi = std::min(g.row_hi, n - 4) - a;   // owned rows with an f3 / plan step
             CK(launch_f3_rows(dl + 1, d.Ls, row_hi, row_lo, Ln.codes.as<unsigned char>(), Ln.C.as<int>(), Ln.F.as<int>(), D.dP, st));
-            CK(cudaEventRecord(Ln.ev[4], st));
+            CK(cudaEventRecord(Ln.ev[EV_F3_END], st));
             out.st.kernel_launches += (J.force_wide ? 1 : 2) + (row_hi >= row_lo ? 1 : 0);
             if (J.sink == SINK_TOTALS) {
-                CK(cudaEventRecord(Ln.ev[5], st));
-                CK(cudaEventRecord(Ln.ev[6], st));
+                CK(cudaEventRecord(Ln.ev[EV_PACK_END], st));
+                CK(cudaEventRecord(Ln.ev[EV_D2H_END], st));
                 CK(cudaStreamSynchronize(st));
-                segment_times(Ln);
+                add_stage_times(Ln, sg == 0);
                 continue;
             }
             // ---- emission plan over the owned rows, resumed from the segment above
@@ -1114,29 +1161,15 @@ struct DevicePipeline {
             CK(Ln.startlist.ensure(((size_t)(g.row_hi - g.row_lo + 1) / 2 + 4) * 4));
             CK(launch_plan_seg(Fs, row_hi, row_lo, g.row_lo == 1 ? 1 : 0, Ln.segstate.as<int>(), Ln.startlist.as<int>(),
                                Ln.tbbase.as<unsigned long long>(), Ln.tbcount.as<int>(), st));
-            CK(cudaMemcpyAsync(&hs[0], Ln.tbbase.as<unsigned long long>() + 1, 8, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(&hs[HS_NTB], Ln.tbbase.as<unsigned long long>() + 1, 8, cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));
             const int nc = carry ? 1 : 0;
-            const unsigned long long m = hs[0], ntb = m + (unsigned long long)nc;
+            const unsigned long long m = hs[HS_NTB], ntb = m + (unsigned long long)nc;
             out.st.tracebacks += m;
             // ---- tracebacks of the segment's starts behind the carried entry 0
-            CK(Ln.slots.ensure((size_t)ntb * slot_stride + 16));
-            CK(Ln.tblen.ensure((size_t)ntb * 4 + 16)); CK(Ln.tbstart.ensure((size_t)ntb * 4 + 16));
-            CK(Ln.tblocus.ensure((size_t)ntb * 4 + 16)); CK(Ln.tbflag.ensure((size_t)ntb * 4 + 16));
-            CK(Ln.tbenergy.ensure((size_t)ntb * 4 + 16));
-            CK(Ln.stackscr.ensure((size_t)ntb * stack_cap * 8 + 16));
-            CK(Ln.ssoff.ensure((size_t)(ntb + 1) * 8)); CK(Ln.hitidx.ensure((size_t)(ntb + 1) * 8));
-            CK(Ln.scan_in.ensure((size_t)(ntb + 1) * 8)); CK(Ln.scan_out.ensure((size_t)(ntb + 1) * 8));
-            TraceBuffers tb{};
-            tb.loci = dl + 1; tb.nloci = 1; tb.codes = Ln.codes.as<unsigned char>();
-            tb.C = Ln.C.as<int>(); tb.M = Ln.M.as<int>(); tb.F = Ln.F.as<int>(); tb.Ib = Ln.Ib.as<unsigned char>(); tb.P = D.dP;
-            tb.tb_count = Ln.tbcount.as<int>(); tb.tb_base = Ln.tbbase.as<unsigned long long>();
-            tb.list_off = Ln.listoff.as<unsigned long long>(); tb.tb_start_list = Ln.startlist.as<int>();
-            tb.fail_flag = Ln.fail.as<int>();
-            tb.slot_stride = slot_stride; tb.stack_cap = stack_cap; tb.code_win = (d.Ls + 8 + 15) & ~15;
-            tb.slots = Ln.slots.as<char>(); tb.tb_len = Ln.tblen.as<int>(); tb.tb_start = Ln.tbstart.as<int>();
-            tb.tb_locus = Ln.tblocus.as<int>(); tb.tb_flag = Ln.tbflag.as<int>(); tb.tb_energy = Ln.tbenergy.as<int>();
-            tb.stack_scratch = Ln.stackscr.as<int>();
+            TraceBuffers tb = trace_buffers(Ln, dl + 1, 1);
+            if (!trace_scratch(Ln, tb, ntb, d.Ls)) return false;
+            const int slot_stride = tb.slot_stride;
             if (carry) {
                 CK(cudaMemcpyAsync(tb.slots, carry_slot.data(), (size_t)slot_stride, cudaMemcpyHostToDevice, st));
                 CK(cudaMemcpyAsync(tb.tb_len, &carry_len, 4, cudaMemcpyHostToDevice, st));
@@ -1145,26 +1178,12 @@ struct DevicePipeline {
             TraceBuffers tv = tb;   // the segment's own tracebacks: entries nc .. ntb-1
             tv.ntb = m;
             tv.slots += (size_t)nc * slot_stride; tv.tb_len += nc; tv.tb_start += nc; tv.tb_locus += nc; tv.tb_flag += nc; tv.tb_energy += nc;
-            tv.stack_scratch += (size_t)nc * stack_cap * 2;
+            tv.stack_scratch += (size_t)nc * tb.stack_cap * 2;
             CK(launch_traceback(tv, st));
-            tb.ntb = ntb;
             int *abs_start = Ln.tblocus.as<int>();
             CK(launch_emit_seg(tb, nc, a, last ? 1 : 0, Ln.F.as<int>() + d.seq_off, n, abs_start, st));
-            uint64_t nhits = 0, abytes = 0;
-            if (ntb) {
-                k_emit_sizes<<<(unsigned)((ntb + 1 + 255) / 256), 256, 0, st>>>(tb.tb_flag, tb.tb_len, Ln.scan_in.as<unsigned long long>(),
-                                                                              Ln.scan_out.as<unsigned long long>(), ntb);
-                CK(cudaGetLastError());
-                CK(exclusive_scan(Ln, Ln.scan_in.as<unsigned long long>(), Ln.ssoff.as<unsigned long long>(), (size_t)ntb + 1, st));
-                CK(exclusive_scan(Ln, Ln.scan_out.as<unsigned long long>(), Ln.hitidx.as<unsigned long long>(), (size_t)ntb + 1, st));
-                CK(cudaMemcpyAsync(&hs[1], Ln.ssoff.as<unsigned long long>() + ntb, 8, cudaMemcpyDeviceToHost, st));
-                CK(cudaMemcpyAsync(&hs[2], Ln.hitidx.as<unsigned long long>() + ntb, 8, cudaMemcpyDeviceToHost, st));
-                out.st.kernel_launches += 8;
-            }
-            CK(cudaMemcpyAsync(&hs[3], Ln.fail.p, 4, cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-            if (*(int *)&hs[3]) { out.err = MIRFOLD_ERR_BACKTRACK; out.errmsg = "traceback found no decomposition"; return false; }
-            if (ntb) { abytes = hs[1]; nhits = hs[2]; }
+            if (!emission_sizes(Ln, tb, st)) return false;
+            const uint64_t nhits = Ln.nhits, abytes = Ln.abytes;
             // ---- pack and download the printed hits; carry the undecided last traceback to the next segment
             CK(Ln.o_hits.ensure(nhits * sizeof(mirfold_hit) + 16));
             CK(Ln.o_arena.ensure(abytes + 16));
@@ -1174,7 +1193,7 @@ struct DevicePipeline {
             tp.tb_start = abs_start;
             CK(launch_pack(tp, Ln.ssoff.as<unsigned long long>(), Ln.hitidx.as<unsigned long long>(), Ln.o_arena.as<char>(),
                            Ln.o_hits.as<mirfold_hit>(), (unsigned long long)arena.size(), st));
-            CK(cudaEventRecord(Ln.ev[5], st));
+            CK(cudaEventRecord(Ln.ev[EV_PACK_END], st));
             if (nhits) CK(cudaMemcpyAsync(Ln.h_hits.p, Ln.o_hits.p, nhits * sizeof(mirfold_hit), cudaMemcpyDeviceToHost, st));
             if (abytes) CK(cudaMemcpyAsync(Ln.h_arena.p, Ln.o_arena.p, abytes, cudaMemcpyDeviceToHost, st));
             carry = !last && ntb > 0;
@@ -1184,13 +1203,13 @@ struct DevicePipeline {
                 CK(cudaMemcpyAsync(&carry_len, tb.tb_len + (ntb - 1), 4, cudaMemcpyDeviceToHost, st));
                 CK(cudaMemcpyAsync(&carry_start, abs_start + (ntb - 1), 4, cudaMemcpyDeviceToHost, st));
             }
-            CK(cudaEventRecord(Ln.ev[6], st));
+            CK(cudaEventRecord(Ln.ev[EV_D2H_END], st));
             CK(cudaStreamSynchronize(st));
             out.st.kernel_launches += 1 + (m ? 1 : 0) + (ntb ? 2 : 0);   // k_plan_seg, k_traceback, k_emit_seg, k_pack
             out.st.d2h_bytes += nhits * sizeof(mirfold_hit) + abytes + 32;
             hits.insert(hits.end(), Ln.h_hits.as<mirfold_hit>(), Ln.h_hits.as<mirfold_hit>() + nhits);
             arena.insert(arena.end(), Ln.h_arena.as<char>(), Ln.h_arena.as<char>() + abytes);
-            segment_times(Ln);
+            add_stage_times(Ln, sg == 0);
         }
         int total = 0;
         CK(cudaMemcpyAsync(&total, Ln.F.as<int>() + d.seq_off + 1, 4, cudaMemcpyDeviceToHost, st));
@@ -1198,58 +1217,17 @@ struct DevicePipeline {
         CK(cudaStreamSynchronize(st));
         out.st.d2h_bytes += 4;
         ht.mark("segmented locus");
-        return publish_segmented(Ln, l.rec, hits, arena, total, last_chunk);
+        return publish_segmented(Ln, hits, arena, total, last_chunk);
     }
 
-    void segment_times(Lane &Ln)
-    {
-        float ms = 0;
-        cudaEventElapsedTime(&ms, Ln.ev[2], Ln.ev[3]); out.st.ms_fill += ms;
-        cudaEventElapsedTime(&ms, Ln.ev[3], Ln.ev[4]); out.st.ms_f3 += ms;
-        cudaEventElapsedTime(&ms, Ln.ev[4], Ln.ev[5]); out.st.ms_trace += ms;
-        cudaEventElapsedTime(&ms, Ln.ev[5], Ln.ev[6]); out.st.ms_d2h += ms;
-    }
-
-    // the segmented record's staged hits (ss_off relative to its own arena) into the call's sink, as one record
-    bool publish_segmented(Lane &Ln, uint32_t r, const std::vector<mirfold_hit> &hits, const std::vector<char> &arena, int total,
-                           bool last_chunk)
+    // the segmented record's staged hits (ss_off relative to its own arena) into the call's sink, as a chunk of one record
+    bool publish_segmented(Lane &Ln, const std::vector<mirfold_hit> &hits, const std::vector<char> &arena, int total, bool last_chunk)
     {
         const uint64_t nh = hits.size(), ab = arena.size();
-        float ms = 0;
-        cudaEventElapsedTime(&ms, Ln.ev[0], Ln.ev[1]); out.st.ms_h2d += ms;
-        if (J.sink == SINK_TOTALS) { J.totals[r] = total; return true; }
         out.nhits += nh;
         out.arena_bytes += ab;
-        if (J.sink == SINK_SHARED) {
-            SharedOut &S = *J.shared;
-            uint64_t hb = 0, abase = 0;
-            mirfold_hit *dh;
-            char *da;
-            std::unique_ptr<OverflowChunk> O;
-            if (S.reserve(nh, ab, hb, abase)) { dh = S.hits.as<mirfold_hit>() + hb; da = S.arena.as<char>() + abase; }
-            else {
-                O.reset(new OverflowChunk());
-                CK(O->hits.ensure(nh * sizeof(mirfold_hit) + 16));
-                CK(O->arena.ensure(ab + 16));
-                O->nhits = nh; O->abytes = ab;
-                O->recs = {r}; O->begin = {0}; O->count = {(uint32_t)nh};
-                dh = O->hits.as<mirfold_hit>(); da = O->arena.as<char>();
-            }
-            for (uint64_t k = 0; k < nh; k++) { dh[k] = hits[k]; dh[k].ss_off += abase; }
-            if (ab) memcpy(da, arena.data(), ab);
-            S.totals[r] = total;
-            if (O) { std::lock_guard<std::mutex> lk(S.mu); S.overflow.push_back(std::move(O)); }
-            else { S.hit_begin[r] = hb; S.hit_count[r] = (uint32_t)nh; }
-        } else if (J.sink == SINK_STREAM) {
-            uint64_t begin = 0;
-            uint32_t count = (uint32_t)nh;
-            mirfold_chunk c{};
-            c.n_records = 1; c.device = D.id;
-            c.record = &r; c.hit_begin = &begin; c.hit_count = &count; c.total_mfe_dcal = &total;
-            c.nhits = nh; c.hits = hits.data(); c.ss_arena = arena.data(); c.ss_bytes = ab;
-            std::lock_guard<std::mutex> lk(*J.cb_mu);
-            if (!J.cb_abort->load() && J.fn(J.user, &c) != 0) J.cb_abort->store(1);
-        } else if (J.sink == SINK_CAND) {   // stages 1 + 3 on the record's hits, uploaded again as a chunk of one locus
+        Ln.nhits = nh; Ln.abytes = ab;
+        if (J.sink == SINK_CAND) {   // stages 1 + 3 on the record's hits, uploaded again as a chunk of one locus
             cudaStream_t hi = Ln.s_hi;
             const unsigned long long bounds[2] = {0, nh};
             CK(Ln.o_hits.ensure(nh * sizeof(mirfold_hit) + 16));
@@ -1263,12 +1241,26 @@ struct DevicePipeline {
             out.st.h2d_bytes += nh * sizeof(mirfold_hit) + ab + 20;
             Ln.tb = TraceBuffers{};
             Ln.tb.loci = Ln.loci.as<LocusDesc>(); Ln.tb.nloci = 1;
-            Ln.nhits = nh; Ln.abytes = ab; Ln.arena_base = 0;
+            Ln.arena_base = 0;
             if (!back_candidates(Ln, last_chunk, true)) return false;
-            CK(cudaEventRecord(Ln.ev[6], hi));
-            CK(cudaEventSynchronize(Ln.ev[6]));
+            CK(cudaEventRecord(Ln.ev[EV_D2H_END], hi));
+            CK(cudaEventSynchronize(Ln.ev[EV_D2H_END]));
             retire_candidates(Ln);
+            return true;
         }
+        // the segment loop is done with Ln.h_hits / h_arena: the stream sink's destination may be those
+        mirfold_hit *dst_hits;
+        char *dst_arena;
+        if (!pick_destination(Ln, dst_hits, dst_arena)) return false;
+        if (dst_hits) {
+            for (uint64_t k = 0; k < nh; k++) { dst_hits[k] = hits[k]; dst_hits[k].ss_off += Ln.arena_base; }   // as k_pack adds it
+            if (ab) memcpy(dst_arena, arena.data(), ab);
+        }
+        CK(Ln.h_out.ensure(2 * 8 + 4 + 64));
+        unsigned long long *h_bounds = Ln.h_out.as<unsigned long long>();
+        h_bounds[0] = 0; h_bounds[1] = nh;
+        *(int *)(h_bounds + 2) = total;
+        publish(Ln);
         return true;
     }
 
@@ -1294,37 +1286,29 @@ struct DevicePipeline {
         }
     }
 
-    // ---- retire: wait for the lane's download, publish the chunk's per-record tables, collect stage times
-    bool retire(Lane &Ln)
+    // stage times of the chunk or segment whose events the lane last recorded (all complete); h2d: its uploads too
+    void add_stage_times(const Lane &Ln, bool h2d)
     {
-        if (!Ln.pending) return true;
-        Ln.pending = false;
-        CK(cudaEventSynchronize(Ln.ev[6]));
+        float ms = 0;
+        if (h2d) { cudaEventElapsedTime(&ms, Ln.ev[EV_H2D], Ln.ev[EV_KERNELS]); out.st.ms_h2d += ms; }
+        cudaEventElapsedTime(&ms, Ln.ev[EV_FILL], Ln.ev[EV_FILL_END]); out.st.ms_fill += ms;
+        cudaEventElapsedTime(&ms, Ln.ev[EV_FILL_END], Ln.ev[EV_F3_END]); out.st.ms_f3 += ms;
+        cudaEventElapsedTime(&ms, Ln.ev[EV_F3_END], Ln.ev[EV_PACK_END]); out.st.ms_trace += ms;
+        cudaEventElapsedTime(&ms, Ln.ev[EV_PACK_END], Ln.ev[EV_D2H_END]); out.st.ms_d2h += ms;
+    }
+
+    // the chunk's per-record tables (first-hit bounds and totals in Ln.h_out) into the sink; its hits are already where
+    // pick_destination put them
+    void publish(Lane &Ln)
+    {
+        if (J.sink == SINK_NONE) return;
         const Prep &P = Ln.prep;
         const int nl = P.nl;
-        float ms = 0;
-        cudaEventElapsedTime(&ms, Ln.ev[0], Ln.ev[1]); out.st.ms_h2d += ms;
-        cudaEventElapsedTime(&ms, Ln.ev[2], Ln.ev[3]); out.st.ms_fill += ms;
-        cudaEventElapsedTime(&ms, Ln.ev[3], Ln.ev[4]); out.st.ms_f3 += ms;
-        cudaEventElapsedTime(&ms, Ln.ev[4], Ln.ev[5]); out.st.ms_trace += ms;
-        cudaEventElapsedTime(&ms, Ln.ev[5], Ln.ev[6]); out.st.ms_d2h += ms;
-        static const bool trace_events = getenv("MIRFOLD_TRACE_EVENTS") != nullptr;
-        if (trace_events) {   // device timeline of the chunk relative to the call's first event (ms)
-            float t[7];
-            for (int k = 0; k < 7; k++) cudaEventElapsedTime(&t[k], D.ev_first, Ln.ev[k]);
-            fprintf(stderr, "[mirfold events] dev %d lane %d loci %6d  h2d %.2f-%.2f  fill %.2f-%.2f  f3 -%.2f  pack -%.2f  d2h -%.2f\n", D.id,
-                    (int)(&Ln - D.lane), nl, t[0], t[1], t[2], t[3], t[4], t[5], t[6]);
-        }
-        if (J.sink == SINK_NONE) return true;
-        if (J.sink == SINK_CAND) { retire_candidates(Ln); return true; }
-        if (J.sink == SINK_TOTALS) {
-            const int *h = Ln.h_out.as<int>();
-            for (int k = 0; k < nl; k++) J.totals[loci[P.cb + k].rec] = h[k];
-            return true;
-        }
         const unsigned long long *h_bounds = Ln.h_out.as<unsigned long long>();
         const int *h_total = (const int *)(h_bounds + nl + 1);
-        if (J.sink == SINK_SHARED) {
+        if (J.sink == SINK_TOTALS) {
+            for (int k = 0; k < nl; k++) J.totals[loci[P.cb + k].rec] = h_total[k];
+        } else if (J.sink == SINK_SHARED) {
             SharedOut &S = *J.shared;
             if (!Ln.ovf) {
                 for (int k = 0; k < nl; k++) {
@@ -1344,7 +1328,7 @@ struct DevicePipeline {
                 std::lock_guard<std::mutex> lk(S.mu);
                 S.overflow.push_back(std::move(Ln.ovf));
             }
-        } else {
+        } else if (J.sink == SINK_STREAM) {
             Ln.s_rec.resize(nl); Ln.s_begin.resize(nl); Ln.s_count.resize(nl); Ln.s_total.resize(nl);
             for (int k = 0; k < nl; k++) {
                 Ln.s_rec[k] = loci[P.cb + k].rec;
@@ -1361,6 +1345,24 @@ struct DevicePipeline {
             std::lock_guard<std::mutex> lk(*J.cb_mu);
             if (!J.cb_abort->load() && J.fn(J.user, &c) != 0) J.cb_abort->store(1);
         }
+    }
+
+    // ---- retire: wait for the lane's download, collect stage times, publish the chunk's per-record tables
+    bool retire(Lane &Ln)
+    {
+        if (!Ln.pending) return true;
+        Ln.pending = false;
+        CK(cudaEventSynchronize(Ln.ev[EV_D2H_END]));
+        add_stage_times(Ln, true);
+        static const bool trace_events = getenv("MIRFOLD_TRACE_EVENTS") != nullptr;
+        if (trace_events) {   // device timeline of the chunk relative to the call's first event (ms)
+            float t[EV_D2H_END + 1];
+            for (int k = 0; k <= EV_D2H_END; k++) cudaEventElapsedTime(&t[k], D.ev_first, Ln.ev[k]);
+            fprintf(stderr, "[mirfold events] dev %d lane %d loci %6d  h2d %.2f-%.2f  fill %.2f-%.2f  f3 -%.2f  pack -%.2f  d2h -%.2f\n", D.id,
+                    (int)(&Ln - D.lane), Ln.prep.nl, t[0], t[1], t[2], t[3], t[4], t[5], t[6]);
+        }
+        if (J.sink == SINK_CAND) retire_candidates(Ln);
+        else publish(Ln);
         ht.mark("retire (download wait + record tables)");
         return true;
     }
@@ -2321,11 +2323,7 @@ int mirfold_debug_matrices(mirfold_ctx *ctx, const char *seq, uint32_t n, int sp
     CK(launch_prepare(Ln.raw.as<char>(), dl, 1, n + 3, Ln.codes.as<unsigned char>(), Ln.F.as<int>(), st));
     CK(Ln.fillflags.ensure((size_t)nu * 4 + 4));
     CK(cudaMemsetAsync(Ln.fillflags.p, 0, (size_t)nu * 4 + 4, st));
-    FillLaunch fa{Ln.units.as<LocusDesc>(), nu, max_n, Ln.codes.as<unsigned char>(), Ln.C.as<int>(), Ln.M.as<int>(), Ln.ring.as<int>(),
-                  Ln.Ib.as<unsigned char>(), Ln.Mp.as<unsigned int>(), D.dP, {0, 0, 0, 0, 0, 0}, Ln.fillflags.as<int>(),
-                  ((flags & MIRFOLD_FLAG_WIDE) || span_L > MF16_MAX_SPAN) ? 1 : 0, env_opts() | (span_L >= MF_DYNW_MIN_SPAN ? 8 : 0)};
-    for (int b = 0; b < 6; b++) fa.bucket_first[b] = bucket_first[b];
-    CK(launch_fill(fa, st));
+    CK(launch_fill(fill_launch(Ln, D.dP, nu, max_n, bucket_first, (flags & MIRFOLD_FLAG_WIDE) || span_L > MF16_MAX_SPAN, span_L), st));
     CK(launch_f3(dl, 1, d.n > MF_TILE_LEN ? 1 : 0, d.Ls, Ln.codes.as<unsigned char>(), Ln.C.as<int>(), Ln.F.as<int>(), D.dP, st));
     std::vector<int> hc(cells), hm(cells), hf(n + 3);
     CK(cudaMemcpyAsync(hc.data(), Ln.C.p, cells * 4, cudaMemcpyDeviceToHost, st));

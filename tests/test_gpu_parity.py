@@ -372,9 +372,12 @@ def test_multi_device_sharding_matches_single(mf):
 
 def test_result_buffer_overflow_path(mf):
     """The shared result buffers are sized from an estimate; chunks that do not fit take the overflow path and the
-    result is rebuilt once at exact size.  MIRFOLD_RESULT_CAP_SCALE shrinks the estimate to force it."""
+    result is rebuilt once at exact size.  MIRFOLD_RESULT_CAP_SCALE shrinks the estimate to force it.  The 12 kb locus
+    is larger than the 16 MB budget and is folded in segments, so a segmented record takes the overflow path too."""
     import mir_prefer_b200 as mp
-    seqs = synth_loci(43, 120, (200, 420))
+    from mir_prefer_b200.fold import plan_segments
+    seqs = synth_loci(43, 120, (200, 420)) + synth_loci(47, 1, (12_000, 12_000))
+    assert len(plan_segments(12_000, 300, (16 << 20) // 2)) > 1   # one lane's share of the budget
     with mf.fold(seqs, 300) as a:
         want = _records(a, len(seqs))
     os.environ["MIRFOLD_MEM_BUDGET_MB"] = "16"

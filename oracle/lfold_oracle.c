@@ -87,7 +87,25 @@ typedef struct {
     short *S, *S1;  /* 1-based codes                                                         */
     int *c, *m, *dml; /* [ (n+2) rows ][ W ]                                                 */
     int *f3;        /* n+3                                                                   */
+    int mut;        /* TB_* tie-break mutations of traceback(); 0 = the reference's rules    */
 } fold_t;
+
+/* Tie-break mutants (tests only).  Each bit flips one "first match wins" rule of traceback(), so
+ * that a test corpus can show it contains ties that rule has to break: a corpus on which a
+ * mutant prints the same records as the unmodified oracle cannot tell a GPU traceback that
+ * breaks that tie the other way from a correct one.  mut = 0 is the reference's traceback. */
+enum {
+    TB_F3_LAST = 1 << 0,        /* exterior scan: last k instead of first                       */
+    TB_F3_ORDER = 1 << 1,       /* exterior scan, one k: (i+1,k) wins over (i,k)                */
+    TB_HAIRPIN_LAST = 1 << 2,   /* pair: two-loop tried before hairpin                          */
+    TB_LOOP_LAST = 1 << 3,      /* two-loop scan: last (p,q) instead of first                   */
+    TB_ML_BEFORE_LOOP = 1 << 4, /* pair: multiloop closing tried before two-loop                */
+    TB_MLC_LAST = 1 << 5,       /* multiloop closing: last split k instead of first             */
+    TB_MLC_VARIANT = 1 << 6,    /* multiloop closing, one k: dangle variants in reverse order    */
+    TB_FML_PEEL_5 = 1 << 7,     /* fML segment: peel the 5' base before the 3' base             */
+    TB_FML_PAIR_ORDER = 1 << 8, /* fML segment: cij > ci1j1 > cij1 > ci1j instead of the reverse */
+    TB_FML_SPLIT_LAST = 1 << 9, /* fML segment: last split k instead of first                   */
+};
 
 static inline int enc(char ch)
 {   /* A.1: index in "_ACGUTXKI", indices >4 decremented; anything else 0 */
@@ -237,6 +255,45 @@ static void f3_row(fold_t *f, int i)
 /* ------------------------------------------------------------------ A.4 traceback */
 typedef struct { int i, j, ml; } sect_t;
 
+/* two-loop (p,q) that reproduces c(i,j): p ascending, q descending, first match (last with TB_LOOP_LAST) */
+static int two_loop_split(const fold_t *f, int i, int j, int cij, int t, int *pp, int *qq)
+{
+    int found = 0;
+    int pmax = imin(j - 2 - TURN, i + MAXLOOP + 1);
+    for (int p = i + 1; p <= pmax; p++) {
+        int minq = j - i + p - MAXLOOP - 2;
+        if (minq < p + 1 + TURN) minq = p + 1 + TURN;
+        for (int q = j - 1; q >= minq; q--) {
+            int t2 = ptype(f, p, q);
+            if (!t2) continue;
+            if (cij == loop_E(f, i, j, p, q, t, P.rtype[t2]) + C_(p, q)) {
+                *pp = p; *qq = q; found = 1;
+                if (!(f->mut & TB_LOOP_LAST)) return 1;
+            }
+        }
+    }
+    return found;
+}
+
+/* multiloop closed by (i,j): split k ascending (descending with TB_MLC_LAST), four dangle variants per k */
+static int ml_split(const fold_t *f, int i, int j, int cij, int t, int *kk, int *i1, int *j1)
+{
+    int tt = P.rtype[t];
+    int mm = P.MLclosing + P.MLintern[tt];
+    int d5 = P.dangle5[tt][f->S1[j - 1]], d3 = P.dangle3[tt][f->S1[i + 1]];
+    const int klo = i + 2 + TURN, khi = j - 3 - TURN;
+    const int last = (f->mut & TB_MLC_LAST) != 0, rev = (f->mut & TB_MLC_VARIANT) != 0;
+    for (int s = 0; s <= khi - klo; s++) {
+        int k = last ? khi - s : klo + s;
+        for (int o = 0; o < 4; o++) {
+            int v = rev ? 3 - o : o, a = v & 1, b = v >> 1;   /* v: 0 (i+1,j-1), 1 (i+2,j-1), 2 (i+1,j-2), 3 (i+2,j-2) */
+            int e = M_(i + 1 + a, k) + M_(k + 1, j - 1 - b) + mm + (a ? d3 : 0) + (b ? d5 : 0) + (a + b) * P.MLbase;
+            if (cij == e) { *kk = k; *i1 = i + 1 + a; *j1 = j - 1 - b; return 1; }
+        }
+    }
+    return 0;
+}
+
 /* returns malloc'ed finalised structure string, or NULL on "backtrack failed" */
 static char *traceback(fold_t *f, int start, int md)
 {
@@ -256,32 +313,36 @@ static char *traceback(fold_t *f, int start, int md)
         if (ml == 0) {
             int fij = F_(f, i);
             if (fij == F_(f, i + 1)) { PUSH(i + 1, j, 0); continue; }
-            int traced = 0, jj = 0, k;
+            /* per k the later match wins: (i+1,k) then (i,k) (reversed by TB_F3_ORDER), no dangle then 3' dangle */
+            int traced = 0, jj = 0, k, bt = 0, bjj = 0, bk = 0;
             for (k = i + TURN + 1; k <= j; k++) {
                 jj = k + 1;
-                int t = ptype(f, i + 1, k);
-                if (t) {
-                    int cc = C_(i + 1, k) + P.dangle5[t][S1[i]] + AU(t);
-                    if (fij == cc + F_(f, k + 1)) traced = i + 1;
-                    if (k < n && fij == F_(f, k + 2) + cc + P.dangle3[t][S1[k + 1]]) { traced = i + 1; jj = k + 2; }
+                traced = 0;
+                for (int o = 0; o < 2; o++) {
+                    int a = (o == 0) == !(f->mut & TB_F3_ORDER) ? i + 1 : i;
+                    int t = ptype(f, a, k);
+                    if (!t) continue;
+                    int cc = C_(a, k) + (a > i ? P.dangle5[t][S1[i]] : 0) + AU(t);
+                    if (fij == cc + F_(f, k + 1)) traced = a;
+                    if (k < n && fij == F_(f, k + 2) + cc + P.dangle3[t][S1[k + 1]]) { traced = a; jj = k + 2; }
                 }
-                t = ptype(f, i, k);
-                if (t) {
-                    int cc = C_(i, k) + AU(t);
-                    if (fij == cc + F_(f, k + 1)) traced = i;
-                    if (k < n && fij == F_(f, k + 2) + cc + P.dangle3[t][S1[k + 1]]) { traced = i; jj = k + 2; }
+                if (traced) {
+                    bt = traced; bjj = jj; bk = k;
+                    if (!(f->mut & TB_F3_LAST)) break;
                 }
-                if (traced) break;
             }
-            if (!traced) goto fail;
+            if (!bt) goto fail;
+            traced = bt; jj = bjj; k = bk;
             if (j == n) PUSH(jj, j, 0);
             i = traced; j = k;
             st[i - start] = '('; st[j - start] = ')';
             if (jj == j + 2 && j < n) st[j + 1 - start] = '.';
         } else {
             int fij = M_(i, j);
-            if (M_(i, j - 1) + P.MLbase == fij) { PUSH(i, j - 1, 1); continue; }
-            if (M_(i + 1, j) + P.MLbase == fij) { PUSH(i + 1, j, 1); continue; }
+            for (int o = 0; o < 2; o++) {   /* 3' base first (5' first with TB_FML_PEEL_5) */
+                int five = (o == 0) == !!(f->mut & TB_FML_PEEL_5);
+                if (M_(i + five, j - !five) + P.MLbase == fij) { PUSH(i + five, j - !five, 1); goto next; }
+            }
             int t = ptype(f, i, j);
             int cij = C_(i, j) + P.MLintern[t];
             t = ptype(f, i + 1, j);
@@ -291,56 +352,49 @@ static char *traceback(fold_t *f, int start, int md)
             t = ptype(f, i + 1, j - 1);
             int ci1j1 = C_(i + 1, j - 1) + P.dangle5[t][S1[i]] + P.dangle3[t][S1[j]] + P.MLintern[t] + 2 * P.MLbase;
             if (fij == cij || fij == ci1j || fij == cij1 || fij == ci1j1) {
-                if (fij == ci1j) i++;
-                else if (fij == cij1) j--;
-                else if (fij == ci1j1) { i++; j--; }
+                /* first match of ci1j, cij1, ci1j1, cij (the reverse with TB_FML_PAIR_ORDER) */
+                const int e[4] = {ci1j, cij1, ci1j1, cij}, di[4] = {1, 0, 1, 0}, dj[4] = {0, 1, 1, 0};
+                for (int o = 0; o < 4; o++) {
+                    int v = (f->mut & TB_FML_PAIR_ORDER) ? 3 - o : o;
+                    if (fij == e[v]) { i += di[v]; j -= dj[v]; break; }
+                }
                 st[i - start] = '('; st[j - start] = ')';
             } else {
-                int k;
-                for (k = i + 1 + TURN; k <= j - 2 - TURN; k++)
-                    if (fij == M_(i, k) + M_(k + 1, j)) break;
-                if (k > j - 2 - TURN) goto fail;
+                int k, found = 0;
+                for (k = i + 1 + TURN; k <= j - 2 - TURN; k++) {
+                    int kk = (f->mut & TB_FML_SPLIT_LAST) ? i + j - 1 - k : k;   /* j-2-TURN .. i+1+TURN */
+                    if (fij == M_(i, kk) + M_(kk + 1, j)) { k = kk; found = 1; break; }
+                }
+                if (!found) goto fail;
                 PUSH(i, k, 1);
                 PUSH(k + 1, j, 1);
                 continue;
             }
         }
-        /* "repeat": (i,j) is a known pair; walk the stem/interior loops down */
+        /* "repeat": (i,j) is a known pair; walk the stem/interior loops down.  Hairpin, then two-loop, then
+         * multiloop; TB_HAIRPIN_LAST and TB_ML_BEFORE_LOOP reorder these (0 hairpin, 1 two-loop, 2 multiloop). */
         for (;;) {
             int cij = C_(i, j), t = ptype(f, i, j);
-            if (cij == hairpin_E(f, i, j)) break;
-            int found = 0;
-            int pmax = imin(j - 2 - TURN, i + MAXLOOP + 1);
-            for (int p = i + 1; p <= pmax && !found; p++) {
-                int minq = j - i + p - MAXLOOP - 2;
-                if (minq < p + 1 + TURN) minq = p + 1 + TURN;
-                for (int q = j - 1; q >= minq; q--) {
-                    int t2 = ptype(f, p, q);
-                    if (!t2) continue;
-                    if (cij == loop_E(f, i, j, p, q, t, P.rtype[t2]) + C_(p, q)) {
-                        st[p - start] = '('; st[q - start] = ')';
-                        i = p; j = q; found = 1;
-                        break;
-                    }
-                }
+            static const int ORDER[4][3] = {{0, 1, 2}, {1, 0, 2}, {0, 2, 1}, {2, 1, 0}};
+            const int *ord = ORDER[((f->mut & TB_HAIRPIN_LAST) ? 1 : 0) + ((f->mut & TB_ML_BEFORE_LOOP) ? 2 : 0)];
+            int step = -1, p = 0, q = 0, k = 0, i1 = 0, j1 = 0;
+            for (int o = 0; o < 3 && step < 0; o++) {
+                if (ord[o] == 0 && cij == hairpin_E(f, i, j)) step = 0;
+                else if (ord[o] == 1 && two_loop_split(f, i, j, cij, t, &p, &q)) step = 1;
+                else if (ord[o] == 2 && ml_split(f, i, j, cij, t, &k, &i1, &j1)) step = 2;
             }
-            if (found) continue;
-            /* multiloop */
-            int tt = P.rtype[t];
-            int mm = P.MLclosing + P.MLintern[tt];
-            int d5 = P.dangle5[tt][S1[j - 1]], d3 = P.dangle3[tt][S1[i + 1]];
-            int i1 = i + 1, j1 = j - 1, k;
-            for (k = i + 2 + TURN; k < j - 2 - TURN; k++) {
-                if (cij == M_(i + 1, k) + M_(k + 1, j - 1) + mm) break;
-                if (cij == M_(i + 2, k) + M_(k + 1, j - 1) + mm + d3 + P.MLbase) { i1 = i + 2; break; }
-                if (cij == M_(i + 1, k) + M_(k + 1, j - 2) + mm + d5 + P.MLbase) { j1 = j - 2; break; }
-                if (cij == M_(i + 2, k) + M_(k + 1, j - 2) + mm + d3 + d5 + 2 * P.MLbase) { i1 = i + 2; j1 = j - 2; break; }
+            if (step < 0) goto fail;
+            if (step == 0) break;
+            if (step == 1) {
+                st[p - start] = '('; st[q - start] = ')';
+                i = p; j = q;
+                continue;
             }
-            if (k > j - 3 - TURN) goto fail;
             PUSH(i1, k, 1);
             PUSH(k + 1, j1, 1);
             break;
         }
+    next:
         if (sp + 4 > cap) { cap *= 2; stk = (sect_t *)realloc(stk, sizeof(sect_t) * (size_t)cap); }
     }
     free(stk);
@@ -387,8 +441,9 @@ static void add_hit(lfold_result *r, const fold_t *f, char *ss, int start)
     r->n_hits++;
 }
 
-/* Fold one raw sequence token (A.6 conversion, A.3 fill, A.5 emission). */
-lfold_result *lfold_oracle_fold(const char *raw, int n, int L, int keep_matrices)
+/* Fold one raw sequence token (A.6 conversion, A.3 fill, A.5 emission); `mut`: TB_* bits of the
+ * tracebacks (0 = RNALfold's). */
+lfold_result *lfold_oracle_fold_mut(const char *raw, int n, int L, int keep_matrices, int mut)
 {
     params_init();
     lfold_result *r = (lfold_result *)calloc(1, sizeof *r);
@@ -415,6 +470,7 @@ lfold_result *lfold_oracle_fold(const char *raw, int n, int L, int keep_matrices
     f->dml = (int *)malloc(sizeof(int) * cells);
     for (size_t k = 0; k < cells; k++) f->c[k] = f->m[k] = f->dml[k] = INF;
     f->f3 = (int *)calloc((size_t)n + 4, sizeof(int));
+    f->mut = mut;
 
     /* A.5 emission state machine, static state is per-call here (one Lfold() per process
      * call sequence in the reference keeps statics across records, but they are always
@@ -455,6 +511,11 @@ lfold_result *lfold_oracle_fold(const char *raw, int n, int L, int keep_matrices
     else { free(f->c); free(f->m); free(f->f3); }
     free(f->dml); free(f->S); free(f->S1);
     return r;
+}
+
+lfold_result *lfold_oracle_fold(const char *raw, int n, int L, int keep_matrices)
+{
+    return lfold_oracle_fold_mut(raw, n, L, keep_matrices, 0);
 }
 
 void lfold_oracle_free(lfold_result *r)

@@ -12,6 +12,21 @@ CLI = os.path.join(HERE, "_build", "lfold_oracle")
 RLF = os.path.join(HERE, "_ref", "RNALfold")
 _lib = None
 
+# Tie-break mutants of the traceback (lfold_oracle.c, TB_*): each bit flips one "first match wins" rule.  Tests only:
+# a corpus whose output changes under a bit contains ties that rule must break.
+TIEBREAK = {
+    "F3_LAST": 1 << 0,          # exterior scan: last k instead of first
+    "F3_ORDER": 1 << 1,         # exterior scan, one k: (i+1,k) wins over (i,k)
+    "HAIRPIN_LAST": 1 << 2,     # pair: two-loop tried before hairpin
+    "LOOP_LAST": 1 << 3,        # two-loop scan: last (p,q) instead of first
+    "ML_BEFORE_LOOP": 1 << 4,   # pair: multiloop closing tried before two-loop
+    "MLC_LAST": 1 << 5,         # multiloop closing: last split k
+    "MLC_VARIANT": 1 << 6,      # multiloop closing, one k: dangle variants in reverse order
+    "FML_PEEL_5": 1 << 7,       # fML segment: peel the 5' base before the 3' base
+    "FML_PAIR_ORDER": 1 << 8,   # fML segment: cij > ci1j1 > cij1 > ci1j
+    "FML_SPLIT_LAST": 1 << 9,   # fML segment: last split k
+}
+
 
 def build():
     subprocess.run(["make", "-C", HERE, "all"], check=True, stdout=subprocess.DEVNULL)
@@ -25,6 +40,8 @@ def lib():
         L = C.CDLL(SO)
         L.lfold_oracle_fold.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_int]
         L.lfold_oracle_fold.restype = C.c_void_p
+        L.lfold_oracle_fold_mut.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int]
+        L.lfold_oracle_fold_mut.restype = C.c_void_p
         L.lfold_oracle_free.argtypes = [C.c_void_p]
         for name in ("nhits", "total", "failed", "W"):
             getattr(L, "lfold_oracle_" + name).argtypes = [C.c_void_p]
@@ -43,11 +60,11 @@ def lib():
     return _lib
 
 
-def fold(seq, span, matrices=False):
-    """-> dict(hits=[(ss, energy_dcal, start)], total=int[, c, m, f3])"""
+def fold(seq, span, matrices=False, tiebreak=0):
+    """-> dict(hits=[(ss, energy_dcal, start)], total=int[, c, m, f3]).  tiebreak: OR of TIEBREAK bits (0 = RNALfold)."""
     L = lib()
     b = seq.encode() if isinstance(seq, str) else seq
-    r = L.lfold_oracle_fold(b, len(b), span, 1 if matrices else 0)
+    r = L.lfold_oracle_fold_mut(b, len(b), span, 1 if matrices else 0, int(tiebreak))
     try:
         if L.lfold_oracle_failed(r):
             raise RuntimeError("oracle: backtrack failed")

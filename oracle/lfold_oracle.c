@@ -43,7 +43,7 @@ typedef struct {
     int pair[8][8], rtype[8];
 } params_t;
 
-static params_t P;
+static params_t P0;
 static int P_ready = 0;
 
 /* scale_parameters at T=37: tables are taken as-is; dangles clamped to <= 0; MLintern[t] gets
@@ -51,31 +51,31 @@ static int P_ready = 0;
 static void params_init(void)
 {
     if (P_ready) return;
-    memcpy(P.stack, T99_stack37, sizeof P.stack);
-    memcpy(P.hairpin, T99_hairpin37, sizeof P.hairpin);
-    memcpy(P.bulge, T99_bulge37, sizeof P.bulge);
-    memcpy(P.internal_loop, T99_internal_loop37, sizeof P.internal_loop);
-    memcpy(P.mismatchI, T99_mismatchI37, sizeof P.mismatchI);
-    memcpy(P.mismatchH, T99_mismatchH37, sizeof P.mismatchH);
-    memcpy(P.int11, T99_int11_37, sizeof P.int11);
-    memcpy(P.int21, T99_int21_37, sizeof P.int21);
-    memcpy(P.int22, T99_int22_37, sizeof P.int22);
-    memcpy(P.pair, T99_BP_pair, sizeof P.pair);
-    memcpy(P.rtype, T99_rtype, sizeof P.rtype);
+    memcpy(P0.stack, T99_stack37, sizeof P0.stack);
+    memcpy(P0.hairpin, T99_hairpin37, sizeof P0.hairpin);
+    memcpy(P0.bulge, T99_bulge37, sizeof P0.bulge);
+    memcpy(P0.internal_loop, T99_internal_loop37, sizeof P0.internal_loop);
+    memcpy(P0.mismatchI, T99_mismatchI37, sizeof P0.mismatchI);
+    memcpy(P0.mismatchH, T99_mismatchH37, sizeof P0.mismatchH);
+    memcpy(P0.int11, T99_int11_37, sizeof P0.int11);
+    memcpy(P0.int21, T99_int21_37, sizeof P0.int21);
+    memcpy(P0.int22, T99_int22_37, sizeof P0.int22);
+    memcpy(P0.pair, T99_BP_pair, sizeof P0.pair);
+    memcpy(P0.rtype, T99_rtype, sizeof P0.rtype);
     for (int t = 0; t < 8; t++)
         for (int b = 0; b < 5; b++) {
             int d5 = T99_dangle5_37[t * 5 + b], d3 = T99_dangle3_37[t * 5 + b];
-            P.dangle5[t][b] = d5 > 0 ? 0 : d5;
-            P.dangle3[t][b] = d3 > 0 ? 0 : d3;
+            P0.dangle5[t][b] = d5 > 0 ? 0 : d5;
+            P0.dangle3[t][b] = d3 > 0 ? 0 : d3;
         }
-    P.TerminalAU = T99_TerminalAU;
-    for (int t = 0; t < 8; t++) P.MLintern[t] = T99_ML_intern37 + (t > 2 ? P.TerminalAU : 0);
-    P.MLbase = 0;
-    P.MLclosing = T99_ML_closing37;
-    P.ninio2 = T99_F_ninio37[2];
-    P.max_ninio = T99_MAX_NINIO;
-    P.lxc = T99_lxc37;
-    for (int k = 0; k < T99_N_TETRALOOPS; k++) P.tetra_energy[k] = T99_TETRA_ENERGY37[k];
+    P0.TerminalAU = T99_TerminalAU;
+    for (int t = 0; t < 8; t++) P0.MLintern[t] = T99_ML_intern37 + (t > 2 ? P0.TerminalAU : 0);
+    P0.MLbase = 0;
+    P0.MLclosing = T99_ML_closing37;
+    P0.ninio2 = T99_F_ninio37[2];
+    P0.max_ninio = T99_MAX_NINIO;
+    P0.lxc = T99_lxc37;
+    for (int k = 0; k < T99_N_TETRALOOPS; k++) P0.tetra_energy[k] = T99_TETRA_ENERGY37[k];
     P_ready = 1;
 }
 
@@ -88,7 +88,20 @@ typedef struct {
     int *c, *m, *dml; /* [ (n+2) rows ][ W ]                                                 */
     int *f3;        /* n+3                                                                   */
     int mut;        /* TB_* tie-break mutations of traceback(); 0 = the reference's rules    */
+    const params_t *P;  /* energy tables of this fold (&P0, or a copy with one entry changed) */
+    const params_t *PL; /* tables of the two-loops the filter selects (P unless a filter-only entry changes) */
+    int ln1, ln2, lpar, ls, ld; /* two-loop filter: n1, n2, parity of j-i, n1+n2, j-i; -1 = any; ln1 < -1: none */
+    int ldelta;     /* added to every two-loop the filter selects                            */
+    int hs, hdelta; /* added to every hairpin of size hs (after the log extrapolation)       */
 } fold_t;
+
+/* Energy perturbations (tests only): a fold in which one term class costs `delta` more.  A class whose raise changes the c
+ * matrix is the unique minimiser of some cell, so a kernel that computes that class wrongly must differ from the oracle
+ * in that cell.  PERT_NONE is the reference. */
+enum {
+    PERT_NONE, PERT_SHAPE, PERT_RING, PERT_HAIRPIN_SIZE, PERT_STACK, PERT_BULGE, PERT_INTERNAL, PERT_INT11, PERT_INT21,
+    PERT_INT22, PERT_MISMATCH_I, PERT_MISMATCH_H, PERT_HAIRPIN, PERT_TETRA,
+};
 
 /* Tie-break mutants (tests only).  Each bit flips one "first match wins" rule of traceback(), so
  * that a test corpus can show it contains ties that rule has to break: a corpus on which a
@@ -121,7 +134,7 @@ static inline int ptype(const fold_t *f, int i, int j)
 {   /* A.1: typed only for 4 <= j-i <= L*-1, j <= n */
     int d = j - i;
     if (i < 1 || j > f->n || d < TURN + 1 || d >= f->Ls) return 0;
-    return P.pair[f->S[i]][f->S[j]];
+    return P0.pair[f->S[i]][f->S[j]];
 }
 static inline int band_get(const fold_t *f, const int *a, int i, int j)
 {
@@ -133,45 +146,56 @@ static inline int band_get(const fold_t *f, const int *a, int i, int j)
 #define M_(i, j) band_get(f, f->m, (i), (j))
 #define D_(i, j) band_get(f, f->dml, (i), (j))
 static inline int F_(const fold_t *f, int i) { return (i >= 1 && i <= f->n + 2) ? f->f3[i] : 0; }
-static inline int AU(int t) { return t > 2 ? P.TerminalAU : 0; }
+static inline int AU(const params_t *P, int t) { return t > 2 ? P->TerminalAU : 0; }
 
-/* A.2 hairpin */
-static int hairpin_E(const fold_t *f, int i, int j)
+/* A.2 hairpin, size s = j-i-1 before any perturbation */
+static int hairpin_tab(const params_t *P, const char *seq, const short *S1, int i, int j, int t)
 {
-    int s = j - i - 1, t = ptype(f, i, j);
-    int e = s <= 30 ? P.hairpin[s] : P.hairpin[30] + (int)(P.lxc * log(s / 30.));
+    int s = j - i - 1;
+    int e = s <= 30 ? P->hairpin[s] : P->hairpin[30] + (int)(P->lxc * log(s / 30.));
     if (s == 4) {
         char six[7];
-        memcpy(six, f->seq + (i - 1), 6);
+        memcpy(six, seq + (i - 1), 6);
         six[6] = 0;
         const char *hit = strstr(T99_Tetraloops, six);
-        if (hit) e += P.tetra_energy[(hit - T99_Tetraloops) / 7];
+        if (hit) e += P->tetra_energy[(hit - T99_Tetraloops) / 7];
     }
-    if (s == 3) e += AU(t);            /* no mismatch, Triloops empty */
-    else e += P.mismatchH[t][f->S1[i + 1]][f->S1[j - 1]];
+    if (s == 3) e += AU(P, t);            /* no mismatch, Triloops empty */
+    else e += P->mismatchH[t][S1[i + 1]][S1[j - 1]];
     return e;
+}
+static int hairpin_E(const fold_t *f, int i, int j)
+{
+    return hairpin_tab(f->P, f->seq, f->S1, i, j, ptype(f, i, j)) + (j - i - 1 == f->hs ? f->hdelta : 0);
 }
 
 /* A.2 two-loop closed by (i,j) [type t] and (p,q) [t2 = rtype of its type] */
-static int loop_E(const fold_t *f, int i, int j, int p, int q, int t, int t2)
+static int loop_tab(const params_t *P, const short *S1, int i, int j, int p, int q, int t, int t2)
 {
     int n1 = p - i - 1, n2 = j - q - 1;
     int nl = n1 > n2 ? n1 : n2, ns = n1 > n2 ? n2 : n1;
-    const short *S1 = f->S1;
-    if (nl == 0) return P.stack[t][t2];
+    if (nl == 0) return P->stack[t][t2];
     if (ns == 0) {
-        int e = P.bulge[nl];
-        return nl == 1 ? e + P.stack[t][t2] : e + AU(t) + AU(t2);
+        int e = P->bulge[nl];
+        return nl == 1 ? e + P->stack[t][t2] : e + AU(P, t) + AU(P, t2);
     }
-    if (ns == 1 && nl == 1) return P.int11[t][t2][S1[i + 1]][S1[j - 1]];
+    if (ns == 1 && nl == 1) return P->int11[t][t2][S1[i + 1]][S1[j - 1]];
     if (ns == 1 && nl == 2)
-        return n1 == 1 ? P.int21[t][t2][S1[i + 1]][S1[q + 1]][S1[j - 1]]
-                       : P.int21[t2][t][S1[q + 1]][S1[i + 1]][S1[p - 1]];
-    if (n1 == 2 && n2 == 2) return P.int22[t][t2][S1[i + 1]][S1[p - 1]][S1[q + 1]][S1[j - 1]];
-    int nin = (nl - ns) * P.ninio2;
-    if (nin > P.max_ninio) nin = P.max_ninio;
-    return P.internal_loop[n1 + n2] + nin + P.mismatchI[t][S1[i + 1]][S1[j - 1]] +
-           P.mismatchI[t2][S1[q + 1]][S1[p - 1]];
+        return n1 == 1 ? P->int21[t][t2][S1[i + 1]][S1[q + 1]][S1[j - 1]]
+                       : P->int21[t2][t][S1[q + 1]][S1[i + 1]][S1[p - 1]];
+    if (n1 == 2 && n2 == 2) return P->int22[t][t2][S1[i + 1]][S1[p - 1]][S1[q + 1]][S1[j - 1]];
+    int nin = (nl - ns) * P->ninio2;
+    if (nin > P->max_ninio) nin = P->max_ninio;
+    return P->internal_loop[n1 + n2] + nin + P->mismatchI[t][S1[i + 1]][S1[j - 1]] +
+           P->mismatchI[t2][S1[q + 1]][S1[p - 1]];
+}
+static int loop_E(const fold_t *f, int i, int j, int p, int q, int t, int t2)
+{
+    int n1 = p - i - 1, n2 = j - q - 1, d = j - i;
+    if (f->ln1 < -1 || (f->ln1 >= 0 && f->ln1 != n1) || (f->ln2 >= 0 && f->ln2 != n2) ||
+        (f->lpar >= 0 && f->lpar != (d & 1)) || (f->ls >= 0 && f->ls != n1 + n2) || (f->ld >= 0 && f->ld != d))
+        return loop_tab(f->P, f->S1, i, j, p, q, t, t2);
+    return loop_tab(f->PL, f->S1, i, j, p, q, t, t2) + f->ldelta;
 }
 
 static inline int imin(int a, int b) { return a < b ? a : b; }
@@ -179,6 +203,7 @@ static inline int imin(int a, int b) { return a < b ? a : b; }
 /* ------------------------------------------------------------------ A.3 fill */
 static void fill_row(fold_t *f, int i)
 {
+    const params_t *P = f->P;
     const int n = f->n, Ls = f->Ls, W = f->W;
     const short *S1 = f->S1;
     int jmax = imin(n, i + Ls);
@@ -193,29 +218,29 @@ static void fill_row(fold_t *f, int i)
                 for (int q = minq; q < j; q++) {
                     int t2 = ptype(f, p, q);
                     if (!t2) continue;
-                    cij = imin(cij, loop_E(f, i, j, p, q, t, P.rtype[t2]) + C_(p, q));
+                    cij = imin(cij, loop_E(f, i, j, p, q, t, P->rtype[t2]) + C_(p, q));
                 }
             }
-            int tt = P.rtype[t];
-            int d3 = P.dangle3[tt][S1[i + 1]], d5 = P.dangle5[tt][S1[j - 1]];
+            int tt = P->rtype[t];
+            int d3 = P->dangle3[tt][S1[i + 1]], d5 = P->dangle5[tt][S1[j - 1]];
             int dec = D_(i + 1, j - 1);
-            dec = imin(dec, D_(i + 2, j - 1) + d3 + P.MLbase);
-            dec = imin(dec, D_(i + 1, j - 2) + d5 + P.MLbase);
-            dec = imin(dec, D_(i + 2, j - 2) + d3 + d5 + 2 * P.MLbase);
-            cij = imin(cij, P.MLclosing + P.MLintern[t] + dec);
+            dec = imin(dec, D_(i + 2, j - 1) + d3 + P->MLbase);
+            dec = imin(dec, D_(i + 1, j - 2) + d5 + P->MLbase);
+            dec = imin(dec, D_(i + 2, j - 2) + d3 + d5 + 2 * P->MLbase);
+            cij = imin(cij, P->MLclosing + P->MLintern[t] + dec);
         }
         f->c[(size_t)i * W + (j - i)] = cij;
 
-        int mij = M_(i + 1, j) + P.MLbase;
-        mij = imin(mij, M_(i, j - 1) + P.MLbase);
-        mij = imin(mij, cij + P.MLintern[t]);
+        int mij = M_(i + 1, j) + P->MLbase;
+        mij = imin(mij, M_(i, j - 1) + P->MLbase);
+        mij = imin(mij, cij + P->MLintern[t]);
         int ta = ptype(f, i + 1, j);
-        mij = imin(mij, C_(i + 1, j) + P.dangle5[ta][S1[i]] + P.MLintern[ta] + P.MLbase);
+        mij = imin(mij, C_(i + 1, j) + P->dangle5[ta][S1[i]] + P->MLintern[ta] + P->MLbase);
         int tb = ptype(f, i, j - 1);
-        mij = imin(mij, C_(i, j - 1) + P.dangle3[tb][S1[j]] + P.MLintern[tb] + P.MLbase);
+        mij = imin(mij, C_(i, j - 1) + P->dangle3[tb][S1[j]] + P->MLintern[tb] + P->MLbase);
         int tc = ptype(f, i + 1, j - 1);
-        mij = imin(mij, C_(i + 1, j - 1) + P.dangle5[tc][S1[i]] + P.dangle3[tc][S1[j]] +
-                            P.MLintern[tc] + 2 * P.MLbase);
+        mij = imin(mij, C_(i + 1, j - 1) + P->dangle5[tc][S1[i]] + P->dangle3[tc][S1[j]] +
+                            P->MLintern[tc] + 2 * P->MLbase);
         int dec = INF;
         for (int k = i + 1 + TURN; k <= j - 2 - TURN; k++) dec = imin(dec, M_(i, k) + M_(k + 1, j));
         f->dml[(size_t)i * W + (j - i)] = dec;
@@ -226,28 +251,29 @@ static void fill_row(fold_t *f, int i)
 
 static void f3_row(fold_t *f, int i)
 {
+    const params_t *P = f->P;
     const int n = f->n, Ls = f->Ls;
     const short *S1 = f->S1;
     int fi = F_(f, i + 1);
     for (int j = i + TURN + 1; j < n && j <= i + Ls; j++) {
         int t = ptype(f, i, j);
         if (t) {
-            int e = C_(i, j) + AU(t);
+            int e = C_(i, j) + AU(P, t);
             fi = imin(fi, e + F_(f, j + 1));
-            fi = imin(fi, e + P.dangle3[t][S1[j + 1]] + F_(f, j + 2));
+            fi = imin(fi, e + P->dangle3[t][S1[j + 1]] + F_(f, j + 2));
         }
         t = ptype(f, i + 1, j);
         if (t) {
-            int e = C_(i + 1, j) + P.dangle5[t][S1[i]] + AU(t);
+            int e = C_(i + 1, j) + P->dangle5[t][S1[i]] + AU(P, t);
             fi = imin(fi, e + F_(f, j + 1));
-            fi = imin(fi, e + P.dangle3[t][S1[j + 1]] + F_(f, j + 2));
+            fi = imin(fi, e + P->dangle3[t][S1[j + 1]] + F_(f, j + 2));
         }
     }
     if (n <= i + Ls) {
         int t = ptype(f, i, n);
-        if (t) fi = imin(fi, C_(i, n) + AU(t));
+        if (t) fi = imin(fi, C_(i, n) + AU(P, t));
         t = ptype(f, i + 1, n);
-        if (t) fi = imin(fi, C_(i + 1, n) + P.dangle5[t][S1[i]] + AU(t));
+        if (t) fi = imin(fi, C_(i + 1, n) + P->dangle5[t][S1[i]] + AU(P, t));
     }
     f->f3[i] = fi;
 }
@@ -258,6 +284,7 @@ typedef struct { int i, j, ml; } sect_t;
 /* two-loop (p,q) that reproduces c(i,j): p ascending, q descending, first match (last with TB_LOOP_LAST) */
 static int two_loop_split(const fold_t *f, int i, int j, int cij, int t, int *pp, int *qq)
 {
+    const params_t *P = f->P;
     int found = 0;
     int pmax = imin(j - 2 - TURN, i + MAXLOOP + 1);
     for (int p = i + 1; p <= pmax; p++) {
@@ -266,7 +293,7 @@ static int two_loop_split(const fold_t *f, int i, int j, int cij, int t, int *pp
         for (int q = j - 1; q >= minq; q--) {
             int t2 = ptype(f, p, q);
             if (!t2) continue;
-            if (cij == loop_E(f, i, j, p, q, t, P.rtype[t2]) + C_(p, q)) {
+            if (cij == loop_E(f, i, j, p, q, t, P->rtype[t2]) + C_(p, q)) {
                 *pp = p; *qq = q; found = 1;
                 if (!(f->mut & TB_LOOP_LAST)) return 1;
             }
@@ -278,16 +305,17 @@ static int two_loop_split(const fold_t *f, int i, int j, int cij, int t, int *pp
 /* multiloop closed by (i,j): split k ascending (descending with TB_MLC_LAST), four dangle variants per k */
 static int ml_split(const fold_t *f, int i, int j, int cij, int t, int *kk, int *i1, int *j1)
 {
-    int tt = P.rtype[t];
-    int mm = P.MLclosing + P.MLintern[tt];
-    int d5 = P.dangle5[tt][f->S1[j - 1]], d3 = P.dangle3[tt][f->S1[i + 1]];
+    const params_t *P = f->P;
+    int tt = P->rtype[t];
+    int mm = P->MLclosing + P->MLintern[tt];
+    int d5 = P->dangle5[tt][f->S1[j - 1]], d3 = P->dangle3[tt][f->S1[i + 1]];
     const int klo = i + 2 + TURN, khi = j - 3 - TURN;
     const int last = (f->mut & TB_MLC_LAST) != 0, rev = (f->mut & TB_MLC_VARIANT) != 0;
     for (int s = 0; s <= khi - klo; s++) {
         int k = last ? khi - s : klo + s;
         for (int o = 0; o < 4; o++) {
             int v = rev ? 3 - o : o, a = v & 1, b = v >> 1;   /* v: 0 (i+1,j-1), 1 (i+2,j-1), 2 (i+1,j-2), 3 (i+2,j-2) */
-            int e = M_(i + 1 + a, k) + M_(k + 1, j - 1 - b) + mm + (a ? d3 : 0) + (b ? d5 : 0) + (a + b) * P.MLbase;
+            int e = M_(i + 1 + a, k) + M_(k + 1, j - 1 - b) + mm + (a ? d3 : 0) + (b ? d5 : 0) + (a + b) * P->MLbase;
             if (cij == e) { *kk = k; *i1 = i + 1 + a; *j1 = j - 1 - b; return 1; }
         }
     }
@@ -297,6 +325,7 @@ static int ml_split(const fold_t *f, int i, int j, int cij, int t, int *kk, int 
 /* returns malloc'ed finalised structure string, or NULL on "backtrack failed" */
 static char *traceback(fold_t *f, int start, int md)
 {
+    const params_t *P = f->P;
     const int n = f->n;
     const short *S1 = f->S1;
     int ndash = imin(n - start, md) + 1;
@@ -322,9 +351,9 @@ static char *traceback(fold_t *f, int start, int md)
                     int a = (o == 0) == !(f->mut & TB_F3_ORDER) ? i + 1 : i;
                     int t = ptype(f, a, k);
                     if (!t) continue;
-                    int cc = C_(a, k) + (a > i ? P.dangle5[t][S1[i]] : 0) + AU(t);
+                    int cc = C_(a, k) + (a > i ? P->dangle5[t][S1[i]] : 0) + AU(P, t);
                     if (fij == cc + F_(f, k + 1)) traced = a;
-                    if (k < n && fij == F_(f, k + 2) + cc + P.dangle3[t][S1[k + 1]]) { traced = a; jj = k + 2; }
+                    if (k < n && fij == F_(f, k + 2) + cc + P->dangle3[t][S1[k + 1]]) { traced = a; jj = k + 2; }
                 }
                 if (traced) {
                     bt = traced; bjj = jj; bk = k;
@@ -341,16 +370,16 @@ static char *traceback(fold_t *f, int start, int md)
             int fij = M_(i, j);
             for (int o = 0; o < 2; o++) {   /* 3' base first (5' first with TB_FML_PEEL_5) */
                 int five = (o == 0) == !!(f->mut & TB_FML_PEEL_5);
-                if (M_(i + five, j - !five) + P.MLbase == fij) { PUSH(i + five, j - !five, 1); goto next; }
+                if (M_(i + five, j - !five) + P->MLbase == fij) { PUSH(i + five, j - !five, 1); goto next; }
             }
             int t = ptype(f, i, j);
-            int cij = C_(i, j) + P.MLintern[t];
+            int cij = C_(i, j) + P->MLintern[t];
             t = ptype(f, i + 1, j);
-            int ci1j = C_(i + 1, j) + P.dangle5[t][S1[i]] + P.MLintern[t] + P.MLbase;
+            int ci1j = C_(i + 1, j) + P->dangle5[t][S1[i]] + P->MLintern[t] + P->MLbase;
             t = ptype(f, i, j - 1);
-            int cij1 = C_(i, j - 1) + P.dangle3[t][S1[j]] + P.MLintern[t] + P.MLbase;
+            int cij1 = C_(i, j - 1) + P->dangle3[t][S1[j]] + P->MLintern[t] + P->MLbase;
             t = ptype(f, i + 1, j - 1);
-            int ci1j1 = C_(i + 1, j - 1) + P.dangle5[t][S1[i]] + P.dangle3[t][S1[j]] + P.MLintern[t] + 2 * P.MLbase;
+            int ci1j1 = C_(i + 1, j - 1) + P->dangle5[t][S1[i]] + P->dangle3[t][S1[j]] + P->MLintern[t] + 2 * P->MLbase;
             if (fij == cij || fij == ci1j || fij == cij1 || fij == ci1j1) {
                 /* first match of ci1j, cij1, ci1j1, cij (the reverse with TB_FML_PAIR_ORDER) */
                 const int e[4] = {ci1j, cij1, ci1j1, cij}, di[4] = {1, 0, 1, 0}, dj[4] = {0, 1, 1, 0};
@@ -441,11 +470,10 @@ static void add_hit(lfold_result *r, const fold_t *f, char *ss, int start)
     r->n_hits++;
 }
 
-/* Fold one raw sequence token (A.6 conversion, A.3 fill, A.5 emission); `mut`: TB_* bits of the
- * tracebacks (0 = RNALfold's). */
-lfold_result *lfold_oracle_fold_mut(const char *raw, int n, int L, int keep_matrices, int mut)
+/* Fold one raw sequence token (A.6 conversion, A.3 fill, A.5 emission) with the tables, two-loop filter and hairpin
+ * perturbation of `pert`; `mut`: TB_* bits of the tracebacks (0 = RNALfold's). */
+static lfold_result *fold_core(const char *raw, int n, int L, int keep_matrices, int mut, const fold_t *pert)
 {
-    params_init();
     lfold_result *r = (lfold_result *)calloc(1, sizeof *r);
     r->n = n;
     r->conv = (char *)malloc((size_t)n + 1);
@@ -471,6 +499,10 @@ lfold_result *lfold_oracle_fold_mut(const char *raw, int n, int L, int keep_matr
     for (size_t k = 0; k < cells; k++) f->c[k] = f->m[k] = f->dml[k] = INF;
     f->f3 = (int *)calloc((size_t)n + 4, sizeof(int));
     f->mut = mut;
+    f->P = pert->P; f->PL = pert->PL;
+    f->ln1 = pert->ln1; f->ln2 = pert->ln2; f->lpar = pert->lpar; f->ls = pert->ls; f->ld = pert->ld;
+    f->ldelta = pert->ldelta;
+    f->hs = pert->hs; f->hdelta = pert->hdelta;
 
     /* A.5 emission state machine, static state is per-call here (one Lfold() per process
      * call sequence in the reference keeps statics across records, but they are always
@@ -513,9 +545,113 @@ lfold_result *lfold_oracle_fold_mut(const char *raw, int n, int L, int keep_matr
     return r;
 }
 
+static void pert_none(fold_t *pf)
+{
+    params_init();
+    memset(pf, 0, sizeof *pf);
+    pf->P = pf->PL = &P0;
+    pf->ln1 = -2;
+    pf->hs = -1;
+}
+
+lfold_result *lfold_oracle_fold_mut(const char *raw, int n, int L, int keep_matrices, int mut)
+{
+    fold_t pf;
+    pert_none(&pf);
+    return fold_core(raw, n, L, keep_matrices, mut, &pf);
+}
+
 lfold_result *lfold_oracle_fold(const char *raw, int n, int L, int keep_matrices)
 {
     return lfold_oracle_fold_mut(raw, n, L, keep_matrices, 0);
+}
+
+static int in_range(const int *x, int k, int lo, int hi)
+{
+    for (int a = 0; a < k; a++)
+        if (x[a] < lo || x[a] > hi) return 0;
+    return 1;
+}
+
+/* The fold of lfold_oracle_fold_mut with one term class raised by `delta` dcal (PERT_*, index x[]):
+ *   SHAPE (n1, n2, parity)   every two-loop with n1 / n2 unpaired bases whose outer pair has j-i of that parity (stacks
+ *                            and bulges included)
+ *   RING (s, d)              every two-loop of n1+n2 = s closed by a pair with j-i = d
+ *   HAIRPIN_SIZE (s)         every hairpin of s unpaired bases, after the lxc*log extrapolation of s > 30
+ *   STACK (t, t2), BULGE (s), INTERNAL (s), INT11 (t, t2, x, y), INT22 (t, t2, a, b, c, d), MISMATCH_I (t, x, y),
+ *   MISMATCH_H (t, x, y), HAIRPIN (s), TETRA (k)
+ *                            that entry of the table, wherever it is read
+ *   INT21 (n1, t, t2, x, y, z)   int21[t][t2][x][y][z], read by 1x2 loops of that n1 only (1: 5' side 1 nt, 2: 2 nt)
+ * Returns NULL for an unknown kind or an index out of range. */
+lfold_result *lfold_oracle_fold_pert(const char *raw, int n, int L, int keep_matrices, int mut, int kind, const int *x,
+                                     int delta)
+{
+    fold_t pf;
+    pert_none(&pf);
+    params_t *Q = (params_t *)malloc(sizeof *Q);
+    *Q = P0;
+    int *e = NULL, ok = 1;
+    switch (kind) {
+    case PERT_NONE: break;
+    case PERT_SHAPE:
+        ok = in_range(x, 2, 0, MAXLOOP) && x[0] + x[1] <= MAXLOOP && in_range(x + 2, 1, 0, 1);
+        pf.ln1 = x[0]; pf.ln2 = x[1]; pf.lpar = x[2]; pf.ls = pf.ld = -1; pf.ldelta = delta;
+        break;
+    case PERT_RING:
+        ok = in_range(x, 1, 0, MAXLOOP) && x[1] >= 0;
+        pf.ln1 = pf.ln2 = pf.lpar = -1; pf.ls = x[0]; pf.ld = x[1]; pf.ldelta = delta;
+        break;
+    case PERT_HAIRPIN_SIZE: ok = x[0] >= 3; pf.hs = x[0]; pf.hdelta = delta; break;
+    case PERT_STACK: if ((ok = in_range(x, 2, 0, 7))) e = &Q->stack[x[0]][x[1]]; break;
+    case PERT_BULGE: if ((ok = in_range(x, 1, 0, MAXLOOP))) e = &Q->bulge[x[0]]; break;
+    case PERT_INTERNAL: if ((ok = in_range(x, 1, 0, MAXLOOP))) e = &Q->internal_loop[x[0]]; break;
+    case PERT_HAIRPIN: if ((ok = in_range(x, 1, 0, MAXLOOP))) e = &Q->hairpin[x[0]]; break;
+    case PERT_TETRA: if ((ok = in_range(x, 1, 0, T99_N_TETRALOOPS - 1))) e = &Q->tetra_energy[x[0]]; break;
+    case PERT_INT11: if ((ok = in_range(x, 2, 0, 7) && in_range(x + 2, 2, 0, 4))) e = &Q->int11[x[0]][x[1]][x[2]][x[3]]; break;
+    case PERT_INT22:
+        if ((ok = in_range(x, 2, 0, 7) && in_range(x + 2, 4, 0, 4))) e = &Q->int22[x[0]][x[1]][x[2]][x[3]][x[4]][x[5]];
+        break;
+    case PERT_MISMATCH_I: if ((ok = in_range(x, 1, 0, 7) && in_range(x + 1, 2, 0, 4))) e = &Q->mismatchI[x[0]][x[1]][x[2]]; break;
+    case PERT_MISMATCH_H: if ((ok = in_range(x, 1, 0, 7) && in_range(x + 1, 2, 0, 4))) e = &Q->mismatchH[x[0]][x[1]][x[2]]; break;
+    case PERT_INT21:
+        if ((ok = in_range(x, 1, 1, 2) && in_range(x + 1, 2, 0, 7) && in_range(x + 3, 3, 0, 4))) {
+            e = &Q->int21[x[1]][x[2]][x[3]][x[4]][x[5]];
+            pf.ln1 = x[0]; pf.ln2 = 3 - x[0]; pf.lpar = pf.ls = pf.ld = -1;
+        }
+        break;
+    default: ok = 0;
+    }
+    lfold_result *r = NULL;
+    if (ok) {
+        if (e) *e += delta;
+        if (kind == PERT_INT21) pf.PL = Q;
+        else if (e) pf.P = pf.PL = Q;
+        r = fold_core(raw, n, L, keep_matrices, mut, &pf);
+    }
+    free(Q);
+    return r;
+}
+
+/* hairpin_E of the pair (i, j) (1-based) of a raw sequence, with the unmodified tables: the energy of a long hairpin,
+ * whose fold would cost O(n^3) in the multiloop decomposition */
+int lfold_oracle_hairpin_energy(const char *raw, int n, int i, int j)
+{
+    params_init();
+    if (i < 1 || j > n || j - i - 1 < TURN) return INF;
+    char *conv = (char *)malloc((size_t)n + 1);
+    short *S = (short *)calloc((size_t)n + 3, sizeof(short)), *S1 = (short *)calloc((size_t)n + 3, sizeof(short));
+    for (int k = 0; k < n; k++) {
+        char ch = raw[k];
+        if (ch >= 'a' && ch <= 'z') ch = (char)(ch - 32);
+        conv[k] = ch == 'T' ? 'U' : ch;
+        S[k + 1] = (short)enc(conv[k]);
+        S1[k + 1] = (short)ALIAS[S[k + 1]];
+    }
+    conv[n] = 0;
+    int t = P0.pair[S[i]][S[j]];
+    int e = t ? hairpin_tab(&P0, conv, S1, i, j, t) : INF;
+    free(conv); free(S); free(S1);
+    return e;
 }
 
 void lfold_oracle_free(lfold_result *r)

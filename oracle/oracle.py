@@ -27,6 +27,25 @@ TIEBREAK = {
     "FML_SPLIT_LAST": 1 << 9,   # fML segment: last split k
 }
 
+# Energy perturbations (lfold_oracle_fold_pert, PERT_*): kind -> (code, index length).  fold(..., perturb=(kind, *index),
+# delta=d) raises that term class by d dcal.  Tests only: a class whose raise changes the c matrix is the unique minimiser
+# of some cell, where a kernel that computes it wrongly must differ from the oracle.
+PERTURB = {
+    "shape": (1, 3),            # (n1, n2, parity of j-i): every two-loop of that shape (stacks and bulges included)
+    "ring": (2, 2),             # (s, d): every two-loop of n1+n2 = s closed by a pair on diagonal j-i = d
+    "hairpin_size": (3, 1),     # (s,): every hairpin of s unpaired bases, after the log extrapolation of s > 30
+    "stack": (4, 2),            # table entries: stack[t][t2], bulge[s], internal_loop[s], int11[t][t2][x][y], ...
+    "bulge": (5, 1),
+    "internal_loop": (6, 1),
+    "int11": (7, 4),
+    "int21": (8, 6),            # (n1, t, t2, x, y, z): int21[t][t2][x][y][z] as read by 1x2 loops with that n1 only
+    "int22": (9, 6),
+    "mismatchI": (10, 3),
+    "mismatchH": (11, 3),
+    "hairpin": (12, 1),
+    "tetra": (13, 1),           # (k,): the k-th entry of the tetraloop list
+}
+
 
 def build():
     subprocess.run(["make", "-C", HERE, "all"], check=True, stdout=subprocess.DEVNULL)
@@ -42,6 +61,10 @@ def lib():
         L.lfold_oracle_fold.restype = C.c_void_p
         L.lfold_oracle_fold_mut.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int]
         L.lfold_oracle_fold_mut.restype = C.c_void_p
+        L.lfold_oracle_fold_pert.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.c_int]
+        L.lfold_oracle_fold_pert.restype = C.c_void_p
+        L.lfold_oracle_hairpin_energy.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_int]
+        L.lfold_oracle_hairpin_energy.restype = C.c_int
         L.lfold_oracle_free.argtypes = [C.c_void_p]
         for name in ("nhits", "total", "failed", "W"):
             getattr(L, "lfold_oracle_" + name).argtypes = [C.c_void_p]
@@ -60,11 +83,21 @@ def lib():
     return _lib
 
 
-def fold(seq, span, matrices=False, tiebreak=0):
-    """-> dict(hits=[(ss, energy_dcal, start)], total=int[, c, m, f3]).  tiebreak: OR of TIEBREAK bits (0 = RNALfold)."""
+def fold(seq, span, matrices=False, tiebreak=0, perturb=None, delta=1):
+    """-> dict(hits=[(ss, energy_dcal, start)], total=int[, c, m, f3]).  tiebreak: OR of TIEBREAK bits (0 = RNALfold);
+    perturb: (kind, *index) of PERTURB, whose term class costs `delta` dcal more in this fold (None = RNALfold)."""
     L = lib()
     b = seq.encode() if isinstance(seq, str) else seq
-    r = L.lfold_oracle_fold_mut(b, len(b), span, 1 if matrices else 0, int(tiebreak))
+    if perturb is None:
+        r = L.lfold_oracle_fold_mut(b, len(b), span, 1 if matrices else 0, int(tiebreak))
+    else:
+        code, nidx = PERTURB[perturb[0]]
+        if len(perturb) != 1 + nidx:
+            raise ValueError("perturb %r: %s takes %d indices" % (perturb, perturb[0], nidx))
+        idx = (C.c_int * 6)(*[int(v) for v in perturb[1:]])
+        r = L.lfold_oracle_fold_pert(b, len(b), span, 1 if matrices else 0, int(tiebreak), code, idx, int(delta))
+        if not r:
+            raise ValueError("perturb %r: index out of range" % (perturb,))
     try:
         if L.lfold_oracle_failed(r):
             raise RuntimeError("oracle: backtrack failed")
@@ -79,6 +112,12 @@ def fold(seq, span, matrices=False, tiebreak=0):
         return out
     finally:
         L.lfold_oracle_free(r)
+
+
+def hairpin_energy(seq, i, j):
+    """Energy (dcal) of the hairpin closed by (i, j), 1-based, with the unmodified tables; 1000000 if (i, j) cannot pair."""
+    b = seq.encode() if isinstance(seq, str) else seq
+    return lib().lfold_oracle_hairpin_energy(b, len(b), int(i), int(j))
 
 
 def fold_text(text, span, binary=None):
